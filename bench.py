@@ -7,7 +7,7 @@ optimize=True) + all-pairs set-graph build (tol 0.01).  One "step" = one pass of
 that hot path over the seed batch.  Metric: convex sets built per second
 (whole job), with set-pair checks/s alongside.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU): every rank builds its own 256
 seeds over the replicated scene (weak scaling), the sets are exchanged by peer
@@ -22,6 +22,10 @@ clocks, gpu_launches) the line carries
               (strong scaling over the ranks), the MPC step geometry (us per step)
   adjacency_equals_single_rank   (N > 1) the exchanged global graph re-tested by
               rank 0 alone, outside the timed region
+
+--dump-outputs DIR saves the results of the last timed step as .npy files.  The
+inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -352,6 +356,10 @@ def run_gpu(args):
     barrier()
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # before the end-to-end and per-stage runs below, which write into the same buffers
+        dump_outputs(args.dump_outputs, out, spipe.adjacency_bits() if spipe is not None else bits, S_total, geo,
+                     world, rank, dist)
 
     # ---- end to end through the public API with host buffers
     for _ in range(2):
@@ -509,6 +517,39 @@ def run_gpu(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_LIMIT = 64_000_000      # bytes, all files written by --dump-outputs together
+
+
+def dump_outputs(out_dir, out, bits, S_total, geo, world, rank, dist):
+    """What the last timed step handed its callers, one .npy per array: the sets of every rank's seeds in rank
+    order (halfspaces padded to m_max rows, row counts, ellipsoids, centres, status) and the global adjacency
+    matrix (upper triangle, 0/1).  Integer arrays are stored as float64, which holds them exactly.  When the dense
+    adjacency would take the files over DUMP_LIMIT, a fixed, seeded sample of its rows is stored instead and
+    adjacency_rows.npy lists their indices.  Every rank calls this (the sets are gathered); rank 0 writes."""
+    import torch
+
+    arrays = {}
+    for name in ("A", "b", "m", "q_ellipse", "p_mid", "status"):
+        t = getattr(out, name).contiguous()
+        if world > 1:
+            parts = [torch.empty_like(t) for _ in range(world)]
+            dist.all_gather(parts, t)
+            t = torch.cat(parts)
+        arrays[name] = t.cpu().numpy().astype(np.float64)
+    if rank != 0:
+        return
+    adj = geo.unpack_adjacency(bits, S_total)
+    room = DUMP_LIMIT - sum(a.nbytes for a in arrays.values()) - 8 * 4096       # 4 KiB per file for .npy headers
+    if S_total * S_total * 4 > room:
+        rows = np.sort(np.random.default_rng(0).choice(S_total, room // (S_total * 4 + 8), replace=False))
+        arrays["adjacency_rows"] = rows.astype(np.float64)
+        adj = adj[torch.as_tensor(rows, device=adj.device)]
+    arrays["adjacency"] = adj.cpu().numpy().astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ----------------------------------------------------------------------------
@@ -967,7 +1008,13 @@ def main():
     ap.add_argument("--no-plan-latency", action="store_true")
     ap.add_argument("--no-cuda-graph", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C3 / C4 / C5 measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (all sets and the global graph)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; the reference arm has none to write")
     if args.impl == "reference":
         run_reference(args)
     else:

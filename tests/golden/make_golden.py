@@ -12,7 +12,8 @@ fk_reference_blobs.npz  The reference's OWN serialized CasADi functions (bound_p
                     209,229 load) evaluated at 64 configurations by oracle/casadi_blob.py (a CasADi-free
                     decoder + SX virtual machine); djacobian = the directional derivative of jacobian.ca
                     along dq (forward-mode AD through the same program).  Reference-generated golden vectors: they pin the FK oracle
-                    and the FK kernel.  Needs /root/reference (this container only).
+                    and the FK kernel.  Needs a checkout of the reference named by
+                    BOUNDPLANNER_REFERENCE.
 c1_sets_golden.npz  The first two convex sets the reference's example plan builds
                     (boundplanner_example.py:89-92 -> BoundPlanner.py:278-294,
                     :381-389) as computed by the ORACLE; lets the GPU box check
@@ -45,8 +46,8 @@ def main():
              T_ee=np.array([ofk.hom_transform_endeffector(x) for x in q]),
              jac=np.array([ofk.jacobian_fk(x) for x in q]))
 
-    ref_dir = "/root/reference/bound_planner/RobotModel/"
-    if os.path.isdir(ref_dir):
+    ref_dir = os.path.join(os.environ.get("BOUNDPLANNER_REFERENCE", ""), "bound_planner", "RobotModel", "")
+    if os.environ.get("BOUNDPLANNER_REFERENCE") and os.path.isdir(ref_dir):
         from oracle.casadi_blob import SXFunctionBlob
 
         qg = rng.uniform(ofk.Q_LOWER, ofk.Q_UPPER, (64, 7))

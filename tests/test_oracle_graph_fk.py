@@ -8,6 +8,9 @@ from oracle import fk_iiwa14 as ofk
 from oracle.set_graph import adjacency, intersection_margin, set_intersection
 
 BOX = np.vstack((np.eye(3), -np.eye(3)))
+# the reference's RobotModel directory, in a checkout named by BOUNDPLANNER_REFERENCE (not part of this repository)
+REF_MODEL = os.path.join(os.environ.get("BOUNDPLANNER_REFERENCE", ""), "bound_planner", "RobotModel")
+NO_REF = "reference checkout not available (set BOUNDPLANNER_REFERENCE)"
 
 
 def _box(lb, ub):
@@ -75,13 +78,13 @@ def test_fk_golden_fixture():
         assert np.abs(ofk.hom_transform_endeffector(q) - g["T_ee"][i]).max() < 1e-12
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/bound_planner/RobotModel/iiwa.urdf"),
-                    reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not os.environ.get("BOUNDPLANNER_REFERENCE") or
+                    not os.path.exists(os.path.join(REF_MODEL, "iiwa.urdf")), reason=NO_REF)
 def test_fk_constants_equal_the_reference_urdf():
     """Re-read the joint origins straight from the reference's URDF."""
     import xml.etree.ElementTree as ET
 
-    root = ET.parse("/root/reference/bound_planner/RobotModel/iiwa.urdf").getroot()
+    root = ET.parse(os.path.join(REF_MODEL, "iiwa.urdf")).getroot()
     joints = {j.get("name"): j for j in root.findall("joint")}
     for k in range(7):
         o = joints[f"joint_{k + 1}"].find("origin")
@@ -124,14 +127,13 @@ def test_fk_oracle_pinned_to_reference_casadi_blobs():
         assert np.abs(ofk.jacobian_fk(q) - g["jacobian"][i]).max() < 1e-12
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/bound_planner/RobotModel/fk_pos.ca"),
-                    reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not os.environ.get("BOUNDPLANNER_REFERENCE") or
+                    not os.path.exists(os.path.join(REF_MODEL, "fk_pos.ca")), reason=NO_REF)
 def test_casadi_blob_decoder_reproduces_committed_golden():
     from oracle.casadi_blob import SXFunctionBlob
 
     g = np.load(os.path.join(os.path.dirname(__file__), "golden", "fk_reference_blobs.npz"))
-    d = "/root/reference/bound_planner/RobotModel/"
-    f_pos, f_c5, f_jac = SXFunctionBlob(d + "fk_pos.ca"), SXFunctionBlob(d + "fk_pos_col_5.ca"), SXFunctionBlob(d + "jacobian.ca")
+    f_pos, f_c5, f_jac = (SXFunctionBlob(os.path.join(REF_MODEL, f)) for f in ("fk_pos.ca", "fk_pos_col_5.ca", "jacobian.ca"))
     assert f_pos.name_in == ["i0"] and f_pos.sp_in[0][:2] == (7, 1) and f_jac.sp_out[0][:2] == (6, 7)
     for i in (0, 1, 17, 63):
         q = g["q"][i]

@@ -11,7 +11,7 @@ import sys
 import numpy as np
 import pytest
 
-REF = os.environ.get("BOUNDPLANNER_REFERENCE", "/root/reference")
+REF = os.environ.get("BOUNDPLANNER_REFERENCE", "")     # a checkout of the reference, not part of this repository
 NEEDED = ("casadi", "cvxpy", "cdd", "pinocchio")
 
 
@@ -22,9 +22,9 @@ def _reference():
             importlib.import_module(name)
         except Exception:  # noqa: BLE001
             missing.append(name)
-    if missing or not os.path.isdir(os.path.join(REF, "bound_planner")):
+    if missing or not REF or not os.path.isdir(os.path.join(REF, "bound_planner")):
         pytest.skip("true reference unavailable: " + (", ".join(missing) + " not importable" if missing
-                                                      else f"{REF} not present"))
+                                                      else "set BOUNDPLANNER_REFERENCE to a checkout of it"))
     if REF not in sys.path:
         sys.path.insert(0, REF)
     os.chdir(REF)                       # CA_SAVE_PATH is relative (RobotModel.py:9)

@@ -37,6 +37,7 @@ constexpr int SET_ROWS = 48;      // BP_MAX_ROWS
 constexpr int REF_MAX_ROWS = 20;  // the reference's MVIE buffers (quirk Q5)
 constexpr int MAX_PATH = 64;
 constexpr int FIT_SAMPLES = 20;   // check_intersection walks 20 rotations (:745-772)
+constexpr int OBS_ROWS = 15;      // rows of a polytope obstacle (normalize_set_size, padded with a = 0, b = 10)
 
 // error classes of the Python planner: RuntimeError / ValueError
 enum ErrKind { ERR_NONE = 0, ERR_RUNTIME = 1, ERR_VALUE = 2 };
@@ -116,7 +117,8 @@ struct Params {           // BoundPlanner.__init__ (:47-58)
 };
 
 struct QueryInput {
-  const double* boxes;    // [n_obs,6] (lb, ub), uninflated
+  const double* boxes;    // [n_obs,6] (lb, ub), uninflated; or NULL when obs_rows is set
+  const double* obs_rows; // [n_obs,OBS_ROWS,4] (a0, a1, a2, b) of inflated polytope obstacles, or NULL
   int n_obs;
   double start[3], end[3], l_ee[3], l_ee_end[3];
   double ee_samples[FIT_SAMPLES * 3];    // Rodrigues(omega_hat, |omega| k/19) l_ee, k = 0..19
@@ -243,6 +245,29 @@ struct Query {
     // :199-204, obstacle by obstacle in order: an `end` inside an inflated obstacle is pushed out through the
     // face of largest A x - b (rows [I; -I], b = [ub + r, -lb + r], padded rows -10)
     const double r = par->obs_size_increase;
+    if (qi.obs_rows) {
+      // general polytopes: all 15 rows, padding (0, 0, 0, 10) included.  A x - b is formed as (a0 x0 + a1 x1) + a2 x2
+      // - b without contraction, as the Python planner's general path does: this differs from the reference's
+      // ob[0] @ end (BLAS, may fuse) in the last bits only, and is exact for box rows (+-e_k), where it equals the
+      // box arithmetic below
+      for (int o = 0; o < qi.n_obs; ++o) {
+        const double* ro = qi.obs_rows + (size_t)o * OBS_ROWS * 4;
+        double viol[OBS_ROWS];
+        bool any_pos = false;
+        for (int i = 0; i < OBS_ROWS; ++i) {
+          const double* a = ro + 4 * i;
+          viol[i] = (a[0] * end[0] + a[1] * end[1]) + a[2] * end[2] - a[3];
+          any_pos = any_pos || (viol[i] > 0.0);
+        }
+        if (any_pos) continue;
+        int idx = 0;                                             // first index of the maximum (np.argmax)
+        for (int i = 1; i < OBS_ROWS; ++i)
+          if (viol[i] > viol[idx]) idx = i;
+        const double step = viol[idx] - r;
+        for (int k = 0; k < 3; ++k) end[k] -= step * ro[4 * idx + k];
+      }
+      return;
+    }
     for (int o = 0; o < qi.n_obs; ++o) {
       const double* bx = qi.boxes + 6 * o;
       double viol[6];
@@ -956,7 +981,8 @@ inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& 
   qs.resize((size_t)in.Q);
   for (int q = 0; q < in.Q; ++q) {
     QueryInput qi;
-    qi.boxes = in.boxes + 6 * (size_t)in.box_off[q];
+    qi.boxes = in.obs_rows ? nullptr : in.boxes + 6 * (size_t)in.box_off[q];
+    qi.obs_rows = in.obs_rows ? in.obs_rows + (size_t)OBS_ROWS * 4 * in.box_off[q] : nullptr;
     qi.n_obs = in.box_off[q + 1] - in.box_off[q];
     for (int k = 0; k < 3; ++k) {
       qi.start[k] = in.starts[3 * q + k]; qi.end[k] = in.ends[3 * q + k];

@@ -72,11 +72,18 @@ def _set_errors(status, rows):
 
 class GpuBackend:
     """Answers planner requests one at a time: a batch of one through the same executor the lock-step driver
-    uses, so every request is one chain of kernels on the device and one read-back."""
+    uses, so every request is one chain of kernels on the device and one read-back.  Obstacles: boxes
+    (``obstacles`` [N,6], inflated by obs_size_increase) or, with ``obs_sets``, inflated convex polytopes (vertex
+    lists from ``obs_points_sets``, enumerated on the device when missing)."""
 
     device_loop = True       # sampling / duplicate test / shortest path on the device (K11-K13)
 
-    def __init__(self, obstacles, obs_size_increase, workspace_max, workspace_min):
+    def __init__(self, obstacles, obs_size_increase, workspace_max, workspace_min, obs_sets=None, obs_points_sets=None):
+        if obs_sets is not None:
+            self.obs_sets = obs_sets
+            self._bx = BatchedGpuExecutor(None, obs_size_increase, workspace_max, workspace_min,
+                                          polytope_scenes=[(obs_sets, obs_points_sets)])
+            return
         self.obs_sets = obstacle_sets(obstacles, obs_size_increase)
         self._bx = BatchedGpuExecutor([np.asarray(obstacles, float).reshape(-1, 6)], obs_size_increase, workspace_max,
                                       workspace_min)
@@ -100,9 +107,27 @@ def obstacle_sets(obstacles, obs_size_increase):
     return [[a_all[i], b_all[i]] for i in range(n)]
 
 
+_BOX_ROWS = np.concatenate((np.eye(3), -np.eye(3)))
+
+
+def is_box_obstacle(a_set):
+    """The rows of an axis-aligned box as add_obstacle_reps builds them (A = [I; -I], zero padding): the test of
+    convex_set_finder.boxes_from_obs_sets."""
+    a_set = np.asarray(a_set, float)
+    return a_set.shape[0] >= 6 and np.array_equal(a_set[:6], _BOX_ROWS) and not np.any(a_set[6:] != 0.0)
+
+
+def _rows_minus_b(A, b, x):
+    """A x - b over stacked padded rows (A [..., 15, 3], b [..., 15]) as (a0 x0 + a1 x1) + a2 x2 - b, element by
+    element: no BLAS, no fused multiply-add, the operation order of the native driver's push-out (bp_planner.h).  It
+    differs from the reference's ob[0] @ x in the last bits only, and is exact for box rows."""
+    return (A[..., 0] * x[0] + A[..., 1] * x[1]) + A[..., 2] * x[2] - b
+
+
 class SetSequencePlanner:
     def __init__(self, obstacles=(), obs_size_increase=0.08, workspace_max=(1.0, 1.0, 1.2),
-                 workspace_min=(-1.0, -1.0, 0.0), backend=None, rng=None, obs_sets=None, device_loop=None):
+                 workspace_min=(-1.0, -1.0, 0.0), backend=None, rng=None, obs_sets=None, device_loop=None,
+                 obs_points_sets=None):
         # device_loop: sampling / duplicate test / shortest path answered by the backend's kernels (K11-K13)
         # instead of the host loops below; default: whatever the backend offers
         self.device_loop = bool(getattr(backend, "device_loop", False)) if device_loop is None else bool(device_loop)
@@ -130,9 +155,22 @@ class SetSequencePlanner:
         else:
             self.obs_sets = obstacle_sets(obstacles, obs_size_increase)
         self._obstacles = obstacles
+        self.obs_points_sets = obs_points_sets
+        # general convex polytopes (any obstacle that is not a box): the host tests run on all 15 rows of every
+        # obstacle (_rows_minus_b); box-shaped obs_sets keep the vectorised box forms below
+        self.polytopes = not all(is_box_obstacle(ob[0]) for ob in self.obs_sets)
+        if self.polytopes:
+            n = len(self.obs_sets)
+            self._obs_A = np.zeros((n, 15, 3))
+            self._obs_b = np.full((n, 15), 10.0)
+            for k, (a_set, b_set) in enumerate(self.obs_sets):
+                a_set = np.asarray(a_set, float).reshape(-1, 3)
+                self._obs_A[k, : a_set.shape[0]] = a_set
+                self._obs_b[k, : a_set.shape[0]] = np.asarray(b_set, float).reshape(-1)
         # inflated box bounds for the vectorised form of the "sample in collision" test (:467-471): for a box
         # row (+-e_k) the reference's A x - b is exactly x_k - ub_k / lb_k - x_k, padded rows give -10
-        ob_b = np.array([ob[1][:6] for ob in self.obs_sets]).reshape(-1, 6)
+        ob_b = (np.zeros((len(self.obs_sets), 6)) if self.polytopes else       # (polytopes: not used)
+                np.array([ob[1][:6] for ob in self.obs_sets]).reshape(-1, 6))
         self._ub, self._lb = ob_b[:, :3], -ob_b[:, 3:]
         self._b6 = np.ascontiguousarray(ob_b)                 # b of the rows [I; -I]: A x - b = [x; -x] - b6
 
@@ -170,8 +208,44 @@ class SetSequencePlanner:
     def _in_collision(self, sample):
         if self._ub.shape[0] == 0:
             return False
+        if self.polytopes:                                    # max over all 15 rows < 1e-3 (sample_flags)
+            return bool((_rows_minus_b(self._obs_A, self._obs_b, sample).max(axis=1) < 1e-3).any())
         s6 = np.concatenate((sample, -sample))                # x - ub and lb - x = (-x) - (-lb), exactly
         return bool(((s6 - self._b6).max(axis=1) < 1e-3).any())
+
+    def _push_out_boxes(self, end):
+        """:199-204 over box obstacles, in place: obstacle by obstacle in order; the scan for the next obstacle that
+        contains `end` is vectorised (box rows: A x - b is x_k - ub_k / lb_k - x_k; the padded rows give -10 and never
+        decide)."""
+        cursor = 0
+        while cursor < len(self.obs_sets):
+            inside = np.flatnonzero((np.maximum(end - self._ub[cursor:], self._lb[cursor:] - end) <= 0).all(axis=1))
+            if inside.size == 0:
+                break
+            ob = self.obs_sets[cursor + int(inside[0])]
+            viol = ob[0] @ end - ob[1]
+            if not np.any(viol > 0):
+                idx = np.argmax(viol)
+                end -= (viol[idx] - self.obs_size_increase) * ob[0][idx, :]
+            cursor += int(inside[0]) + 1
+        return end
+
+    def _push_out_general(self, end):
+        """:199-204 over general polytope rows, in place: obstacle by obstacle in order, each tested with `end` as
+        already moved; one without a positive A x - b over its 15 rows (padding included) pushes `end` out along its
+        first row of largest A x - b (np.argmax).  The scan for the next such obstacle is vectorised; every A x - b
+        is the element-wise form of _rows_minus_b."""
+        cursor = 0
+        while cursor < len(self.obs_sets):
+            viol = _rows_minus_b(self._obs_A[cursor:], self._obs_b[cursor:], end)
+            inside = np.flatnonzero(~(viol > 0).any(axis=1))
+            if inside.size == 0:
+                break
+            k = int(inside[0])
+            idx = int(np.argmax(viol[k]))
+            end -= (viol[k, idx] - self.obs_size_increase) * self._obs_A[cursor + k, idx]
+            cursor += k + 1
+        return end
 
     # ---- :459-478 on the device ---------------------------------------------------
     def _sample_set_on_device(self, optimize):
@@ -326,19 +400,10 @@ class SetSequencePlanner:
         start = np.array(start, float)
         end = np.array(end, float)
         sampled_first = False
-        # :199-204, obstacle by obstacle in order; the scan for the next obstacle that contains `end` is vectorised
-        # (box rows: A x - b is x_k - ub_k / lb_k - x_k; the padded rows give -10 and never decide)
-        cursor = 0
-        while cursor < len(self.obs_sets):
-            inside = np.flatnonzero((np.maximum(end - self._ub[cursor:], self._lb[cursor:] - end) <= 0).all(axis=1))
-            if inside.size == 0:
-                break
-            ob = self.obs_sets[cursor + int(inside[0])]
-            viol = ob[0] @ end - ob[1]
-            if not np.any(viol > 0):
-                idx = np.argmax(viol)
-                end -= (viol[idx] - self.obs_size_increase) * ob[0][idx, :]
-            cursor += int(inside[0]) + 1
+        if self.polytopes:                                        # :199-204
+            self._push_out_general(end)
+        else:
+            self._push_out_boxes(end)
         self.omega = R.from_matrix(r1 @ r0.T).as_rotvec()        # :207-219
         self.omega_norm = np.linalg.norm(self.omega)
         self.omega_normed = self.omega / self.omega_norm if self.omega_norm > 1e-6 else np.array([0, 0, 1.0])
@@ -364,7 +429,9 @@ class SetSequencePlanner:
                 # the reference pushes `start` out of every inflated obstacle that contains it -- through
                 # `ob.A()[idx, :]` on a list (:311), i.e. it raises AttributeError as soon as one does (quirk Q12);
                 # without such an obstacle the loop does nothing and the start set is built around `start`
-                for k in range(len(self.obs_sets)):
+                if self.polytopes and not (_rows_minus_b(self._obs_A, self._obs_b, start) > 0).any(axis=1).all():
+                    raise AttributeError("'list' object has no attribute 'A'")
+                for k in range(0 if self.polytopes else len(self.obs_sets)):
                     if not np.any(np.concatenate((start, -start)) - self._b6[k] > 0):
                         raise AttributeError("'list' object has no attribute 'A'")
                 a_set, b_set, q_start, p_mid_start, a_red, b_red = yield ("set_point", start, True, True)
@@ -480,7 +547,12 @@ class SetSequencePlanner:
         plan_convex_set_path (:180-183): the start set then comes from the segment start .. horizon point that the
         previous plan's sets (``sets_via_prev``) still cover."""
         if self.backend is None:
-            self.backend = GpuBackend(self._obstacles, self.obs_size_increase, self.workspace_max, self.workspace_min)
+            if self.polytopes:
+                self.backend = GpuBackend(None, self.obs_size_increase, self.workspace_max, self.workspace_min,
+                                          obs_sets=self.obs_sets, obs_points_sets=self.obs_points_sets)
+            else:
+                self.backend = GpuBackend(self._obstacles, self.obs_size_increase, self.workspace_max,
+                                          self.workspace_min)
         gen = self.plan_gen(start, end, r0, r1, first_sample, replanning, p_horizon, new_obs)
         try:
             req = next(gen)
@@ -510,15 +582,21 @@ class BatchedGpuExecutor:
     MAX_NODES = 64           # graph nodes per query the tables hold (2 + 20 samples + via-point re-samples)
     NODE_ROWS = 24           # rows per reduced node set (the reference's sets have at most 20)
 
-    def __init__(self, obstacles_list, obs_size_increase, workspace_max, workspace_min):
+    def __init__(self, obstacles_list, obs_size_increase, workspace_max, workspace_min, polytope_scenes=None):
+        """obstacles_list: one [N_k,6] box array per query; or polytope_scenes: one (obs_sets, obs_points_sets |
+        None) pair per query (inflated polytopes, PolytopeSceneBatch), obstacles_list then unused."""
         from . import geometry as geo
 
         self.geo = geo
-        self.scene = geo.SceneBatch(obstacles_list, obs_size_increase)
+        if polytope_scenes is not None:
+            self.scene = geo.PolytopeSceneBatch(polytope_scenes)
+            self._n_queries = len(polytope_scenes)
+        else:
+            self.scene = geo.SceneBatch(obstacles_list, obs_size_increase)
+            self._n_queries = len(obstacles_list)
         self.ws_min = np.asarray(workspace_min, float)
         self.ws_max = np.asarray(workspace_max, float)
         self.calls = 0
-        self._n_queries = len(obstacles_list)
         self._tab = None
 
     # -- device tables of the queries' graph nodes -------------------------------------
@@ -850,21 +928,32 @@ def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), w
                rng_seeds=None, executor=None):
     """Plan many independent queries in lock step.
 
-    queries: list of dicts(obstacles [N,6], start, end, r0, r1[, first_sample]).
+    queries: list of dicts(obstacles [N,6], start, end, r0, r1[, first_sample]); or, for polytope obstacles,
+    obs_sets (inflated [A (<= 15 x 3), b] per obstacle) [and obs_points_sets] instead of obstacles.  One kind per
+    batch: a batch that mixes them raises ValueError.
     Returns (results, stats): results[i] is the planner's dict or the exception the sequential planner
     would have raised for that query."""
+    from .planner_native import query_kind
+
+    polytopes = query_kind(queries) == "polytopes"
     if executor is None:
-        executor = BatchedGpuExecutor([q["obstacles"] for q in queries], obs_size_increase, workspace_max,
-                                      workspace_min)
+        if polytopes:
+            executor = BatchedGpuExecutor(None, obs_size_increase, workspace_max, workspace_min,
+                                          polytope_scenes=[(q["obs_sets"], q.get("obs_points_sets")) for q in queries])
+        else:
+            executor = BatchedGpuExecutor([q["obstacles"] for q in queries], obs_size_increase, workspace_max,
+                                          workspace_min)
     import time
 
     t_start = time.perf_counter()
     planners, gens, pending, results = [], {}, {}, [None] * len(queries)
     finish = [0.0] * len(queries)              # seconds after the start of the batch at which query i was answered
     for i, q in enumerate(queries):
-        pl = SetSequencePlanner(q["obstacles"], obs_size_increase, workspace_max, workspace_min,
+        pl = SetSequencePlanner(() if polytopes else q["obstacles"], obs_size_increase, workspace_max, workspace_min,
                                 rng=np.random.default_rng(rng_seeds[i] if rng_seeds is not None else None),
-                                device_loop=bool(getattr(executor, "device_loop", False)))
+                                device_loop=bool(getattr(executor, "device_loop", False)),
+                                obs_sets=q["obs_sets"] if polytopes else None,
+                                obs_points_sets=q.get("obs_points_sets") if polytopes else None)
         planners.append(pl)
         gens[i] = pl.plan_gen(q["start"], q["end"], q["r0"], q["r1"], q.get("first_sample"))
         try:

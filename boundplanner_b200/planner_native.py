@@ -15,6 +15,7 @@ import ctypes
 import numpy as np
 
 MAX_NODES, NODE_ROWS, SET_ROWS, MAX_PATH, FIT_SAMPLES = 64, 24, 48, 64, 20
+OBS_ROWS = 15               # rows of a polytope obstacle (normalize_set_size)
 LENGTH_EE = 0.05            # BoundPlanner.__init__ (:54)
 
 _dp = ctypes.POINTER(ctypes.c_double)
@@ -26,7 +27,7 @@ class BpPlanIn(ctypes.Structure):
     _fields_ = [("Q", ctypes.c_int), ("boxes", _dp), ("box_off", _ip), ("inflate", ctypes.c_double), ("ws_min", _dp),
                 ("ws_max", _dp), ("starts", _dp), ("ends", _dp), ("l_ee", _dp), ("l_ee_end", _dp), ("ee_samples", _dp),
                 ("rng", _up), ("has_first", _ip), ("first_sample", _dp), ("sample_chunk", ctypes.c_int),
-                ("max_rounds", ctypes.c_int)]
+                ("max_rounds", ctypes.c_int), ("obs_rows", _dp)]
 
 
 class BpPlanOut(ctypes.Structure):
@@ -56,6 +57,45 @@ def ee_setup(r0, r1, length_ee=LENGTH_EE):
     return l_ee, l_ee_end, samples
 
 
+def query_kind(queries):
+    """'boxes' when every query carries ``obstacles`` ([N,6] lb | ub), 'polytopes' when every query carries
+    ``obs_sets`` (inflated [A (<= 15 x 3), b] per obstacle, optionally ``obs_points_sets``).  One scene batch holds
+    one kind: a batch that mixes them, or a query with both or neither, raises ValueError."""
+    kinds = set()
+    for i, q in enumerate(queries):
+        has_boxes, has_sets = q.get("obstacles") is not None, q.get("obs_sets") is not None
+        if has_boxes == has_sets:
+            raise ValueError(f"query {i} must carry either 'obstacles' (boxes) or 'obs_sets' (polytopes)")
+        kinds.add("polytopes" if has_sets else "boxes")
+    if len(kinds) > 1:
+        raise ValueError("a batch mixes box and polytope queries: one scene batch holds one obstacle kind")
+    return kinds.pop() if kinds else "boxes"
+
+
+def obs_rows_of(obs_sets):
+    """obs_sets -> [N, 15, 4] (a0, a1, a2, b) rows in the given order, padded with (0, 0, 0, 10) as
+    normalize_set_size pads them."""
+    rows = np.zeros((len(obs_sets), OBS_ROWS, 4))
+    rows[:, :, 3] = 10.0
+    for j, (a_set, b_set) in enumerate(obs_sets):
+        a_set = np.asarray(a_set, float).reshape(-1, 3)
+        b_set = np.asarray(b_set, float).reshape(-1)
+        if a_set.shape[0] > OBS_ROWS or b_set.shape[0] != a_set.shape[0]:
+            raise ValueError(f"obstacle {j}: at most {OBS_ROWS} rows (a, b) per polytope")
+        rows[j, : a_set.shape[0], :3], rows[j, : a_set.shape[0], 3] = a_set, b_set
+    return rows
+
+
+def scene_batch(queries, obs_size_increase):
+    """The device scene batch of a batch of queries: SceneBatch over the boxes, or PolytopeSceneBatch over the
+    obs_sets (vertex lists from ``obs_points_sets``, enumerated on the device when missing)."""
+    from . import geometry as geo
+
+    if query_kind(queries) == "polytopes":
+        return geo.PolytopeSceneBatch([(q["obs_sets"], q.get("obs_points_sets")) for q in queries])
+    return geo.SceneBatch([q["obstacles"] for q in queries], obs_size_increase)
+
+
 def rng_state_words(rng):
     """(state_hi, state_lo, inc_hi, inc_lo) of a numpy Generator over PCG64."""
     st = rng.bit_generator.state
@@ -73,10 +113,18 @@ class PackedQueries:
                  want_nodes=True):
         Q = len(queries)
         self.Q = Q
-        boxes = [np.asarray(q["obstacles"], float).reshape(-1, 6) for q in queries]
+        self.kind = query_kind(queries)
         self.box_off = np.zeros(Q + 1, np.int32)
-        self.box_off[1:] = np.cumsum([b.shape[0] for b in boxes])
-        self.boxes = np.ascontiguousarray(np.vstack(boxes)) if Q else np.zeros((0, 6))
+        if self.kind == "polytopes":
+            rows = [obs_rows_of(q["obs_sets"]) for q in queries]
+            self.box_off[1:] = np.cumsum([r.shape[0] for r in rows])
+            self.obs_rows = np.ascontiguousarray(np.concatenate(rows)) if Q else np.zeros((0, OBS_ROWS, 4))
+            self.boxes = None
+        else:
+            boxes = [np.asarray(q["obstacles"], float).reshape(-1, 6) for q in queries]
+            self.box_off[1:] = np.cumsum([b.shape[0] for b in boxes])
+            self.boxes = np.ascontiguousarray(np.vstack(boxes)) if Q else np.zeros((0, 6))
+            self.obs_rows = None
         self.ws_min = np.ascontiguousarray(np.asarray(workspace_min, float).reshape(3))
         self.ws_max = np.ascontiguousarray(np.asarray(workspace_max, float).reshape(3))
         self.starts = np.ascontiguousarray([np.asarray(q["start"], float) for q in queries]).reshape(Q, 3)
@@ -101,12 +149,14 @@ class PackedQueries:
             if q.get("first_sample") is not None:
                 self.has_first[i] = 1
                 self.first_sample[i] = np.asarray(q["first_sample"], float)
-        self.inp = BpPlanIn(Q, self.boxes.ctypes.data_as(_dp), self.box_off.ctypes.data_as(_ip), float(obs_size_increase),
+        self.inp = BpPlanIn(Q, self.boxes.ctypes.data_as(_dp) if self.boxes is not None else None,
+                            self.box_off.ctypes.data_as(_ip), float(obs_size_increase),
                             self.ws_min.ctypes.data_as(_dp), self.ws_max.ctypes.data_as(_dp),
                             self.starts.ctypes.data_as(_dp), self.ends.ctypes.data_as(_dp), self.l_ee.ctypes.data_as(_dp),
                             self.l_ee_end.ctypes.data_as(_dp), self.ee_samples.ctypes.data_as(_dp),
                             self.rng.ctypes.data_as(_up), self.has_first.ctypes.data_as(_ip),
-                            self.first_sample.ctypes.data_as(_dp), int(sample_chunk), 0)
+                            self.first_sample.ctypes.data_as(_dp), int(sample_chunk), 0,
+                            self.obs_rows.ctypes.data_as(_dp) if self.obs_rows is not None else None)
         # outputs
         self.err_kind = np.zeros(Q, np.int32)
         self.err_msg = ctypes.create_string_buffer(160 * max(Q, 1))
@@ -167,20 +217,21 @@ class PackedQueries:
 
 class NativePlanner:
     """A batch of independent planning queries, one scene each, planned in lock step by libbpgeo's native driver.
+    The queries carry boxes (``obstacles``) or polytopes (``obs_sets`` [, ``obs_points_sets``]), all of one kind.
     The scene batch and the device tables are created once; ``run`` can be called again (same scenes)."""
 
     def __init__(self, queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0)):
         import torch
 
         from . import _lib
-        from . import geometry as geo
 
+        query_kind(queries)                      # (a mixed batch fails before anything touches the device)
         if not torch.cuda.is_available():
             raise _lib.BpGeoError("boundplanner_b200 needs a CUDA device (no CPU fallback)")
         self._lib = _lib.load()
         self.queries = queries
         self.infl, self.ws_max, self.ws_min = float(obs_size_increase), list(workspace_max), list(workspace_min)
-        self.scene = geo.SceneBatch([q["obstacles"] for q in queries], obs_size_increase)
+        self.scene = scene_batch(queries, obs_size_increase)
         self._h = ctypes.c_void_p(0)
         self._packed = {}
         _lib.check(self._lib.bp_plan_create(self.scene._h, len(queries), ctypes.byref(self._h)))
@@ -216,7 +267,7 @@ class NativePlanner:
 
 def plan_batch_native(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0),
                       rng_seeds=None, sample_chunk=32):
-    """Drop-in for ``planner.plan_batch``: (results, stats)."""
+    """Drop-in for ``planner.plan_batch``: (results, stats).  Box or polytope queries, one kind per batch."""
     pl = NativePlanner(queries, obs_size_increase, workspace_max, workspace_min)
     try:
         return pl.run(rng_seeds, sample_chunk)

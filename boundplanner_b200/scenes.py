@@ -9,6 +9,7 @@ Definitions follow SURVEY.md section 8(d) / BASELINE.md section 3:
   (BoundPlanner.py:32-33).
 * ``shelf_scene`` -- C4: lattice of thin shelf plates (thickness 0.02 like the
   example's box walls) plus random clutter.
+* ``config_c3_polytope_query`` -- C3 over general convex polytopes (``random_polytope_scene``).
 * ``free_points`` -- rejection sampling that mirrors the planner's test
   "max(A x - b) < 1e-3 for any inflated obstacle => in collision"
   (BoundPlanner.py:467-471).
@@ -120,6 +121,21 @@ def config_c3_query(i, n_obs=200):
         if np.linalg.norm(pts[0] - pts[1]) >= 0.3:
             break
     return obstacles, inflate, pts[0], pts[1], WORKSPACE_MIN.copy(), WORKSPACE_MAX.copy()
+
+
+def config_c3_polytope_query(i, n_obs=200):
+    """Query i of C3 over general convex polytopes: 200 obstacles of random_polytope_scene (boxes with edges
+    U[0.05,0.2], as C3's, cut by up to 9 random planes; taken as already inflated), obs_size_increase 0.01, free
+    start/end (max(A x - b) >= 0.06 for every obstacle) at least 0.3 m apart.
+    Returns (obs_sets, obs_points_sets, inflate, start, end, workspace_min, workspace_max)."""
+    rng = np.random.default_rng(2000 + i)
+    inflate = 0.01
+    obs_sets, obs_points = random_polytope_scene(n_obs, rng, 0.05, 0.2)
+    while True:
+        pts = polytope_free_points(2, obs_sets, 0.06, rng, WORKSPACE_MIN + 0.1, WORKSPACE_MAX - 0.1)
+        if np.linalg.norm(pts[0] - pts[1]) >= 0.3:
+            break
+    return obs_sets, obs_points, inflate, pts[0], pts[1], WORKSPACE_MIN.copy(), WORKSPACE_MAX.copy()
 
 
 def random_polytope_scene(n_obs, rng, size_lo=0.03, size_hi=0.12, max_rows=15, ws_min=WORKSPACE_MIN, ws_max=WORKSPACE_MAX):

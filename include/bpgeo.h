@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define BPGEO_ABI_VERSION 2
+#define BPGEO_ABI_VERSION 3
 #define BP_MAX_ROWS 48 /* hard cap on rows per convex set (reference MVIE cap: 20, quirk Q5) */
 
 typedef struct bp_scene bp_scene;
@@ -310,11 +310,16 @@ int bp_shortest_paths(const int* node_off_dev, const int* edge_off_dev, const in
  * node tables resident on the device, with one H2D and one D2H copy per round.  Each query consumes its own
  * numpy-compatible PCG64 stream exactly as the reference's rng.uniform calls would.
  * The caller provides what involves rotations (scipy's as_rotvec in the reference, :207-219): l_ee, l_ee_end and
- * the 20 rotated offsets of check_intersection (:745-772) per query. */
+ * the 20 rotated offsets of check_intersection (:745-772) per query.
+ * Obstacles come in one of two forms, the form of the plan's scene batch: boxes (obs_rows NULL; the batch from
+ * bp_scene_create_batch) or general convex polytopes (obs_rows set, boxes may be NULL; the batch from
+ * bp_scene_create_polytopes_batch).  bp_plan_run fails when the form of `in` is not the batch's, or when a query's
+ * obstacle count is not its scene's: the host-side push-out of `end` (:199-204) and the device scene must agree. */
 typedef struct {
   int Q;
-  const double* boxes;        /* all scenes back to back [sum n_obs, 6] (lb, ub), as given to bp_scene_create_batch */
-  const int* box_off;         /* [Q+1] */
+  const double* boxes;        /* all scenes back to back [sum n_obs, 6] (lb, ub), as given to bp_scene_create_batch;
+                                 NULL when obs_rows is set */
+  const int* box_off;         /* [Q+1] obstacle offsets of every query (boxes or polytopes) */
   double inflate;             /* obs_size_increase */
   const double* ws_min;       /* [3] */
   const double* ws_max;       /* [3] */
@@ -328,6 +333,7 @@ typedef struct {
   const double* first_sample; /* [Q,3] or NULL */
   int sample_chunk;           /* candidates drawn ahead per sampling request (<= 0: 32; at most 64) */
   int max_rounds;             /* <= 0: default (4000) */
+  const double* obs_rows;     /* [sum n_obs, 15, 4] (a, b) rows of inflated polytope obstacles, or NULL: boxes */
 } bp_plan_in;
 
 typedef struct {
@@ -352,6 +358,8 @@ typedef struct {
                                  kernel chains launched, microseconds spent waiting for the device */
 } bp_plan_out;
 
+/* bp_plan_create takes a box or a polytope scene batch with one scene per query; the per-scene limits of the kernels
+ * the rounds launch are checked here, not in the middle of a run (polytope scenes: at most 16384 obstacles). */
 typedef struct bp_plan bp_plan;
 int bp_plan_create(const bp_scene* scene_batch, int Q, bp_plan** out);
 int bp_plan_run(bp_plan* plan, const bp_plan_in* in, bp_plan_out* out, void* stream);

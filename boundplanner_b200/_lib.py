@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libbpgeo.so")
 
 BP_MAX_ROWS = 48
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 STATUS_OK = 0
 STATUS_ELLIPSE_VIOLATION = 1

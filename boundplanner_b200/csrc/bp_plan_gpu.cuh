@@ -5,7 +5,8 @@
 //   H2D of the round's input arena (one copy)
 //   new graph nodes:  k_set_aabb (their boxes) -> k_plan_commit (rows, box, ellipsoid into the per-query tables)
 //   set requests:     k_sample_filter (K11, sampling requests) -> k_plan_gather_seeds -> K5 (optimised / single
-//                     pass groups) | K2+K3' (segment sets) -> K12 (duplicate distance) -> K8 (reduce_ineqs)
+//                     pass groups) | K2+K3' (segment sets) | k_plan_scatter_rows (given sets to reduce: the previous
+//                     end set of the start fallback) -> K12 (duplicate distance) -> K8 (reduce_ineqs, all groups)
 //   add_edges:        k_pair_list (K6) on the node tables -> k_fit_check (K9) per end-effector group
 //   projections:      k_project (K10) on the node tables
 //   shortest paths:   k_shortest_path (K13)
@@ -44,6 +45,22 @@ __global__ void k_plan_gather_seeds(const double* __restrict__ cand, const int* 
   for (int k = 0; k < 3; ++k) seeds[3 * (size_t)slot[i] + k] = cand[((size_t)i * C + f) * 3 + k];
 }
 
+// set i of a round's reduce group = rows row_off[i] .. row_off[i+1]-1 of rows [.,4] (a0, a1, a2, b), padded to m_max
+// rows with A = 0, b = 10 (what bp_reduce_ineqs takes)
+__global__ void __launch_bounds__(64) k_plan_scatter_rows(const int* __restrict__ row_off, const double* __restrict__ rows,
+                                                          int m_max, double* A, double* b, int* m) {
+  const int i = blockIdx.x;
+  const int r0 = row_off[i], n = row_off[i + 1] - r0;
+  for (int t = threadIdx.x; t < m_max; t += blockDim.x) {
+    const size_t o = (size_t)i * m_max + t;
+    const double* src = rows + 4 * (size_t)(r0 + t);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) A[3 * o + k] = t < n ? src[k] : 0.0;
+    b[o] = t < n ? src[3] : 10.0;
+  }
+  if (threadIdx.x == 0) m[i] = n;
+}
+
 // One lock-step lane: its own streams, arenas and build workspace; the node tables are shared (disjoint slots).
 struct PlanLane {
   // shared with the other lanes (set by bp_plan_create / bp_plan_run)
@@ -72,7 +89,7 @@ struct PlanLane {
   std::string error;
   // what collect() needs to know about the round submit() laid out
   struct Layout {
-    int nS = 0, nE = 0, nProj = 0, nG = 0, nSmp = 0, nPairs = 0, nNew = 0;
+    int nS = 0, nR = 0, nE = 0, nProj = 0, nG = 0, nSmp = 0, nPairs = 0, nNew = 0;
     int n_grp[3] = {0, 0, 0};
     std::vector<int> order, smp_of, e_off;
     size_t o_A, o_b, o_m, o_q, o_p, o_st, o_peak, o_coll, o_Ar, o_br, o_mr, o_dv, o_first, o_res, o_x, o_fits, o_fk, o_epx,
@@ -146,6 +163,10 @@ struct PlanLane {
     const int nProj = (int)r.projs.size(), nG = (int)r.paths.size();
     const int nNew = (int)new_slots.size();
     const int nNodesCsr = nG ? r.node_off.back() : 0, nEdgesCsr = (int)r.edge_dst.size();
+    // given sets to reduce: a fourth group after the set builds, in the same output slots (K8 reduces them all)
+    const int nR = (int)r.reduces.size(), nSet = nS + nR;
+    int nRows = 0;
+    for (const ReduceReq& rq : r.reduces) nRows += rq.m;
 
     // ---- arena layout
     in_used = out_used = 0;
@@ -156,10 +177,11 @@ struct PlanLane {
                            al(sizeof(int) * 2 * nPairs) + al(sizeof(int) * nPairs) + al(sizeof(double) * 3 * nPairs) +
                            al(sizeof(int) * 2 * nProj) + al(sizeof(double) * 3 * nProj) +
                            al(sizeof(int) * (nG + 1)) + 2 * al(sizeof(int) * nG) + al(sizeof(int) * (nNodesCsr + 1)) +
-                           al(sizeof(int) * nEdgesCsr) + al(sizeof(double) * nEdgesCsr);
-    const size_t need_out = 64 * 16 + al(sizeof(double) * nNew * 6) + 2 * al(sizeof(double) * nS * M * 3) +
-                            2 * al(sizeof(double) * nS * M) + al(sizeof(double) * nS * 9) + al(sizeof(double) * nS * 3) +
-                            8 * al(sizeof(int) * nS) + al(sizeof(double) * nS) + al(sizeof(double) * nS * 3) + al(sizeof(int) * nSmp) +
+                           al(sizeof(int) * nEdgesCsr) + al(sizeof(double) * nEdgesCsr) + al(sizeof(int) * (nR + 1)) +
+                           al(sizeof(double) * 4 * nRows);
+    const size_t need_out = 64 * 16 + al(sizeof(double) * nNew * 6) + 2 * al(sizeof(double) * nSet * M * 3) +
+                            2 * al(sizeof(double) * nSet * M) + al(sizeof(double) * nS * 9) + al(sizeof(double) * nS * 3) +
+                            8 * al(sizeof(int) * nSet) + al(sizeof(double) * nS) + al(sizeof(double) * nS * 3) + al(sizeof(int) * nSmp) +
                             4 * al(sizeof(int) * nPairs) + 2 * al(sizeof(double) * 3 * nPairs) + al(sizeof(double) * 3 * nProj) +
                             al(sizeof(int) * nProj) + al(sizeof(int) * nG * MAX_PATH) + al(sizeof(int) * nG) + al(sizeof(double) * nG);
     if (int rc = reserve(need_in, need_out)) return rc;
@@ -236,14 +258,23 @@ struct PlanLane {
       }
       for (int g = 0; g < nG; ++g) { IN_H(int, i_src)[g] = 0; IN_H(int, i_dst)[g] = 1; }
     }
+    const size_t i_roff = take_in(sizeof(int) * (nR + 1)), i_rrows = take_in(sizeof(double) * 4 * nRows);
+    if (nR) {
+      IN_H(int, i_roff)[0] = 0;
+      for (int k = 0; k < nR; ++k) {
+        const ReduceReq& rq = r.reduces[k];
+        memcpy(IN_H(double, i_rrows) + 4 * (size_t)IN_H(int, i_roff)[k], rq.rows, sizeof(double) * 4 * rq.m);
+        IN_H(int, i_roff)[k + 1] = IN_H(int, i_roff)[k] + rq.m;
+      }
+    }
     if (in_used > in_cap) return fail("bp_plan: input arena overflow");
     // outputs
     const size_t o_naabb = take_out(sizeof(double) * nNew * 6);
-    const size_t o_A = take_out(sizeof(double) * nS * M * 3), o_b = take_out(sizeof(double) * nS * M), o_m = take_out(sizeof(int) * nS),
+    const size_t o_A = take_out(sizeof(double) * nSet * M * 3), o_b = take_out(sizeof(double) * nSet * M), o_m = take_out(sizeof(int) * nSet),
                  o_q = take_out(sizeof(double) * nS * 9), o_p = take_out(sizeof(double) * nS * 3), o_st = take_out(sizeof(int) * nS),
                  o_it = take_out(sizeof(int) * nS), o_peak = take_out(sizeof(int) * nS), o_coll = take_out(sizeof(int) * nS),
-                 o_Ar = take_out(sizeof(double) * nS * M * 3), o_br = take_out(sizeof(double) * nS * M), o_mr = take_out(sizeof(int) * nS),
-                 o_rst = take_out(sizeof(int) * nS), o_dv = take_out(sizeof(double) * nS), o_arg = take_out(sizeof(int) * nS),
+                 o_Ar = take_out(sizeof(double) * nSet * M * 3), o_br = take_out(sizeof(double) * nSet * M), o_mr = take_out(sizeof(int) * nSet),
+                 o_rst = take_out(sizeof(int) * nSet), o_dv = take_out(sizeof(double) * nS), o_arg = take_out(sizeof(int) * nS),
                  o_seed = take_out(sizeof(double) * nS * 3), o_first = take_out(sizeof(int) * nSmp);
     const size_t o_res = take_out(sizeof(int) * nPairs), o_x = take_out(sizeof(double) * 3 * nPairs),
                  o_fits = take_out(sizeof(int) * nPairs), o_fk = take_out(sizeof(int) * nPairs),
@@ -268,7 +299,7 @@ struct PlanLane {
     }
     // the requests of a round belong to different queries: the set builds (main stream) and the add_edges /
     // projection / shortest-path chain (side stream) run concurrently between the two copies
-    const bool fork = nS && (nPairs || nProj || nG);
+    const bool fork = nSet && (nPairs || nProj || nG);
     cudaStream_t st2 = fork ? side : stream;
     if (fork) {
       e = cudaEventRecord(ev_in, stream);
@@ -304,10 +335,13 @@ struct PlanLane {
       if (nP && bp_dedupe_distance_tables(OUT_D(double, o_q), OUT_D(double, o_p), nP, tabq, tabp, IN_D(int, i_nbeg), IN_D(int, i_ncnt),
                                           OUT_D(double, o_dv), OUT_D(int, o_arg), stream))
         return fail(bp_last_error_string());
-      if (bp_reduce_ineqs(OUT_D(double, o_A), OUT_D(double, o_b), OUT_D(int, o_m), nS, M, OUT_D(double, o_Ar), OUT_D(double, o_br),
-                          OUT_D(int, o_mr), nullptr, OUT_D(int, o_rst), stream))
-        return fail(bp_last_error_string());
     }
+    if (nR)
+      k_plan_scatter_rows<<<nR, 64, 0, stream>>>(IN_D(int, i_roff), IN_D(double, i_rrows), M, OUT_D(double, o_A) + (size_t)nS * M * 3,
+                                                 OUT_D(double, o_b) + (size_t)nS * M, OUT_D(int, o_m) + nS);
+    if (nSet && bp_reduce_ineqs(OUT_D(double, o_A), OUT_D(double, o_b), OUT_D(int, o_m), nSet, M, OUT_D(double, o_Ar), OUT_D(double, o_br),
+                                OUT_D(int, o_mr), nullptr, OUT_D(int, o_rst), stream))
+      return fail(bp_last_error_string());
     if (nPairs) {
       k_pair_list<<<(nPairs + 7) / 8, 256, 0, st2>>>(tabA, tabb, tabm, R, 0.01, tabaabb, (const int2*)IN_D(int, i_pairs), nPairs,
                                                         OUT_D(int, o_res), OUT_D(double, o_x));
@@ -339,7 +373,7 @@ struct PlanLane {
     if (e != cudaSuccess) return fail("bp_plan: D2H", e);
     launch_us += std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t_launch).count();
     // what collect() needs
-    lay.nS = nS; lay.nE = nE; lay.nProj = nProj; lay.nG = nG; lay.nSmp = nSmp; lay.nPairs = nPairs; lay.nNew = nNew;
+    lay.nS = nS; lay.nR = nR; lay.nE = nE; lay.nProj = nProj; lay.nG = nG; lay.nSmp = nSmp; lay.nPairs = nPairs; lay.nNew = nNew;
     lay.n_grp[0] = n_grp[0]; lay.n_grp[1] = n_grp[1]; lay.n_grp[2] = n_grp[2];
     lay.order.swap(order); lay.smp_of.swap(smp_of); lay.e_off.swap(e_off);
     lay.o_A = o_A; lay.o_b = o_b; lay.o_m = o_m; lay.o_q = o_q; lay.o_p = o_p; lay.o_st = o_st; lay.o_peak = o_peak;
@@ -393,6 +427,16 @@ struct PlanLane {
       memcpy(a.br, OUT_H(double, o_br) + (size_t)j * M, sizeof(double) * mr);
       memcpy(a.Q, OUT_H(double, o_q) + (size_t)j * 9, sizeof(double) * 9);
       memcpy(a.P, OUT_H(double, o_p) + (size_t)j * 3, sizeof(double) * 3);
+    }
+    for (int k = 0; k < lay.nR; ++k) {
+      SetAns& a = r.reduce_ans[k];
+      const size_t j = (size_t)nS + k;
+      a.status = 0;
+      a.m = r.reduces[k].m;
+      a.m_red = OUT_H(int, o_mr)[j];
+      const int mr = std::min(std::max(a.m_red, 0), M);
+      memcpy(a.Ar, OUT_H(double, o_Ar) + j * M * 3, sizeof(double) * 3 * mr);
+      memcpy(a.br, OUT_H(double, o_br) + j * M, sizeof(double) * mr);
     }
     for (int k = 0; k < nE; ++k) {
       const EdgeReq& er = r.edges[k];
@@ -549,6 +593,8 @@ int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* strea
       return 1;
     }
   }
+  const std::string bad = bpplan::check_replan_inputs(*in);
+  if (!bad.empty()) return bp_fail(("bp_plan_run: " + bad).c_str());
   bpplan::Params par;
   std::vector<bpplan::Query> qs;
   const auto t_run0 = std::chrono::steady_clock::now();

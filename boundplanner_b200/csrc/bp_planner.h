@@ -1,7 +1,8 @@
 // bp_planner.h -- native lock-step driver of the planner loop (host C++, no CUDA in this file).
 //
-// Restates, per query, the control flow of bound_planner/BoundPlanner/BoundPlanner.py (non-replanning branch):
-//   plan_convex_set_path  :174-584   start / end sets, sampling loop, dedupe, convergence test
+// Restates, per query, the control flow of bound_planner/BoundPlanner/BoundPlanner.py:
+//   plan_convex_set_path  :174-584   start / end sets (incl. the replanning branch :231-276 and the start-in-collision
+//                                    fallbacks :296-324), sampling loop, dedupe, convergence test
 //   compute_via_points    :586-743   with_rot=False branch (the via points are the p_proj's)
 //   add_edges             :789-896   intersection nodes, projection points, edge costs (quirk Q6)
 // as an explicit state machine (bpplan::Query) that emits REQUESTS for geometric primitives and is resumed with
@@ -9,7 +10,8 @@
 // statement of the loop and the thing this file is tested against (same paths, set sequences and via points).
 // bpplan::run_lockstep advances all queries of a batch together: every round it collects the pending request of
 // every live query, hands them to an Executor by KIND (one batched kernel chain per kind on the GPU executor of
-// bpgeo.cu; a callback into the test harness in tests/host_harness.cpp), and resumes the queries.
+// bpgeo.cu; callbacks into the test harnesses tests/host_harness.cpp and tests/host_harness_replan.cpp), and resumes
+// the queries.
 // What is NOT here (as in planner.py): the final via-point NLP with rotations (Ipopt, :540-555).
 #pragma once
 #include <algorithm>
@@ -38,9 +40,10 @@ constexpr int REF_MAX_ROWS = 20;  // the reference's MVIE buffers (quirk Q5)
 constexpr int MAX_PATH = 64;
 constexpr int FIT_SAMPLES = 20;   // check_intersection walks 20 rotations (:745-772)
 constexpr int OBS_ROWS = 15;      // rows of a polytope obstacle (normalize_set_size, padded with a = 0, b = 10)
+constexpr int MAX_PREV_SETS = 64; // previous sets per query (a planned sequence has at most MAX_PATH sets)
 
-// error classes of the Python planner: RuntimeError / ValueError
-enum ErrKind { ERR_NONE = 0, ERR_RUNTIME = 1, ERR_VALUE = 2 };
+// error classes of the Python planner: RuntimeError / ValueError / IndexError / AttributeError
+enum ErrKind { ERR_NONE = 0, ERR_RUNTIME = 1, ERR_VALUE = 2, ERR_INDEX = 3, ERR_ATTRIBUTE = 4 };
 
 // ---- numpy's default generator (PCG64: 128-bit LCG, XSL-RR output), Generator.uniform's stream ----
 struct Pcg64 {
@@ -69,7 +72,7 @@ struct Pcg64 {
 };
 
 // ---- request / answer records (one pending request per live query and round) ----
-enum ReqKind { REQ_NONE = 0, REQ_SET = 1, REQ_EDGES = 2, REQ_PROJECT = 3, REQ_PATH = 4 };
+enum ReqKind { REQ_NONE = 0, REQ_SET = 1, REQ_EDGES = 2, REQ_PROJECT = 3, REQ_PATH = 4, REQ_REDUCE = 5 };
 enum SetKind { SET_POINT = 0, SET_LINE = 1, SET_SAMPLE = 2 };
 
 struct SetReq {           // find_set_around_point / find_set_collision_avoidance / the sampling round
@@ -94,6 +97,10 @@ struct EdgeAns {          // proj: projection of the pair's target point onto th
 struct ProjReq { int qid, id0, id1; double xd[3]; };     // projection onto rows(node id0) + rows(node id1)
 struct ProjAns { double x[3]; int status; };
 struct PathReq { int qid, n_nodes, edge_begin; };        // CSR of the query's intersection graph (see Round)
+struct ReduceReq {        // reduce_ineqs of a given set (the previous end set of the start fallback, :318-327);
+  int qid, m;             // answered in a SetAns (m_red, Ar, br)
+  const double* rows;     // [m,4] (a0, a1, a2, b)
+};
 
 struct Node {             // graph node: reduced set + ellipsoid
   int m;
@@ -125,6 +132,11 @@ struct QueryInput {
   uint64_t rng[4];
   int has_first_sample;
   double first_sample[3];
+  // replanning (:231-276) and the previous sets (sets_via_prev of the reference, oldest first)
+  int replanning, new_obs, n_horizon, n_prev;
+  const double* p_horizon;  // [n_horizon,3]
+  const int* prev_row_off;  // [n_prev+1] offsets into prev_rows (absolute)
+  const double* prev_rows;  // [.,4] (a0, a1, a2, b)
 };
 
 // 3x3 determinant the way LAPACK's unblocked LU does it (np.linalg.det): partial pivoting, column scaled by the
@@ -153,7 +165,8 @@ inline double det3_lu(const double* q) {
 
 struct Query {
   // ---- program counter ----
-  enum Pc { PC_START, PC_WAIT_START_SET, PC_WAIT_START_LINE, PC_WAIT_END_LINE, PC_EDGES_BEGIN, PC_WAIT_EDGES,
+  enum Pc { PC_START, PC_WAIT_START_SET, PC_WAIT_START_LINE, PC_WAIT_START_POINT, PC_WAIT_START_REDUCE,
+            PC_WAIT_END_LINE, PC_EDGES_BEGIN, PC_WAIT_EDGES,
             PC_PROJECT_NEXT, PC_WAIT_PROJECT, PC_EDGES_DONE, PC_LOOP_TOP, PC_WAIT_PATH, PC_WAIT_SAMPLE,
             PC_SAMPLES_NEXT, PC_WAIT_SETPOINT, PC_DONE };
   enum After { AFTER_START_NODE, AFTER_END_NODE, AFTER_SAMPLE_NODE };
@@ -176,6 +189,7 @@ struct Query {
   std::vector<int> spec_target;            // [n_others] intersection node whose p_proj is the target, -1: none yet
   std::vector<double> spec_xd;             // [n_others,3]
   PathReq path_req;
+  ReduceReq reduce_req;
   std::vector<double> cand;                // candidates of the pending sampling request
 
   // result
@@ -184,6 +198,7 @@ struct Query {
   bool finished = false;
   std::vector<int> path, set_ids;
   std::vector<double> p_via;               // [n,3]
+  double p_horizon_max[3] = {0.0, 0.0, 0.0};   // the horizon point of a replanning query's start segment
   int rounds = 0;
 
   // planner state
@@ -234,6 +249,60 @@ struct Query {
       if (s > v) v = s;
     }
     return v;
+  }
+
+  // max over rows [m,4] of A x - b, formed as (a0 x0 + a1 x1) + a2 x2 - b without contraction (planner._rows_minus_b)
+  static double max_rows_minus_b(const double* rows, int m, const double* x) {
+    double v = -INFINITY;
+    for (int i = 0; i < m; ++i) {
+      const double* a = rows + 4 * i;
+      const double s = (a[0] * x[0] + a[1] * x[1]) + a[2] * x[2] - a[3];
+      if (s > v) v = s;
+    }
+    return v;
+  }
+
+  // :231-266 (SetSequencePlanner.replanning_horizon_index): how far along the horizon the previous sets still hold
+  int horizon_index() const {
+    int idx = 1;
+    for (int s = 0; s < in.n_prev; ++s) {
+      const double* rows = in.prev_rows + 4 * (size_t)in.prev_row_off[s];
+      const int m = in.prev_row_off[s + 1] - in.prev_row_off[s];
+      const bool start_in = max_rows_minus_b(rows, m, start) < 1e-8;
+      int first_out = -1;
+      for (int h = 0; h < in.n_horizon && first_out < 0; ++h)
+        if (!(max_rows_minus_b(rows, m, in.p_horizon + 3 * (size_t)h) < 1e-8)) first_out = h;
+      if (first_out >= 0) {
+        if (first_out != 0 && start_in) idx = std::max(idx, first_out - 1);
+      } else if (start_in) {
+        idx = in.n_horizon - 1;
+        break;
+      }
+    }
+    if (in.new_obs) idx = 1;
+    return idx;
+  }
+
+  // the new_obs fallback's test (:306-312, quirk Q12): `start` inside an inflated obstacle (no row with A x - b > 0;
+  // polytopes: all 15 rows, boxes: the six box rows, as the push-out of `end` forms them)
+  bool start_in_obstacle() const {
+    const double r = par->obs_size_increase;
+    for (int o = 0; o < in.n_obs; ++o) {
+      bool any_pos = false;
+      if (in.obs_rows) {
+        const double* ro = in.obs_rows + (size_t)o * OBS_ROWS * 4;
+        for (int i = 0; i < OBS_ROWS; ++i) {
+          const double* a = ro + 4 * i;
+          any_pos = any_pos || ((a[0] * start[0] + a[1] * start[1]) + a[2] * start[2] - a[3] > 0.0);
+        }
+      } else {
+        const double* bx = in.boxes + 6 * o;
+        for (int k = 0; k < 3; ++k)
+          any_pos = any_pos || (start[k] - (bx[3 + k] + r) > 0.0) || (-start[k] - (-bx[k] + r) > 0.0);
+      }
+      if (!any_pos) return true;
+    }
+    return false;
   }
 
   void init(int id, const Params* p, const QueryInput& qi) {
@@ -443,6 +512,21 @@ struct Query {
     for (;;) {
       switch (pc) {
         case PC_START: {
+          if (in.replanning) {                                                            // :231-276
+            int idx = horizon_index();
+            const int H = in.n_horizon;
+            if (idx < -H || idx >= H) {                  // self.p_horizon[idx] of a horizon too short
+              char buf[96];
+              snprintf(buf, sizeof(buf), "index %d is out of bounds for axis 0 with size %d", idx, H);
+              fail(ERR_INDEX, buf);
+              return;
+            }
+            if (idx < 0) idx += H;
+            for (int k = 0; k < 3; ++k) p_horizon_max[k] = in.p_horizon[3 * (size_t)idx + k];
+            emit_set(SET_LINE, start, p_horizon_max, 0, 0, 0);
+            pc = PC_WAIT_START_LINE;
+            return;
+          }
           emit_set(SET_POINT, start, nullptr, 1, 1, 0);                                  // :278-283
           pc = PC_WAIT_START_SET;
           return;
@@ -464,11 +548,39 @@ struct Query {
         case PC_WAIT_START_LINE: {
           const SetAns& a = *set_ans;
           if (set_error(a.status, a.m)) return;
-          if (a.collision) {
-            fail(ERR_RUNTIME, "start point in collision (the replanning fallbacks of :296-324 are not restated)");
+          if (a.collision) {                                                              // :296-324
+            if (in.new_obs) {
+              // the reference pushes `start` out of every inflated obstacle that contains it through `ob.A()` on a
+              // list: AttributeError as soon as one does (quirk Q12); otherwise a start set around `start`
+              if (start_in_obstacle()) { fail(ERR_ATTRIBUTE, "'list' object has no attribute 'A'"); return; }
+              emit_set(SET_POINT, start, nullptr, 1, 1, 0);
+              pc = PC_WAIT_START_POINT;
+              return;
+            }
+            // "Could not find start set, reusing old end set": sets_via_prev[-1], IndexError on a first plan
+            if (in.n_prev == 0) { fail(ERR_INDEX, "list index out of range"); return; }
+            const int s = in.n_prev - 1;
+            req_kind = REQ_REDUCE;
+            reduce_req.qid = qid;
+            reduce_req.m = in.prev_row_off[s + 1] - in.prev_row_off[s];
+            reduce_req.rows = in.prev_rows + 4 * (size_t)in.prev_row_off[s];
+            pc = PC_WAIT_START_REDUCE;
             return;
           }
           if (!add_node(a.Ar, a.br, a.m_red, a.Q, a.P)) return;
+          after_start_node();
+          continue;
+        }
+        case PC_WAIT_START_POINT: {                     // new_obs start set around `start` (no tool-tip test)
+          const SetAns& a = *set_ans;
+          if (set_error(a.status, a.rows_peak)) return;
+          if (!add_node(a.Ar, a.br, a.m_red, a.Q, a.P)) return;
+          after_start_node();
+          continue;
+        }
+        case PC_WAIT_START_REDUCE: {                    // the reused end set: q_ellipse = I, p_mid = start
+          const double eye[9] = {1.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0, 1.0};
+          if (!add_node(set_ans->Ar, set_ans->br, set_ans->m_red, eye, start)) return;
           after_start_node();
           continue;
         }
@@ -732,8 +844,10 @@ struct Round {
   std::vector<int> node_off, edge_off, edge_dst;                         //   node_off[g], edge_off[node], edge_dst
   std::vector<double> edge_w;
   std::vector<int> path_out, path_len;                                   // [G, MAX_PATH], [G]
-  std::vector<int> set_owner, edge_owner, proj_owner, proj_count, path_owner;   // index into the query array
+  std::vector<ReduceReq> reduces;    std::vector<SetAns> reduce_ans;     // answers: m_red, Ar, br
+  std::vector<int> set_owner, edge_owner, proj_owner, proj_count, path_owner, reduce_owner;   // index into the query array
   void clear() {
+    reduces.clear(); reduce_owner.clear();
     sets.clear(); edges.clear(); projs.clear(); paths.clear(); node_off.clear(); edge_off.clear(); edge_dst.clear();
     edge_has_target.clear(); edge_xd.clear();
     edge_w.clear(); set_owner.clear(); edge_owner.clear(); proj_owner.clear(); proj_count.clear(); path_owner.clear();
@@ -809,7 +923,7 @@ struct Executor {
   // a node was added to query qid's graph (the executor keeps the tables the requests refer to)
   virtual void commit_node(int lane, int qid, int node_id, const Node& n) = 0;
   // start answering every request of the round (asynchronously, if the executor can) / wait for the answers
-  // (set_ans / edge_ans / proj_ans / path_out / path_len filled).  queries: for executors that look at the
+  // (set_ans / edge_ans / proj_ans / path_out / path_len / reduce_ans filled).  queries: for executors that look at the
   // planners' state (the test harness).  Return 0, or an error code that aborts the run.
   virtual int submit(int lane, Round& r, const std::vector<Query>& queries) = 0;
   virtual int collect(int lane, Round& r) = 0;
@@ -878,6 +992,7 @@ inline int run_lockstep(std::vector<Query>& qs, Executor& ex, const Params& par,
           r.paths.push_back(p); r.path_owner.push_back((int)i);
           break;
         }
+        case REQ_REDUCE: r.reduces.push_back(q.reduce_req); r.reduce_owner.push_back((int)i); break;
         default:
           q.fail(ERR_RUNTIME, "planner state machine without a pending request");
           --live;
@@ -896,6 +1011,7 @@ inline int run_lockstep(std::vector<Query>& qs, Executor& ex, const Params& par,
       return 0;
     }
     if (r.set_ans.size() < r.sets.size()) r.set_ans.resize(r.sets.size());      // (records are fully written by the executor)
+    if (r.reduce_ans.size() < r.reduces.size()) r.reduce_ans.resize(r.reduces.size());
     const size_t n_pairs = r.edge_has_target.size();
     if (r.edge_ans.size() < n_pairs) r.edge_ans.resize(n_pairs);
     if (r.proj_ans.size() < r.projs.size()) r.proj_ans.resize(r.projs.size());
@@ -929,6 +1045,8 @@ inline int run_lockstep(std::vector<Query>& qs, Executor& ex, const Params& par,
     }
     for (size_t k = 0; k < r.paths.size(); ++k)
       tasks.push_back(Task{r.path_owner[k], nullptr, nullptr, nullptr, r.path_out.data() + k * (size_t)MAX_PATH, r.path_len[k]});
+    for (size_t k = 0; k < r.reduces.size(); ++k)
+      tasks.push_back(Task{r.reduce_owner[k], &r.reduce_ans[k], nullptr, nullptr, nullptr, 0});
     // one task per live query of the lane: the state machines are independent of each other
     const std::function<void(size_t)> fn = [&](size_t k) {
       const Task& t = tasks[k];
@@ -964,6 +1082,49 @@ inline int run_lockstep(std::vector<Query>& qs, Executor& ex, const Params& par,
 
 namespace bpplan {
 
+// The replanning inputs of a batch (bp_plan_in, ABI 4): "" when they are well-formed, else what is wrong.
+inline std::string check_replan_inputs(const bp_plan_in& in) {
+  char buf[160];
+  const int Q = in.Q;
+  bool any_replan = false;
+  for (int q = 0; in.replanning && q < Q; ++q) any_replan = any_replan || in.replanning[q] != 0;
+  if (any_replan && !in.horizon_off) return "replanning queries without horizon_off";
+  if (in.horizon_off) {
+    if (in.horizon_off[0] != 0) return "horizon_off[0] is not 0";
+    for (int q = 0; q < Q; ++q)
+      if (in.horizon_off[q + 1] < in.horizon_off[q]) {
+        snprintf(buf, sizeof(buf), "horizon_off decreases at query %d", q);
+        return buf;
+      }
+    if (in.horizon_off[Q] > 0 && !in.p_horizon) return "horizon points without p_horizon";
+  }
+  if (in.prev_off) {
+    if (in.prev_off[0] != 0) return "prev_off[0] is not 0";
+    for (int q = 0; q < Q; ++q) {
+      const int n = in.prev_off[q + 1] - in.prev_off[q];
+      if (n < 0) {
+        snprintf(buf, sizeof(buf), "prev_off decreases at query %d", q);
+        return buf;
+      }
+      if (n > MAX_PREV_SETS) {
+        snprintf(buf, sizeof(buf), "query %d has %d previous sets (at most %d)", q, n, MAX_PREV_SETS);
+        return buf;
+      }
+    }
+    const int n_prev = in.prev_off[Q];
+    if (n_prev > 0 && (!in.prev_row_off || !in.prev_rows)) return "previous sets without prev_row_off / prev_rows";
+    if (n_prev > 0 && in.prev_row_off[0] != 0) return "prev_row_off[0] is not 0";
+    for (int s = 0; s < n_prev; ++s) {
+      const int m = in.prev_row_off[s + 1] - in.prev_row_off[s];
+      if (m < 1 || m > SET_ROWS) {
+        snprintf(buf, sizeof(buf), "previous set %d has %d rows (1 .. %d)", s, m, SET_ROWS);
+        return buf;
+      }
+    }
+  }
+  return "";
+}
+
 inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& qs) {
   par.obs_size_increase = in.inflate;
   for (int k = 0; k < 3; ++k) { par.ws_min[k] = in.ws_min[k]; par.ws_max[k] = in.ws_max[k]; }
@@ -992,6 +1153,13 @@ inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& 
     for (int k = 0; k < 4; ++k) qi.rng[k] = in.rng[4 * q + k];
     qi.has_first_sample = in.has_first ? in.has_first[q] : 0;
     for (int k = 0; k < 3; ++k) qi.first_sample[k] = (in.first_sample && qi.has_first_sample) ? in.first_sample[3 * q + k] : 0.0;
+    qi.replanning = in.replanning ? in.replanning[q] : 0;
+    qi.new_obs = in.new_obs ? in.new_obs[q] : 0;
+    qi.n_horizon = in.horizon_off ? in.horizon_off[q + 1] - in.horizon_off[q] : 0;
+    qi.p_horizon = in.horizon_off && in.p_horizon ? in.p_horizon + 3 * (size_t)in.horizon_off[q] : nullptr;
+    qi.n_prev = in.prev_off ? in.prev_off[q + 1] - in.prev_off[q] : 0;
+    qi.prev_row_off = in.prev_off && in.prev_row_off ? in.prev_row_off + in.prev_off[q] : nullptr;
+    qi.prev_rows = in.prev_rows;
     qs[(size_t)q].init(q, &par, qi);
   }
 }
@@ -1018,6 +1186,8 @@ inline void store_results(const std::vector<Query>& qs, const RunStats& st, cons
     for (const Inter& it : Qy.inter) ne += (int)it.adj.size();
     out.n_edges[q] = ne / 2;
     out.finish_round[q] = finish_round[q];
+    if (out.p_horizon_max)
+      for (int k = 0; k < 3; ++k) out.p_horizon_max[3 * q + k] = Qy.p_horizon_max[k];
     if (out.finish_ms) out.finish_ms[q] = finish_ms ? std::max(finish_ms[q], 0.0) : 0.0;
     if (out.node_A && out.node_b && out.node_m) {
       for (size_t n = 0; n < (size_t)MAX_NODES; ++n) {

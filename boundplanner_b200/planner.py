@@ -377,14 +377,18 @@ class SetSequencePlanner:
     def replanning_horizon_index(self, start, p_horizon, new_obs=False):
         """:231-266: how far along the MPC horizon the previous plan's sets still hold.  Walks ``sets_via_prev`` in
         order; a set that contains ``start`` extends the index to the last horizon point before the first one
-        outside it (the whole horizon: stop); ``new_obs`` resets it to 1."""
+        outside it (the whole horizon: stop); ``new_obs`` resets it to 1.  Every A x - b is the element-wise form of
+        _rows_minus_b, as in the native driver: the thresholds are decided on the same bits (the reference's `@`
+        differs from it in the last bits only)."""
         p_horizon = np.asarray(p_horizon, float).reshape(-1, 3)
+        start = np.asarray(start, float)
         max_horizon_idx = 1
         for s in self.sets_via_prev:
-            dist_start = s[0] @ start - s[1]
-            dist_horizon = s[0] @ p_horizon.T - np.expand_dims(s[1], 1)
+            a_set, b_set = np.asarray(s[0], float), np.asarray(s[1], float)
+            dist_start = _rows_minus_b(a_set, b_set, start)
+            dist_horizon = _rows_minus_b(a_set[None], b_set[None], p_horizon.T[:, :, None])      # [H, m]
             start_in = np.max(dist_start) < 1e-8
-            horizon_idx = np.where(np.logical_not(np.max(dist_horizon, axis=0) < 1e-8))[0]
+            horizon_idx = np.where(np.logical_not(np.max(dist_horizon, axis=1) < 1e-8))[0]
             if horizon_idx.shape[0] > 0:
                 if horizon_idx[0] != 0 and start_in:
                     max_horizon_idx = int(np.max((max_horizon_idx, horizon_idx[0] - 1)))
@@ -924,6 +928,19 @@ class BatchedGpuExecutor:
         return out
 
 
+# the exits of plan_convex_set_path a query of a batch records (IndexError / AttributeError: the start-in-collision
+# fallbacks of :296-324)
+_QUERY_ERRORS = (RuntimeError, ValueError, IndexError, AttributeError)
+
+
+def _planned(res, pl):
+    """A planned query's result: the planner's dict plus what the next (re)planning call needs."""
+    res["sets_via_prev"] = pl.sets_via_prev
+    if pl.replanning:
+        res["p_horizon_max"] = pl.p_horizon_max
+    return res
+
+
 def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0),
                rng_seeds=None, executor=None):
     """Plan many independent queries in lock step.
@@ -931,8 +948,12 @@ def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), w
     queries: list of dicts(obstacles [N,6], start, end, r0, r1[, first_sample]); or, for polytope obstacles,
     obs_sets (inflated [A (<= 15 x 3), b] per obstacle) [and obs_points_sets] instead of obstacles.  One kind per
     batch: a batch that mixes them raises ValueError.
+    Replanning (an MPC loop calling the planner again, :231-276): a query may also carry ``replanning``,
+    ``p_horizon`` [H,3], ``new_obs`` and ``sets_via_prev`` (the previous call's sets, [A, b] each; also used by the
+    start-in-collision fallback of a first plan, :296-324).  A batch may mix replanning and first-plan queries.
     Returns (results, stats): results[i] is the planner's dict or the exception the sequential planner
-    would have raised for that query."""
+    would have raised for that query.  A planned query's dict also holds ``sets_via_prev`` (what the planner keeps
+    for its next call) and, when it replanned, ``p_horizon_max``."""
     from .planner_native import query_kind
 
     polytopes = query_kind(queries) == "polytopes"
@@ -954,14 +975,16 @@ def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), w
                                 device_loop=bool(getattr(executor, "device_loop", False)),
                                 obs_sets=q["obs_sets"] if polytopes else None,
                                 obs_points_sets=q.get("obs_points_sets") if polytopes else None)
+        pl.sets_via_prev = [[np.array(a, float), np.array(b, float)] for a, b in q.get("sets_via_prev", ())]
         planners.append(pl)
-        gens[i] = pl.plan_gen(q["start"], q["end"], q["r0"], q["r1"], q.get("first_sample"))
+        gens[i] = pl.plan_gen(q["start"], q["end"], q["r0"], q["r1"], q.get("first_sample"),
+                              bool(q.get("replanning", False)), q.get("p_horizon", ()), bool(q.get("new_obs", False)))
         try:
             pending[i] = next(gens[i])
         except StopIteration as stop:
-            results[i] = stop.value
+            results[i] = _planned(stop.value, pl)
             finish[i] = time.perf_counter() - t_start
-        except (RuntimeError, ValueError) as e:
+        except _QUERY_ERRORS as e:
             results[i] = e
             finish[i] = time.perf_counter() - t_start
     rounds = 0
@@ -973,9 +996,9 @@ def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), w
             try:
                 nxt[i] = gens[i].throw(ans) if isinstance(ans, Exception) else gens[i].send(ans)
             except StopIteration as stop:
-                results[i] = stop.value
+                results[i] = _planned(stop.value, planners[i])
                 finish[i] = time.perf_counter() - t_start
-            except (RuntimeError, ValueError) as e:
+            except _QUERY_ERRORS as e:
                 results[i] = e
                 finish[i] = time.perf_counter() - t_start
         pending = nxt

@@ -16,6 +16,7 @@ import numpy as np
 
 MAX_NODES, NODE_ROWS, SET_ROWS, MAX_PATH, FIT_SAMPLES = 64, 24, 48, 64, 20
 OBS_ROWS = 15               # rows of a polytope obstacle (normalize_set_size)
+MAX_PREV_SETS = 64          # previous sets per query (sets_via_prev)
 LENGTH_EE = 0.05            # BoundPlanner.__init__ (:54)
 
 _dp = ctypes.POINTER(ctypes.c_double)
@@ -27,14 +28,58 @@ class BpPlanIn(ctypes.Structure):
     _fields_ = [("Q", ctypes.c_int), ("boxes", _dp), ("box_off", _ip), ("inflate", ctypes.c_double), ("ws_min", _dp),
                 ("ws_max", _dp), ("starts", _dp), ("ends", _dp), ("l_ee", _dp), ("l_ee_end", _dp), ("ee_samples", _dp),
                 ("rng", _up), ("has_first", _ip), ("first_sample", _dp), ("sample_chunk", ctypes.c_int),
-                ("max_rounds", ctypes.c_int), ("obs_rows", _dp)]
+                ("max_rounds", ctypes.c_int), ("obs_rows", _dp), ("replanning", _ip), ("new_obs", _ip),
+                ("horizon_off", _ip), ("p_horizon", _dp), ("prev_off", _ip), ("prev_row_off", _ip), ("prev_rows", _dp)]
 
 
 class BpPlanOut(ctypes.Structure):
     _fields_ = [("err_kind", _ip), ("err_msg", ctypes.c_char_p), ("path", _ip), ("path_len", _ip), ("set_ids", _ip),
                 ("n_ids", _ip), ("p_via", _dp), ("n_via", _ip), ("rng_out", _up), ("n_nodes", _ip), ("n_inter", _ip),
                 ("n_edges", _ip), ("finish_round", _ip), ("finish_ms", _dp), ("node_A", _dp), ("node_b", _dp), ("node_m", _ip),
-                ("stats", ctypes.POINTER(ctypes.c_longlong))]
+                ("stats", ctypes.POINTER(ctypes.c_longlong)), ("p_horizon_max", _dp)]
+
+_ERRORS = {1: RuntimeError, 2: ValueError, 3: IndexError, 4: AttributeError}
+
+
+def _ptr(a, t):
+    return a.ctypes.data_as(t) if a is not None else None
+
+
+def replan_arrays(queries):
+    """The replanning inputs of bp_plan_in (ABI 4) from the queries' optional ``replanning``, ``new_obs``,
+    ``p_horizon`` [H,3] and ``sets_via_prev`` ([A, b] per set): dict of host arrays, or None when no query carries
+    any of them (the fields stay NULL).  ValueError for more than 64 previous sets in a query, or a set without rows
+    or with more than 48 rows."""
+    keys = ("replanning", "new_obs", "p_horizon", "sets_via_prev")
+    if not any(k in q for q in queries for k in keys):
+        return None
+    Q = len(queries)
+    rp = np.zeros(Q, np.int32)
+    no = np.zeros(Q, np.int32)
+    h_off = np.zeros(Q + 1, np.int32)
+    p_off = np.zeros(Q + 1, np.int32)
+    hz, rows, row_n = [], [], []
+    for i, q in enumerate(queries):
+        rp[i], no[i] = bool(q.get("replanning", False)), bool(q.get("new_obs", False))
+        h = np.asarray(q.get("p_horizon", ()), float).reshape(-1, 3)
+        hz.append(h)
+        h_off[i + 1] = h_off[i] + h.shape[0]
+        prev = q.get("sets_via_prev", ())
+        if len(prev) > MAX_PREV_SETS:
+            raise ValueError(f"query {i}: {len(prev)} previous sets (at most {MAX_PREV_SETS})")
+        for a_set, b_set in prev:
+            a_set = np.asarray(a_set, float).reshape(-1, 3)
+            b_set = np.asarray(b_set, float).reshape(-1)
+            if not 1 <= a_set.shape[0] <= SET_ROWS or b_set.shape[0] != a_set.shape[0]:
+                raise ValueError(f"query {i}: a previous set has {a_set.shape[0]} rows (1 .. {SET_ROWS}, one b each)")
+            rows.append(np.concatenate((a_set, b_set[:, None]), axis=1))
+            row_n.append(a_set.shape[0])
+        p_off[i + 1] = p_off[i] + len(prev)
+    row_off = np.zeros(len(row_n) + 1, np.int32)
+    row_off[1:] = np.cumsum(row_n)
+    return dict(replanning=rp, new_obs=no, horizon_off=h_off,
+                p_horizon=np.ascontiguousarray(np.concatenate(hz)) if Q else np.zeros((0, 3)), prev_off=p_off,
+                prev_row_off=row_off, prev_rows=np.ascontiguousarray(np.concatenate(rows)) if rows else np.zeros((0, 4)))
 
 
 def _rodrigues(omega, phi):
@@ -149,6 +194,8 @@ class PackedQueries:
             if q.get("first_sample") is not None:
                 self.has_first[i] = 1
                 self.first_sample[i] = np.asarray(q["first_sample"], float)
+        self.replan = replan_arrays(queries)
+        rpa = self.replan or {}
         self.inp = BpPlanIn(Q, self.boxes.ctypes.data_as(_dp) if self.boxes is not None else None,
                             self.box_off.ctypes.data_as(_ip), float(obs_size_increase),
                             self.ws_min.ctypes.data_as(_dp), self.ws_max.ctypes.data_as(_dp),
@@ -156,7 +203,11 @@ class PackedQueries:
                             self.l_ee_end.ctypes.data_as(_dp), self.ee_samples.ctypes.data_as(_dp),
                             self.rng.ctypes.data_as(_up), self.has_first.ctypes.data_as(_ip),
                             self.first_sample.ctypes.data_as(_dp), int(sample_chunk), 0,
-                            self.obs_rows.ctypes.data_as(_dp) if self.obs_rows is not None else None)
+                            self.obs_rows.ctypes.data_as(_dp) if self.obs_rows is not None else None,
+                            _ptr(rpa.get("replanning"), _ip), _ptr(rpa.get("new_obs"), _ip),
+                            _ptr(rpa.get("horizon_off"), _ip), _ptr(rpa.get("p_horizon"), _dp),
+                            _ptr(rpa.get("prev_off"), _ip), _ptr(rpa.get("prev_row_off"), _ip),
+                            _ptr(rpa.get("prev_rows"), _dp))
         # outputs
         self.err_kind = np.zeros(Q, np.int32)
         self.err_msg = ctypes.create_string_buffer(160 * max(Q, 1))
@@ -176,6 +227,7 @@ class PackedQueries:
         self.node_b = np.zeros((Q, MAX_NODES, NODE_ROWS)) if want_nodes else None
         self.node_m = np.zeros((Q, MAX_NODES), np.int32) if want_nodes else None
         self.stats = np.zeros(8, np.int64)
+        self.p_horizon_max = np.zeros((Q, 3))
         self.out = BpPlanOut(self.err_kind.ctypes.data_as(_ip), ctypes.cast(self.err_msg, ctypes.c_char_p),
                              self.path.ctypes.data_as(_ip), self.path_len.ctypes.data_as(_ip),
                              self.set_ids.ctypes.data_as(_ip), self.n_ids.ctypes.data_as(_ip),
@@ -186,17 +238,22 @@ class PackedQueries:
                              self.node_A.ctypes.data_as(_dp) if want_nodes else None,
                              self.node_b.ctypes.data_as(_dp) if want_nodes else None,
                              self.node_m.ctypes.data_as(_ip) if want_nodes else None,
-                             self.stats.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)))
+                             self.stats.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)),
+                             self.p_horizon_max.ctypes.data_as(_dp))
 
     def results(self):
         """Per query: dict(path, set_ids, sets_via, p_via, n_nodes, n_inter, n_edges) or the exception the Python
-        planner raises for it."""
+        planner raises for it.  With the node sets (want_nodes), a planned query also gets ``sets_via_prev``: what the
+        planner keeps for its next call -- sets_via, or after the early exit of :361-375 (path [0]) the start set
+        padded to 15 rows (:371-372).  A replanning query also gets ``p_horizon_max``."""
+        from .utils import normalize_set_size
+
         out = []
         raw = self.err_msg.raw
         for q in range(self.Q):
             if self.err_kind[q]:
                 msg = raw[160 * q: 160 * (q + 1)].split(b"\0", 1)[0].decode()
-                out.append((RuntimeError if self.err_kind[q] == 1 else ValueError)(msg))
+                out.append(_ERRORS[int(self.err_kind[q])](msg))
                 continue
             ids = [int(v) for v in self.set_ids[q, : self.n_ids[q]]]
             res = dict(path=[int(v) for v in self.path[q, : self.path_len[q]]], set_ids=ids,
@@ -205,6 +262,10 @@ class PackedQueries:
             if self.node_A is not None:
                 res["sets_via"] = [[self.node_A[q, s, : self.node_m[q, s]].copy(), self.node_b[q, s, : self.node_m[q, s]].copy()]
                                    for s in ids]
+                prev = [[a.copy(), b.copy()] for a, b in res["sets_via"]]
+                res["sets_via_prev"] = normalize_set_size(prev, 15) if res["path"] == [0] else prev
+            if self.replan is not None and self.replan["replanning"][q]:
+                res["p_horizon_max"] = self.p_horizon_max[q].copy()
             out.append(res)
         return out
 
@@ -218,7 +279,8 @@ class PackedQueries:
 class NativePlanner:
     """A batch of independent planning queries, one scene each, planned in lock step by libbpgeo's native driver.
     The queries carry boxes (``obstacles``) or polytopes (``obs_sets`` [, ``obs_points_sets``]), all of one kind.
-    The scene batch and the device tables are created once; ``run`` can be called again (same scenes)."""
+    The scene batch and the device tables are created once; ``run`` can be called again (same scenes), also with
+    new per-query inputs (``queries=``: an MPC loop's replanning calls) over the same obstacles."""
 
     def __init__(self, queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0)):
         import torch
@@ -232,15 +294,31 @@ class NativePlanner:
         self.queries = queries
         self.infl, self.ws_max, self.ws_min = float(obs_size_increase), list(workspace_max), list(workspace_min)
         self.scene = scene_batch(queries, obs_size_increase)
+        self._obstacles = None                   # (kind, offsets, rows) of the scenes, for run(queries=...)
         self._h = ctypes.c_void_p(0)
         self._packed = {}
         _lib.check(self._lib.bp_plan_create(self.scene._h, len(queries), ctypes.byref(self._h)))
 
-    def run(self, rng_seeds=None, sample_chunk=32, want_nodes=True):
-        import torch
+    @staticmethod
+    def _obstacles_of(pk):
+        return pk.kind, pk.box_off, pk.boxes if pk.obs_rows is None else pk.obs_rows
 
-        from . import _lib
-
+    def run(self, rng_seeds=None, sample_chunk=32, want_nodes=True, queries=None):
+        """Plan the batch: (results, stats).  queries: new per-query inputs (start, end, r0, r1, first_sample and the
+        replanning keys of planner.plan_batch) to plan against the scenes of this planner; their obstacles must be
+        the ones it was created with (ValueError otherwise: the host push-out of `end` and the device scene must
+        agree)."""
+        if queries is not None:
+            if len(queries) != len(self.queries):
+                raise ValueError(f"{len(queries)} queries for a planner of {len(self.queries)} scenes")
+            pk = PackedQueries(queries, self.infl, self.ws_max, self.ws_min, rng_seeds, sample_chunk, want_nodes)
+            if self._obstacles is None:
+                self._obstacles = self._obstacles_of(
+                    PackedQueries(self.queries, self.infl, self.ws_max, self.ws_min, None, sample_chunk, False))
+            mine, theirs = self._obstacles, self._obstacles_of(pk)
+            if mine[0] != theirs[0] or not np.array_equal(mine[1], theirs[1]) or not np.array_equal(mine[2], theirs[2]):
+                raise ValueError("the queries' obstacles differ from the scenes this planner was created with")
+            return self._run(pk)
         # the packed host arrays of the batch (inputs incl. every query's generator state, output buffers) are kept
         # per seed list: planning the same batch again only runs the driver
         key = (None if rng_seeds is None else tuple(int(v) for v in rng_seeds), int(sample_chunk), bool(want_nodes))
@@ -249,6 +327,13 @@ class NativePlanner:
             pk = PackedQueries(self.queries, self.infl, self.ws_max, self.ws_min, rng_seeds, sample_chunk, want_nodes)
             if rng_seeds is not None:
                 self._packed = {key: pk}
+        return self._run(pk)
+
+    def _run(self, pk):
+        import torch
+
+        from . import _lib
+
         _lib.check(self._lib.bp_plan_run(self._h, ctypes.byref(pk.inp), ctypes.byref(pk.out),
                                          ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
         return pk.results(), pk.stats_dict()

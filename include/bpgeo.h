@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define BPGEO_ABI_VERSION 3
+#define BPGEO_ABI_VERSION 4
 #define BP_MAX_ROWS 48 /* hard cap on rows per convex set (reference MVIE cap: 20, quirk Q5) */
 
 typedef struct bp_scene bp_scene;
@@ -303,7 +303,8 @@ int bp_shortest_paths(const int* node_off_dev, const int* edge_off_dev, const in
 
 /* ---- native lock-step planner driver (SURVEY 8f; BASELINE config C3) ---------------------------------------
  * bp_plan_run plans Q independent queries, one scene each (a scene batch), in lock step: the per-query loop of
- * BoundPlanner.plan_convex_set_path (BoundPlanner.py:174-584, non-replanning branch) up to the planned set
+ * BoundPlanner.plan_convex_set_path (BoundPlanner.py:174-584, replanning branch :231-276 and the start-in-collision
+ * fallbacks :296-324 included) up to the planned set
  * sequence, add_edges (:789-896) and compute_via_points (:586-743, no rotations) run as C++ state machines on the
  * host (csrc/bp_planner.h); every round, the pending requests of all queries are answered by ONE chain of the
  * kernels above (K11 -> K5 -> K12 -> K8 for sampling rounds, K6 + K9 for add_edges, K10, K13) against per-query
@@ -314,7 +315,15 @@ int bp_shortest_paths(const int* node_off_dev, const int* edge_off_dev, const in
  * Obstacles come in one of two forms, the form of the plan's scene batch: boxes (obs_rows NULL; the batch from
  * bp_scene_create_batch) or general convex polytopes (obs_rows set, boxes may be NULL; the batch from
  * bp_scene_create_polytopes_batch).  bp_plan_run fails when the form of `in` is not the batch's, or when a query's
- * obstacle count is not its scene's: the host-side push-out of `end` (:199-204) and the device scene must agree. */
+ * obstacle count is not its scene's: the host-side push-out of `end` (:199-204) and the device scene must agree.
+ * Replanning (an MPC loop calling the planner again): a query with replanning[q] builds its start set around the
+ * segment start .. p_horizon[idx], idx the horizon index of :231-266 over the query's previous sets; the previous
+ * sets (what the reference keeps in sets_via_prev between calls) also serve the fallback of a start segment in
+ * collision (:296-324): reduce_ineqs of the last one, or IndexError without any (err_kind 3); with new_obs a start
+ * set around `start`, or AttributeError when `start` lies in an inflated obstacle (quirk Q12, err_kind 4).  All
+ * replanning fields may be NULL: no query replans, none has previous sets.  Malformed offsets (not starting at 0,
+ * decreasing), more than 64 sets per query or a set with no row or more than 48 rows fail the call before any
+ * round runs. */
 typedef struct {
   int Q;
   const double* boxes;        /* all scenes back to back [sum n_obs, 6] (lb, ub), as given to bp_scene_create_batch;
@@ -334,10 +343,19 @@ typedef struct {
   int sample_chunk;           /* candidates drawn ahead per sampling request (<= 0: 32; at most 64) */
   int max_rounds;             /* <= 0: default (4000) */
   const double* obs_rows;     /* [sum n_obs, 15, 4] (a, b) rows of inflated polytope obstacles, or NULL: boxes */
+  /* replanning (ABI 4); every field may be NULL */
+  const int* replanning;      /* [Q] 1: replanning call (:231-276) */
+  const int* new_obs;         /* [Q] the reference's new_obs flag */
+  const int* horizon_off;     /* [Q+1] MPC horizon points of every query in p_horizon */
+  const double* p_horizon;    /* [sum H, 3] */
+  const int* prev_off;        /* [Q+1] previous sets of every query (at most 64 per query), oldest first */
+  const int* prev_row_off;    /* [n_prev+1] rows of every previous set in prev_rows (1 .. 48 per set) */
+  const double* prev_rows;    /* [sum rows, 4] (a0, a1, a2, b) */
 } bp_plan_in;
 
 typedef struct {
-  int* err_kind;              /* [Q] 0 planned, 1 RuntimeError, 2 ValueError (the reference's exits) */
+  int* err_kind;              /* [Q] 0 planned, 1 RuntimeError, 2 ValueError, 3 IndexError, 4 AttributeError
+                                 (the reference's exits) */
   char* err_msg;              /* [Q,160] */
   int* path;                  /* [Q,64] intersection-graph node ids of the shortest path */
   int* path_len;              /* [Q] */
@@ -356,6 +374,7 @@ typedef struct {
   int* node_m;                /* [Q,64]      or NULL */
   long long* stats;           /* [8] or NULL: rounds, set requests, pair tests, projections, shortest paths,
                                  kernel chains launched, microseconds spent waiting for the device */
+  double* p_horizon_max;      /* [Q,3] or NULL (ABI 4): p_horizon[idx] of every replanning query */
 } bp_plan_out;
 
 /* bp_plan_create takes a box or a polytope scene batch with one scene per query; the per-scene limits of the kernels

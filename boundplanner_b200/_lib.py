@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libbpgeo.so")
 
 BP_MAX_ROWS = 48
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 STATUS_OK = 0
 STATUS_ELLIPSE_VIOLATION = 1
@@ -44,6 +44,9 @@ SIGNATURES = {
     "bp_scene_create_polytopes_batch": (_i, [_dp, _c.POINTER(_c.c_int), _dp, _c.POINTER(_c.c_int),
                                              _c.POINTER(_c.c_int), _i, _i, _c.POINTER(_vp)]),
     "bp_scene_update": (_i, [_vp, _dp, _i, _d, _vp]),
+    "bp_scene_update_batch": (_i, [_vp, _dp, _c.POINTER(_c.c_int), _i, _d, _vp]),
+    "bp_scene_update_polytopes_batch": (_i, [_vp, _dp, _c.POINTER(_c.c_int), _dp, _c.POINTER(_c.c_int),
+                                             _c.POINTER(_c.c_int), _i, _i, _vp]),
     "bp_scene_destroy": (_i, [_vp]),
     "bp_scene_size": (_i, [_vp]),
     "bp_closest_points": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp]),

@@ -486,7 +486,6 @@ struct bp_plan : bpplan::Executor {
   const bp_scene* scene = nullptr;
   int Q = 0, L = 1;
   bool polytopes = false;                        // the scene batch holds polytopes (bp_plan_in::obs_rows) or boxes
-  std::vector<int> seg_off;                      // [Q+1] host copy of the batch's obstacle offsets
   double *tabA = nullptr, *tabb = nullptr, *tabq = nullptr, *tabp = nullptr, *tabaabb = nullptr;
   int* tabm = nullptr;
   PlanLane lane[BP_PLAN_LANES];
@@ -513,25 +512,28 @@ struct bp_plan : bpplan::Executor {
   }
 };
 
+// the per-scene limit of the polytope kernels a round launches (k_iris_fused / k_poly_point, k_poly_line_p,
+// k_sample_filter)
+static int plan_scene_limits(const bp_scene* sc, const char* fn) {
+  if (sc->rows && sc->n > BP_POLY_SCENE_MAX) {
+    snprintf(g_err, sizeof(g_err), "%s: polytope scenes hold at most %d obstacles (largest scene: %d)", fn,
+             BP_POLY_SCENE_MAX, sc->n);
+    return 1;
+  }
+  return 0;
+}
+
 extern "C" {
 
 int bp_plan_create(const bp_scene* scene_batch, int Q, bp_plan** out) {
   if (!scene_batch || Q < 1 || !out) return bp_fail("bp_plan_create: bad arguments");
   if (!scene_batch->seg_off || scene_batch->n_seg != Q) return bp_fail("bp_plan_create: needs a scene batch with one scene per query");
-  // the per-scene limits of the polytope kernels a round launches (k_iris_fused / k_poly_point, k_poly_line_p,
-  // k_sample_filter): reported here rather than by the first round that builds a set
-  if (scene_batch->rows && scene_batch->n > BP_POLY_SCENE_MAX) {
-    snprintf(g_err, sizeof(g_err), "bp_plan_create: polytope scenes hold at most %d obstacles (largest scene: %d)",
-             BP_POLY_SCENE_MAX, scene_batch->n);
-    return 1;
-  }
-  std::vector<int> seg_off((size_t)Q + 1);
-  BP_CUDA(cudaMemcpy(seg_off.data(), scene_batch->seg_off, sizeof(int) * ((size_t)Q + 1), cudaMemcpyDeviceToHost));
+  // reported here rather than by the first round that builds a set
+  if (plan_scene_limits(scene_batch, "bp_plan_create")) return 1;
   bp_plan* pl = new bp_plan();
   pl->scene = scene_batch;
   pl->Q = Q;
   pl->polytopes = scene_batch->rows != nullptr;
-  pl->seg_off.swap(seg_off);
   // two lanes once there is enough work to split (BPGEO_PLAN_LANES=1 forces plain lock step)
   pl->L = Q >= 32 ? 2 : 1;
   if (const char* ev = getenv("BPGEO_PLAN_LANES")) pl->L = atoi(ev);
@@ -581,18 +583,21 @@ int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* strea
     return bp_fail("bp_plan_run: bad arguments");
   if (in->sample_chunk > 64) return bp_fail("bp_plan_run: sample_chunk is at most 64");
   // the host pushes `end` out of the obstacles of `in`, the device builds sets around the scene batch: same kind, same
-  // obstacle counts
+  // obstacle counts (against the scene's host copy of its offsets, which bp_scene_update_*batch keeps current); an
+  // update may also have crossed the per-scene limit
   if (pl->polytopes && !in->obs_rows)
     return bp_fail("bp_plan_run: the plan's scene batch holds polytopes, the input has no obs_rows");
   if (!pl->polytopes && in->obs_rows)
     return bp_fail("bp_plan_run: the plan's scene batch holds boxes, the input has obs_rows");
   for (int q = 0; q < pl->Q; ++q) {
-    const int n_in = in->box_off[q + 1] - in->box_off[q], n_scene = pl->seg_off[q + 1] - pl->seg_off[q];
+    const int* so = pl->scene->seg_off_host;
+    const int n_in = in->box_off[q + 1] - in->box_off[q], n_scene = so[q + 1] - so[q];
     if (n_in != n_scene) {
       snprintf(g_err, sizeof(g_err), "bp_plan_run: query %d has %d obstacles, its scene %d", q, n_in, n_scene);
       return 1;
     }
   }
+  if (plan_scene_limits(pl->scene, "bp_plan_run")) return 1;
   const std::string bad = bpplan::check_replan_inputs(*in);
   if (!bad.empty()) return bp_fail(("bp_plan_run: " + bad).c_str());
   bpplan::Params par;

@@ -60,6 +60,15 @@ struct bp_scene {
   double* verts;  // device [n, vmax, 3]
   int* nverts;    // device [n]
   int vmax;
+  // scene batches: host copy of seg_off (bp_plan_run checks its inputs against it without a device round trip)
+  int* seg_off_host;
+  // capacities of rows / nrows / nverts (obstacles) and verts (doubles) of a polytope scene
+  int pcap;
+  size_t vcap;
+  // staging of the batch updates (bp_scene_update_batch, bp_scene_update_polytopes_batch): pinned host and device
+  void* stage_h;
+  void* stage_d;
+  size_t stage_h_cap, stage_d_cap;
 };
 
 struct SceneView {
@@ -2568,19 +2577,15 @@ __global__ void __launch_bounds__(128) k_reduce_rows(const double* __restrict__ 
 // (more than vmax vertices).
 // ---------------------------------------------------------------------------
 #define BP_VERT_MERGE 1e-9
-__global__ void __launch_bounds__(128) k_polytope_vertices(const double* __restrict__ A, const double* __restrict__ b,
-                                                           const int* __restrict__ m, int m_max, int vmax,
-                                                           double* __restrict__ V, int* __restrict__ nv_out,
-                                                           int* __restrict__ status) {
-  __shared__ double sA[BP_MAX_ROWS * 3], sb[BP_MAX_ROWS];
+// The vertices of one polytope {x : sA x <= sb} (ms rows in shared memory) by one 128-thread CTA: V[vmax,3] of the
+// set, *nv_out and the returned status are written by thread 0 (the return value is valid there only).
+__device__ __forceinline__ int polytope_vertices_cta(const double* sA, const double* sb, int ms, int vmax,
+                                                     double* __restrict__ V, int* __restrict__ nv_out) {
   __shared__ double sv[BP_RED_VMAX * 3];
   __shared__ int st[BP_RED_VMAX];                   // triple index of every stored candidate
   __shared__ unsigned char dup[BP_RED_VMAX];
   __shared__ int nverts, unbounded, anypair;
-  const int s = blockIdx.x, tid = threadIdx.x;
-  const int ms = m[s];
-  for (int e = tid; e < ms * 3; e += 128) sA[e] = A[(size_t)s * m_max * 3 + e];
-  for (int e = tid; e < ms; e += 128) sb[e] = b[(size_t)s * m_max + e];
+  const int tid = threadIdx.x;
   if (tid == 0) { nverts = 0; unbounded = 0; anypair = 0; }
   __syncthreads();
   // bounded?  a direction of the recession cone, if there is one, can be taken along +-(a_i x a_j)
@@ -2658,19 +2663,32 @@ __global__ void __launch_bounds__(128) k_polytope_vertices(const double* __restr
     for (int u = 0; u < nc; ++u) rank += (!dup[u] && st[u] < st[v]) ? 1 : 0;
     atomicAdd(&n_unique, 1);
     if (rank < vmax) {
-      double* o = V + ((size_t)s * vmax + rank) * 3;
+      double* o = V + (size_t)rank * 3;
       o[0] = sv[3 * v]; o[1] = sv[3 * v + 1]; o[2] = sv[3 * v + 2];
     }
   }
   __syncthreads();
+  int stt = BP_OK;
   if (tid == 0) {
     const int nu = n_unique;
-    nv_out[s] = nu < vmax ? nu : vmax;
-    int stt = BP_OK;
+    *nv_out = nu < vmax ? nu : vmax;
     if (unbounded || !anypair || nu == 0) stt = BP_NOT_A_POLYTOPE;
     else if (nverts > BP_RED_VMAX || nu > vmax) stt = BP_ROW_OVERFLOW;
-    status[s] = stt;
   }
+  return stt;
+}
+
+__global__ void __launch_bounds__(128) k_polytope_vertices(const double* __restrict__ A, const double* __restrict__ b,
+                                                           const int* __restrict__ m, int m_max, int vmax,
+                                                           double* __restrict__ V, int* __restrict__ nv_out,
+                                                           int* __restrict__ status) {
+  __shared__ double sA[BP_MAX_ROWS * 3], sb[BP_MAX_ROWS];
+  const int s = blockIdx.x, tid = threadIdx.x;
+  const int ms = m[s];
+  for (int e = tid; e < ms * 3; e += 128) sA[e] = A[(size_t)s * m_max * 3 + e];
+  for (int e = tid; e < ms; e += 128) sb[e] = b[(size_t)s * m_max + e];
+  const int stt = polytope_vertices_cta(sA, sb, ms, vmax, V + (size_t)s * vmax * 3, nv_out + s);
+  if (tid == 0) status[s] = stt;
 }
 
 // ---------------------------------------------------------------------------
@@ -3215,6 +3233,82 @@ static int set_dyn_smem(const void* fn, size_t bytes) {
   return 0;
 }
 
+// ---------------------------------------------------------------------------
+// Device ingest of a scene batch (bp_scene_update_batch / bp_scene_update_polytopes_batch): the new obstacles arrive
+// in one staging copy and are written into the resident layout by the kernels below, with the host arithmetic of
+// scene_upload / bp_scene_create_polytopes, so that the updated batch holds the bits of a freshly created one.
+// ---------------------------------------------------------------------------
+// boxes [total,6] (lb | ub) -> the six columns lb - inflate | ub + inflate of stride cap, zeros in [total, cap);
+// offsets [n_seg+1] -> seg_off
+__global__ void __launch_bounds__(256) k_scene_ingest_boxes(const double* __restrict__ boxes, int total, int cap,
+                                                            double inflate, double* __restrict__ cols,
+                                                            const int* __restrict__ offsets, int n_seg,
+                                                            int* __restrict__ seg_off) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < n_seg + 1) seg_off[j] = offsets[j];
+  if (j >= cap) return;
+  const bool real = j < total;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    cols[(size_t)k * cap + j] = real ? boxes[6 * (size_t)j + k] - inflate : 0.0;
+    cols[(size_t)(3 + k) * cap + j] = real ? boxes[6 * (size_t)j + 3 + k] + inflate : 0.0;
+  }
+}
+
+// the vertices of every obstacle (rows [total,15,4], nrows [total]) into V [total,vmax,3] / nv [total]; flags[0]
+// receives the smallest 2 j + (1: too many vertices, 0: not a polytope) over the failing obstacles, flags[1] the
+// largest vertex count
+__global__ void __launch_bounds__(128) k_scene_enum_vertices(const double* __restrict__ rows,
+                                                             const int* __restrict__ nrows, int vmax,
+                                                             double* __restrict__ V, int* __restrict__ nv,
+                                                             int* __restrict__ flags) {
+  __shared__ double sA[BP_OBS_ROWS * 3], sb[BP_OBS_ROWS];
+  const int j = blockIdx.x, tid = threadIdx.x;
+  const int ms = nrows[j];
+  const double* r4 = rows + (size_t)j * BP_OBS_ROWS * 4;
+  for (int e = tid; e < ms * 3; e += 128) sA[e] = r4[4 * (e / 3) + e % 3];
+  for (int e = tid; e < ms; e += 128) sb[e] = r4[4 * e + 3];
+  const int stt = polytope_vertices_cta(sA, sb, ms, vmax, V + (size_t)j * vmax * 3, nv + j);
+  if (tid == 0) {
+    if (stt != BP_OK) atomicMin(&flags[0], 2 * j + (stt == BP_ROW_OVERFLOW ? 1 : 0));
+    else atomicMax(&flags[1], nv[j]);
+  }
+}
+
+// one warp per obstacle: rows / nrows copied, the vertices (src stride vmax_in) re-strided to vmax with zeros after
+// the last one, nverts, and the bounding box of the vertices (the min / max loop of bp_scene_create_polytopes, then
+// scene_upload's "- inflate" / "+ inflate" with inflate = 0) into the columns; zeros in [total, cap); seg_off
+__global__ void __launch_bounds__(256) k_scene_ingest_polytopes(
+    const double* __restrict__ rows_in, const int* __restrict__ nrows_in, const double* __restrict__ verts_in,
+    const int* __restrict__ nverts_in, int vmax_in, int total, int vmax, int cap, double inflate,
+    double* __restrict__ rows, int* __restrict__ nrows, double* __restrict__ verts, int* __restrict__ nverts,
+    double* __restrict__ cols, const int* __restrict__ offsets, int n_seg, int* __restrict__ seg_off) {
+  const int lane = threadIdx.x & 31;
+  const int j = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (blockIdx.x == 0)
+    for (int e = threadIdx.x; e < n_seg + 1; e += blockDim.x) seg_off[e] = offsets[e];
+  if (j >= cap) return;
+  if (j >= total) {
+    if (lane < 6) cols[(size_t)lane * cap + j] = 0.0;
+    return;
+  }
+  for (int e = lane; e < BP_OBS_ROWS * 4; e += 32) rows[(size_t)j * BP_OBS_ROWS * 4 + e] = rows_in[(size_t)j * BP_OBS_ROWS * 4 + e];
+  const int nv = nverts_in[j];
+  const double* src = verts_in + (size_t)j * vmax_in * 3;
+  for (int e = lane; e < vmax * 3; e += 32) verts[(size_t)j * vmax * 3 + e] = e < nv * 3 ? src[e] : 0.0;
+  if (lane == 0) { nrows[j] = nrows_in[j]; nverts[j] = nv; }
+  if (lane < 3) {
+    double lo = BP_INF, hi = -BP_INF;
+    for (int t = 0; t < nv; ++t) {
+      const double v = src[3 * t + lane];
+      if (v < lo) lo = v;
+      if (v > hi) hi = v;
+    }
+    cols[(size_t)lane * cap + j] = lo - inflate;
+    cols[(size_t)(3 + lane) * cap + j] = hi + inflate;
+  }
+}
+
 extern "C" {
 
 int bpgeo_abi_version(void) { return BPGEO_ABI_VERSION; }
@@ -3261,6 +3355,13 @@ int bp_prof_read(long long* host_out, int n_seeds, int reset) {
 }
 #endif
 const char* bp_last_error_string(void) { return g_err; }
+
+static int set_seg_off_host(bp_scene* sc, const int* offsets_host) {
+  if (!sc->seg_off_host) sc->seg_off_host = (int*)malloc(sizeof(int) * (size_t)(sc->n_seg + 1));
+  if (!sc->seg_off_host) return bp_fail("out of host memory");
+  memcpy(sc->seg_off_host, offsets_host, sizeof(int) * (size_t)(sc->n_seg + 1));
+  return 0;
+}
 
 static int scene_upload(bp_scene* sc, const double* boxes_host, int n, double inflate, cudaStream_t stream) {
   if (n > sc->cap) {
@@ -3319,6 +3420,7 @@ int bp_scene_create_batch(const double* boxes_host, const int* offsets_host, int
   if (e == cudaSuccess)
     e = cudaMemcpy(sc->seg_off, offsets_host, sizeof(int) * (size_t)(n_scenes + 1), cudaMemcpyHostToDevice);
   if (e != cudaSuccess) { bp_scene_destroy(sc); return bp_fail("bp_scene_create_batch", e); }
+  if (set_seg_off_host(sc, offsets_host)) { bp_scene_destroy(sc); return 1; }
   *out = sc;
   return 0;
 }
@@ -3356,6 +3458,8 @@ int bp_scene_create_polytopes(const double* rows_host, const int* nrows_host, co
   if (e == cudaSuccess) e = cudaMemcpy(sc->verts, verts_host, sizeof(double) * (size_t)n * vmax * 3, cudaMemcpyHostToDevice);
   if (e == cudaSuccess) e = cudaMemcpy(sc->nverts, nverts_host, sizeof(int) * (size_t)n, cudaMemcpyHostToDevice);
   sc->vmax = vmax;
+  sc->pcap = n;
+  sc->vcap = (size_t)n * vmax * 3;
   if (e != cudaSuccess) { bp_scene_destroy(sc); return bp_fail("bp_scene_create_polytopes", e); }
   *out = sc;
   return 0;
@@ -3381,6 +3485,7 @@ int bp_scene_create_polytopes_batch(const double* rows_host, const int* nrows_ho
   if (e == cudaSuccess)
     e = cudaMemcpy(sc->seg_off, offsets_host, sizeof(int) * (size_t)(n_scenes + 1), cudaMemcpyHostToDevice);
   if (e != cudaSuccess) { bp_scene_destroy(sc); return bp_fail("bp_scene_create_polytopes_batch", e); }
+  if (set_seg_off_host(sc, offsets_host)) { bp_scene_destroy(sc); return 1; }
   *out = sc;
   return 0;
 }
@@ -3392,8 +3497,225 @@ int bp_scene_update(bp_scene* scene, const double* boxes_host, int n, double inf
   return scene_upload(scene, boxes_host, n, inflate, (cudaStream_t)stream);
 }
 
+// checks of a batch update: the scene is a batch of the given kind and of n_scenes scenes, the offsets start at 0
+// and do not decrease; returns the largest scene size, or -1 (g_err set)
+static int update_check(const bp_scene* sc, const int* offsets_host, int n_scenes, bool polytopes, const char* fn) {
+  if (!sc || !offsets_host || n_scenes < 1 || offsets_host[0] != 0) {
+    snprintf(g_err, sizeof(g_err), "%s: bad arguments", fn);
+    return -1;
+  }
+  if (!sc->seg_off) {
+    snprintf(g_err, sizeof(g_err), "%s: not a scene batch", fn);
+    return -1;
+  }
+  if ((sc->rows != nullptr) != polytopes) {
+    snprintf(g_err, sizeof(g_err), "%s: the scene batch holds %s (use %s)", fn, sc->rows ? "polytopes" : "boxes",
+             sc->rows ? "bp_scene_update_polytopes_batch" : "bp_scene_update_batch");
+    return -1;
+  }
+  if (n_scenes != sc->n_seg) {
+    snprintf(g_err, sizeof(g_err), "%s: %d scenes for a batch of %d", fn, n_scenes, sc->n_seg);
+    return -1;
+  }
+  int n_max = 0;
+  for (int k = 0; k < n_scenes; ++k) {
+    const int nk = offsets_host[k + 1] - offsets_host[k];
+    if (nk < 0) {
+      snprintf(g_err, sizeof(g_err), "%s: offsets must be non-decreasing", fn);
+      return -1;
+    }
+    n_max = nk > n_max ? nk : n_max;
+  }
+  return n_max;
+}
+
+// the scene of obstacle j of a batch
+static int scene_of_obstacle(const int* offsets_host, int j) {
+  int k = 0;
+  while (offsets_host[k + 1] <= j) ++k;
+  return k;
+}
+
+static size_t stage_align(size_t b) { return (b + 255) & ~(size_t)255; }
+
+// grow the update staging to hbytes pinned host / dbytes device bytes (the new buffer before the old one is released)
+static int stage_reserve(bp_scene* sc, size_t hbytes, size_t dbytes) {
+  if (hbytes > sc->stage_h_cap) {
+    void* p = nullptr;
+    const size_t cap = hbytes + hbytes / 4;
+    BP_CUDA(cudaMallocHost(&p, cap));
+    if (sc->stage_h) cudaFreeHost(sc->stage_h);
+    sc->stage_h = p;
+    sc->stage_h_cap = cap;
+  }
+  if (dbytes > sc->stage_d_cap) {
+    void* p = nullptr;
+    const size_t cap = dbytes + dbytes / 4;
+    BP_CUDA(cudaMalloc(&p, cap));
+    if (sc->stage_d) cudaFree(sc->stage_d);
+    sc->stage_d = p;
+    sc->stage_d_cap = cap;
+  }
+  return 0;
+}
+
+int bp_scene_update_batch(bp_scene* scene, const double* boxes_host, const int* offsets_host, int n_scenes,
+                          double inflate, void* stream) {
+  const int n_max = update_check(scene, offsets_host, n_scenes, false, "bp_scene_update_batch");
+  if (n_max < 0) return 1;
+  const int total = offsets_host[n_scenes];
+  if (total > 0 && !boxes_host) return bp_fail("bp_scene_update_batch: bad arguments");
+  cudaStream_t st = (cudaStream_t)stream;
+  // staging: boxes [total,6] | offsets [n_scenes+1]
+  const size_t o_off = stage_align(sizeof(double) * 6 * (size_t)total);
+  const size_t bytes = o_off + sizeof(int) * (size_t)(n_scenes + 1);
+  if (stage_reserve(scene, bytes, bytes)) return 1;
+  int new_cap = scene->cap;
+  double* cols = scene->cols;
+  if (total > scene->cap) {
+    new_cap = ((total + 31) / 32) * 32;
+    BP_CUDA(cudaMalloc(&cols, sizeof(double) * 6 * (size_t)new_cap));
+  }
+  char* h = (char*)scene->stage_h;
+  const char* d = (const char*)scene->stage_d;
+  if (total > 0) memcpy(h, boxes_host, sizeof(double) * 6 * (size_t)total);
+  memcpy(h + o_off, offsets_host, sizeof(int) * (size_t)(n_scenes + 1));
+  cudaError_t e = cudaMemcpyAsync(scene->stage_d, h, bytes, cudaMemcpyHostToDevice, st);
+  if (e == cudaSuccess) {
+    const int items = new_cap > n_scenes + 1 ? new_cap : n_scenes + 1;
+    k_scene_ingest_boxes<<<(items + 255) / 256, 256, 0, st>>>((const double*)d, total, new_cap, inflate, cols,
+                                                             (const int*)(d + o_off), n_scenes, scene->seg_off);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);      // (the pinned staging is reused by the next update)
+  if (e != cudaSuccess) {
+    if (cols != scene->cols) cudaFree(cols);
+    return bp_fail("bp_scene_update_batch", e);
+  }
+  if (cols != scene->cols) {
+    if (scene->cols) cudaFree(scene->cols);
+    scene->cols = cols;
+    scene->cap = new_cap;
+  }
+  scene->n = n_max;
+  scene->inflate = inflate;
+  memcpy(scene->seg_off_host, offsets_host, sizeof(int) * (size_t)(n_scenes + 1));
+  return 0;
+}
+
+#define BP_ENUM_VMAX 64                       // vertices per obstacle enumerated by bp_scene_update_polytopes_batch
+
+int bp_scene_update_polytopes_batch(bp_scene* scene, const double* rows_host, const int* nrows_host,
+                                    const double* verts_host, const int* nverts_host, const int* offsets_host,
+                                    int n_scenes, int vmax, void* stream) {
+  const char* fn = "bp_scene_update_polytopes_batch";
+  const int n_max = update_check(scene, offsets_host, n_scenes, true, fn);
+  if (n_max < 0) return 1;
+  const int total = offsets_host[n_scenes];
+  const bool given = verts_host != nullptr;
+  if (!rows_host || !nrows_host || (given && (!nverts_host || vmax < 1)))
+    return bp_fail("bp_scene_update_polytopes_batch: bad arguments");
+  if (total < 1) return bp_fail("bp_scene_update_polytopes_batch: a polytope scene batch needs at least one obstacle");
+  int vmax_new = 0;
+  for (int j = 0; j < total; ++j) {
+    if (nrows_host[j] < 1 || nrows_host[j] > BP_OBS_ROWS || (given && (nverts_host[j] < 1 || nverts_host[j] > vmax))) {
+      const int k = scene_of_obstacle(offsets_host, j);
+      snprintf(g_err, sizeof(g_err), "%s: scene %d, obstacle %d needs 1..15 rows%s", fn, k, j - offsets_host[k],
+               given ? " and 1..vmax vertices" : "");
+      return 1;
+    }
+    if (given && nverts_host[j] > vmax_new) vmax_new = nverts_host[j];
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int vin = given ? vmax : BP_ENUM_VMAX;           // vertex stride of the ingest's source
+  // staging, host and device: rows [total,15,4] | nrows [total] | offsets [n_scenes+1] | flags [2] | (given)
+  // verts [total,vmax,3] | nverts [total]; device only, when enumerating: V [total,64,3] | nv [total]
+  const size_t o_nrows = stage_align(sizeof(double) * (size_t)total * BP_OBS_ROWS * 4);
+  const size_t o_off = o_nrows + stage_align(sizeof(int) * (size_t)total);
+  const size_t o_flags = o_off + stage_align(sizeof(int) * (size_t)(n_scenes + 1));
+  const size_t o_verts = o_flags + stage_align(sizeof(int) * 2);
+  const size_t o_nverts = o_verts + stage_align(sizeof(double) * (size_t)total * vin * 3);
+  const size_t hbytes = given ? o_nverts + sizeof(int) * (size_t)total : o_verts;
+  const size_t dbytes = o_nverts + sizeof(int) * (size_t)total;
+  if (stage_reserve(scene, hbytes, dbytes)) return 1;
+  char* h = (char*)scene->stage_h;
+  char* d = (char*)scene->stage_d;
+  memcpy(h, rows_host, sizeof(double) * (size_t)total * BP_OBS_ROWS * 4);
+  memcpy(h + o_nrows, nrows_host, sizeof(int) * (size_t)total);
+  memcpy(h + o_off, offsets_host, sizeof(int) * (size_t)(n_scenes + 1));
+  int* flags_h = (int*)(h + o_flags);
+  flags_h[0] = 0x7fffffff;
+  flags_h[1] = 0;
+  if (given) {
+    memcpy(h + o_verts, verts_host, sizeof(double) * (size_t)total * vmax * 3);
+    memcpy(h + o_nverts, nverts_host, sizeof(int) * (size_t)total);
+  }
+  BP_CUDA(cudaMemcpyAsync(d, h, hbytes, cudaMemcpyHostToDevice, st));
+  if (!given) {
+    // enumerate into the staging and commit only when every obstacle is a polytope of at most 64 vertices
+    k_scene_enum_vertices<<<total, 128, 0, st>>>((const double*)d, (const int*)(d + o_nrows), BP_ENUM_VMAX,
+                                                 (double*)(d + o_verts), (int*)(d + o_nverts), (int*)(d + o_flags));
+    BP_CUDA(cudaGetLastError());
+    BP_CUDA(cudaMemcpyAsync(flags_h, d + o_flags, sizeof(int) * 2, cudaMemcpyDeviceToHost, st));
+    BP_CUDA(cudaStreamSynchronize(st));
+    if (flags_h[0] != 0x7fffffff) {
+      const int j = flags_h[0] / 2, k = scene_of_obstacle(offsets_host, j);
+      if (flags_h[0] & 1)
+        snprintf(g_err, sizeof(g_err), "%s: scene %d, obstacle %d has more than %d vertices", fn, k, j - offsets_host[k],
+                 BP_ENUM_VMAX);
+      else
+        snprintf(g_err, sizeof(g_err), "%s: scene %d, obstacle %d: Polyhedron is not a polytope", fn, k,
+                 j - offsets_host[k]);
+      return 1;
+    }
+    vmax_new = flags_h[1];
+  }
+  // buffers that have to grow: all allocated before anything is released
+  double *rows = scene->rows, *verts = scene->verts, *cols = scene->cols;
+  int *nrows = scene->nrows, *nverts = scene->nverts;
+  const int pcap = total > scene->pcap ? total : scene->pcap;
+  const size_t vneed = (size_t)total * vmax_new * 3, vcap = vneed > scene->vcap ? vneed : scene->vcap;
+  const int cap = total > scene->cap ? ((total + 31) / 32) * 32 : scene->cap;
+  cudaError_t e = cudaSuccess;
+  if (pcap != scene->pcap) {
+    rows = nullptr; nrows = nullptr; nverts = nullptr;
+    e = cudaMalloc(&rows, sizeof(double) * (size_t)pcap * BP_OBS_ROWS * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&nrows, sizeof(int) * (size_t)pcap);
+    if (e == cudaSuccess) e = cudaMalloc(&nverts, sizeof(int) * (size_t)pcap);
+  }
+  if (e == cudaSuccess && vcap != scene->vcap) { verts = nullptr; e = cudaMalloc(&verts, sizeof(double) * vcap); }
+  if (e == cudaSuccess && cap != scene->cap) { cols = nullptr; e = cudaMalloc(&cols, sizeof(double) * 6 * (size_t)cap); }
+  if (e == cudaSuccess) {
+    const double* vsrc = (const double*)(d + o_verts);
+    const int* nvsrc = (const int*)(d + o_nverts);
+    k_scene_ingest_polytopes<<<(cap + 7) / 8, 256, 0, st>>>(
+        (const double*)d, (const int*)(d + o_nrows), vsrc, nvsrc, vin, total, vmax_new, cap, 0.0, rows, nrows, verts,
+        nverts, cols, (const int*)(d + o_off), n_scenes, scene->seg_off);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);      // (the pinned staging is reused by the next update)
+  // release whichever of each pair is not kept: the new buffers on failure, the replaced ones on success
+  const bool ok = e == cudaSuccess;
+  if (rows != scene->rows) {
+    cudaFree(ok ? scene->rows : rows); cudaFree(ok ? scene->nrows : nrows); cudaFree(ok ? scene->nverts : nverts);
+  }
+  if (verts != scene->verts) cudaFree(ok ? scene->verts : verts);
+  if (cols != scene->cols) cudaFree(ok ? scene->cols : cols);
+  if (!ok) return bp_fail("bp_scene_update_polytopes_batch", e);
+  scene->rows = rows; scene->nrows = nrows; scene->nverts = nverts; scene->pcap = pcap;
+  scene->verts = verts; scene->vcap = vcap;
+  scene->cols = cols; scene->cap = cap;
+  scene->vmax = vmax_new;
+  scene->n = n_max;
+  memcpy(scene->seg_off_host, offsets_host, sizeof(int) * (size_t)(n_scenes + 1));
+  return 0;
+}
+
 int bp_scene_destroy(bp_scene* scene) {
   if (!scene) return 0;
+  if (scene->seg_off_host) free(scene->seg_off_host);
+  if (scene->stage_h) cudaFreeHost(scene->stage_h);
+  if (scene->stage_d) cudaFree(scene->stage_d);
   if (scene->seg_off) cudaFree(scene->seg_off);
   if (scene->rows) cudaFree(scene->rows);
   if (scene->nrows) cudaFree(scene->nrows);

@@ -7,6 +7,7 @@ float64 / int32 CUDA tensors.  Reference sites are cited per function.
 from __future__ import annotations
 
 import ctypes
+import time
 from dataclasses import dataclass
 
 import numpy as np
@@ -139,10 +140,60 @@ class PolytopeScene(Scene):
         raise _lib.BpGeoError("PolytopeScene is immutable: create a new one")
 
 
+def _concat_rows(arrays, width):
+    """Per-obstacle arrays of rows ([R_j, width], or [R_j] for width 1) -> (all rows back to back [sum R_j, width] as
+    float64, R_j [n]).  One concatenate when every array already has that shape, else a reshape per array."""
+    n = len(arrays)
+    if n == 0:
+        return np.zeros((0, width)), np.zeros(0, np.int64)
+    try:
+        flat = np.concatenate(arrays).astype(np.float64, copy=False)
+        if flat.ndim == (1 if width == 1 else 2) and (width == 1 or flat.shape[1] == width):
+            return flat.reshape(-1, width), np.fromiter(map(len, arrays), np.int64, n)
+    except ValueError:                                 # ragged ranks or widths
+        pass
+    arrays = [np.asarray(a, float).reshape(-1, width) for a in arrays]
+    return np.concatenate(arrays), np.fromiter((a.shape[0] for a in arrays), np.int64, n)
+
+
+def pack_polytope_rows(obs_sets, max_rows=PolytopeScene.MAX_ROWS):
+    """obs_sets ([A, b] per obstacle) -> (rows [n, 15, 4] (a0, a1, a2, b), nrows [n] int32) as PolytopeScene packs
+    them: the rows of nonzero norm in their order, then (0, 0, 0, 10).  Vectorised over all obstacles at once.
+    ValueError for an obstacle with more than 15 such rows or with another number of b's than rows."""
+    n = len(obs_sets)
+    A, counts = _concat_rows([s[0] for s in obs_sets], 3)
+    b, b_counts = _concat_rows([s[1] for s in obs_sets], 1)
+    if not np.array_equal(counts, b_counts):
+        raise ValueError("every obstacle needs one b per row of A")
+    rows = np.zeros((n, max_rows, 4))
+    rows[:, :, 3] = 10.0
+    obs = np.repeat(np.arange(n), counts)
+    nz = (A * A).sum(axis=1) > 0                       # (the sign of np.linalg.norm's sqrt(sum(a * a)))
+    nrows = np.bincount(obs[nz], minlength=n)
+    if (nrows > max_rows).any():
+        raise ValueError(f"obstacle {int(np.argmax(nrows > max_rows))} has more than {max_rows} rows")
+    o = obs[nz]
+    start = np.cumsum(nrows) - nrows                   # first kept row of every obstacle among all kept rows
+    rows.reshape(-1, 4)[o * max_rows + np.arange(o.shape[0]) - start[o]] = np.hstack((A[nz], b[nz]))
+    return rows, nrows.astype(np.int32)
+
+
+def pack_vertices(obs_points_sets):
+    """Vertex lists ([V_j, 3] per obstacle) -> (verts [n, vmax, 3] zero-padded, nverts [n] int32, vmax = the largest
+    V_j), as PolytopeScene packs them."""
+    n = len(obs_points_sets)
+    pts, nverts = _concat_rows(list(obs_points_sets), 3)
+    vmax = int(nverts.max()) if n else 0
+    verts = np.zeros((n, vmax, 3))
+    obs = np.repeat(np.arange(n), nverts)
+    verts.reshape(-1, 3)[obs * vmax + np.arange(obs.shape[0]) - (np.cumsum(nverts) - nverts)[obs]] = pts
+    return verts, nverts.astype(np.int32), vmax
+
+
 class PolytopeSceneBatch(PolytopeScene):
     """Several polytope scenes stored back to back in HBM (one per planning query): ``scenes`` is a list of
     (obs_sets, obs_points_sets | None) pairs.  Use with build_sets_point / build_sets_line / sample_filter and
-    ``item_scene`` = scene index of every seed / segment."""
+    ``item_scene`` = scene index of every seed / segment.  ``update_scenes`` moves the obstacles in place."""
 
     def __init__(self, scenes_list):
         from .utils import obstacle_points_sets
@@ -155,6 +206,44 @@ class PolytopeSceneBatch(PolytopeScene):
             pts.extend(obs_points)
             offs.append(len(sets))
         super().__init__(sets, pts, _offsets=offs)
+
+    def update_scenes(self, scenes_list):
+        """Replace every scene's obstacles (the constructor's format, as many scenes as the batch has) in place: one
+        staging copy and a short kernel chain (bp_scene_update_polytopes_batch), the same device contents as a new
+        PolytopeSceneBatch of scenes_list.  Scenes without vertex lists have them enumerated on the device when no
+        scene carries any, else here like the constructor does.  On failure the batch is left as it was.
+        ``pack_seconds``: the host time of the packing (everything before the library call); ``update_events``: CUDA
+        events recorded on the current stream around the library call (staging copy, kernels, synchronisation)."""
+        from .utils import obstacle_points_sets
+
+        t0 = time.perf_counter()
+        if len(scenes_list) != self.n_scenes:
+            raise ValueError(f"{len(scenes_list)} scenes for a batch of {self.n_scenes}")
+        sets, offs = [], np.zeros(len(scenes_list) + 1, np.int32)
+        for k, (obs_sets, _) in enumerate(scenes_list):
+            sets.extend(obs_sets)
+            offs[k + 1] = len(sets)
+        rows, nrows = pack_polytope_rows(sets)
+        ip = ctypes.POINTER(ctypes.c_int)
+        verts = nverts = None
+        vmax = 0
+        if any(pts is not None for _, pts in scenes_list):
+            pts = []
+            for obs_sets, obs_points in scenes_list:
+                pts.extend(obs_points if obs_points is not None else obstacle_points_sets(obs_sets))
+            if len(pts) != len(sets):
+                raise ValueError("PolytopeScene needs one vertex array per obstacle set")
+            verts, nverts, vmax = pack_vertices(pts)
+        self.pack_seconds = time.perf_counter() - t0
+        self.update_events = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+        self.update_events[0].record()
+        check(self._lib.bp_scene_update_polytopes_batch(
+            self._h, rows.ctypes.data_as(_dp), nrows.ctypes.data_as(ip),
+            verts.ctypes.data_as(_dp) if verts is not None else None,
+            nverts.ctypes.data_as(ip) if nverts is not None else None, offs.ctypes.data_as(ip), len(scenes_list),
+            vmax, _stream()))
+        self.update_events[1].record()
+        self.n = int(np.diff(offs).max())
 
 
 class SceneBatch(Scene):
@@ -178,6 +267,28 @@ class SceneBatch(Scene):
 
     def update(self, boxes, inflate=None):
         raise _lib.BpGeoError("SceneBatch is immutable")
+
+    def update_scenes(self, boxes_list):
+        """Replace every scene's boxes (the constructor's format, as many scenes as the batch has; counts may change,
+        down to 0) in place, with the batch's inflate: one staging copy and one kernel (bp_scene_update_batch), the
+        same device contents as a new SceneBatch of boxes_list.  On failure the batch is left as it was.
+        ``pack_seconds``: the host time of the packing (everything before the library call); ``update_events``: CUDA
+        events recorded on the current stream around the library call (staging copy, kernels, synchronisation)."""
+        t0 = time.perf_counter()
+        if len(boxes_list) != self.n_scenes:
+            raise ValueError(f"{len(boxes_list)} scenes for a batch of {self.n_scenes}")
+        boxes_list = [np.asarray(bx, dtype=np.float64).reshape(-1, 6) for bx in boxes_list]
+        offs = np.zeros(len(boxes_list) + 1, dtype=np.int32)
+        offs[1:] = np.cumsum([bx.shape[0] for bx in boxes_list])
+        boxes = np.ascontiguousarray(np.vstack(boxes_list))
+        self.pack_seconds = time.perf_counter() - t0
+        self.update_events = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+        self.update_events[0].record()
+        check(self._lib.bp_scene_update_batch(self._h, boxes.ctypes.data_as(_dp),
+                                              offs.ctypes.data_as(ctypes.POINTER(ctypes.c_int)), len(boxes_list),
+                                              self.inflate, _stream()))
+        self.update_events[1].record()
+        self.n = int(np.diff(offs).max())
 
 
 @dataclass

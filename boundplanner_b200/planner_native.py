@@ -16,6 +16,7 @@ import numpy as np
 
 MAX_NODES, NODE_ROWS, SET_ROWS, MAX_PATH, FIT_SAMPLES = 64, 24, 48, 64, 20
 OBS_ROWS = 15               # rows of a polytope obstacle (normalize_set_size)
+MAX_POLY_OBSTACLES = 16384  # polytope obstacles per scene (the kernels of a planning round)
 MAX_PREV_SETS = 64          # previous sets per query (sets_via_prev)
 LENGTH_EE = 0.05            # BoundPlanner.__init__ (:54)
 
@@ -280,14 +281,15 @@ class NativePlanner:
     """A batch of independent planning queries, one scene each, planned in lock step by libbpgeo's native driver.
     The queries carry boxes (``obstacles``) or polytopes (``obs_sets`` [, ``obs_points_sets``]), all of one kind.
     The scene batch and the device tables are created once; ``run`` can be called again (same scenes), also with
-    new per-query inputs (``queries=``: an MPC loop's replanning calls) over the same obstacles."""
+    new per-query inputs (``queries=``: an MPC loop's replanning calls) over the same obstacles.  When the obstacles
+    move, ``update_obstacles`` rewrites the resident scenes in place."""
 
     def __init__(self, queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0)):
         import torch
 
         from . import _lib
 
-        query_kind(queries)                      # (a mixed batch fails before anything touches the device)
+        self.kind = query_kind(queries)          # (a mixed batch fails before anything touches the device)
         if not torch.cuda.is_available():
             raise _lib.BpGeoError("boundplanner_b200 needs a CUDA device (no CPU fallback)")
         self._lib = _lib.load()
@@ -299,6 +301,28 @@ class NativePlanner:
         self._packed = {}
         _lib.check(self._lib.bp_plan_create(self.scene._h, len(queries), ctypes.byref(self._h)))
 
+    def update_obstacles(self, queries):
+        """Move the obstacles: the scenes become those of ``queries`` (the constructor's format, as many queries, the
+        same obstacle kind; ValueError before the device is touched otherwise), written into the resident scene batch
+        in place (SceneBatch / PolytopeSceneBatch.update_scenes), and ``queries`` become the planner's queries.
+        ``run()`` and ``run(queries=...)`` then plan against the new obstacles.  A failed update leaves the planner
+        as it was."""
+        if len(queries) != len(self.queries):
+            raise ValueError(f"{len(queries)} queries for a planner of {len(self.queries)} scenes")
+        kind = query_kind(queries)
+        if kind != self.kind:
+            raise ValueError(f"the planner's scenes hold {self.kind}, the queries {kind}")
+        if kind == "polytopes":
+            n_max = max(len(q["obs_sets"]) for q in queries)
+            if n_max > MAX_POLY_OBSTACLES:
+                raise ValueError(f"polytope scenes hold at most {MAX_POLY_OBSTACLES} obstacles (largest scene: {n_max})")
+            self.scene.update_scenes([(q["obs_sets"], q.get("obs_points_sets")) for q in queries])
+        else:
+            self.scene.update_scenes([q["obstacles"] for q in queries])
+        self.queries = queries
+        self._packed = {}
+        self._obstacles = None
+
     @staticmethod
     def _obstacles_of(pk):
         return pk.kind, pk.box_off, pk.boxes if pk.obs_rows is None else pk.obs_rows
@@ -306,8 +330,8 @@ class NativePlanner:
     def run(self, rng_seeds=None, sample_chunk=32, want_nodes=True, queries=None):
         """Plan the batch: (results, stats).  queries: new per-query inputs (start, end, r0, r1, first_sample and the
         replanning keys of planner.plan_batch) to plan against the scenes of this planner; their obstacles must be
-        the ones it was created with (ValueError otherwise: the host push-out of `end` and the device scene must
-        agree)."""
+        the ones it was created with, or last updated to (ValueError otherwise: the host push-out of `end` and the
+        device scene must agree)."""
         if queries is not None:
             if len(queries) != len(self.queries):
                 raise ValueError(f"{len(queries)} queries for a planner of {len(self.queries)} scenes")

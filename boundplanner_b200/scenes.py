@@ -180,3 +180,32 @@ def polytope_free_points(n, obs_sets, margin, rng, ws_min=WORKSPACE_MIN, ws_max=
         cand = cand[(viol.max(axis=2) >= margin).all(axis=1)]
         out = np.vstack((out, cand))
     return np.ascontiguousarray(out[:n])
+
+
+def moved_obstacles(obstacles, rng, obs_points=None, move_frac=0.25, max_shift=0.05, n_add=4, n_remove=4):
+    """One step of moving obstacles (an MPC loop's changing scene), seeded by ``rng``: a fraction ``move_frac`` of
+    the obstacles is translated by U[-max_shift, max_shift]^3 each, ``n_remove`` are removed and ``n_add`` new ones
+    (C3-sized: edges U[0.05, 0.2]) are appended.
+    Boxes: ``obstacles`` [N,6] -> [N',6].  Polytopes: ``obstacles`` = obs_sets and ``obs_points`` = obs_points_sets
+    (or None) -> (obs_sets', obs_points_sets' or None); a translation by t sets b += A t and vertices += t (padded rows,
+    A = 0, keep b = 10)."""
+    poly = not isinstance(obstacles, np.ndarray)
+    n = len(obstacles)
+    moved = rng.random(n) < move_frac
+    shift = rng.uniform(-max_shift, max_shift, (n, 3))
+    keep = np.sort(rng.permutation(n)[: max(n - n_remove, 0)])
+    if not poly:
+        out = obstacles + np.where(moved[:, None], np.hstack((shift, shift)), 0.0)
+        return np.vstack((out[keep], random_box_scene(n_add, rng, 0.05, 0.2)))
+    sets, pts = [], [] if obs_points is not None else None
+    for j in keep:
+        A, b = np.asarray(obstacles[j][0], float), np.asarray(obstacles[j][1], float)
+        t = shift[j] if moved[j] else np.zeros(3)
+        sets.append([A.copy(), b + A @ t])
+        if pts is not None:
+            pts.append(np.asarray(obs_points[j], float) + t)
+    new_sets, new_pts = random_polytope_scene(n_add, rng, 0.05, 0.2)
+    sets.extend(new_sets)
+    if pts is not None:
+        pts.extend(new_pts)
+    return sets, pts

@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define BPGEO_ABI_VERSION 4
+#define BPGEO_ABI_VERSION 5
 #define BP_MAX_ROWS 48 /* hard cap on rows per convex set (reference MVIE cap: 20, quirk Q5) */
 
 typedef struct bp_scene bp_scene;
@@ -68,6 +68,21 @@ int bp_scene_create_polytopes_batch(const double* rows_host, const int* nrows_ho
                                     const int* nverts_host, const int* offsets_host /*[n_scenes+1]*/, int n_scenes,
                                     int vmax, bp_scene** out);
 int bp_scene_update(bp_scene* scene, const double* boxes_host, int n, double inflate, void* stream);
+/* Rewrite a resident scene batch in place with new obstacles (ABI 5; an MPC loop whose obstacles move): the inputs of
+ * the matching *_create_*batch, n_scenes equal to the batch's, the per-scene obstacle counts free to change (boxes:
+ * down to 0; polytopes: at least one obstacle in all).  One host-to-device copy of the packed inputs through a staging
+ * buffer owned by the scene (pinned host + device, grown on demand), a short kernel chain on `stream` that writes the
+ * same bits as a freshly created batch, and a synchronisation of `stream` at the end; work on other streams that reads
+ * the scene must have finished.  verts_host NULL: the vertices are enumerated on the device (bp_polytope_vertices, at
+ * most 64 per obstacle, from the given rows) and vmax is ignored; vmax becomes the largest vertex count either way.
+ * All or nothing: a wrong kind of batch, another n_scenes, decreasing offsets, an obstacle without 1..15 rows (or
+ * 1..vmax vertices), a failed allocation or an enumerated obstacle that is not a polytope or has more than 64 vertices
+ * fail the call and leave the scene as it was. */
+int bp_scene_update_batch(bp_scene* scene, const double* boxes_host, const int* offsets_host /*[n_scenes+1]*/,
+                          int n_scenes, double inflate, void* stream);
+int bp_scene_update_polytopes_batch(bp_scene* scene, const double* rows_host, const int* nrows_host,
+                                    const double* verts_host /*NULL: enumerate*/, const int* nverts_host,
+                                    const int* offsets_host /*[n_scenes+1]*/, int n_scenes, int vmax, void* stream);
 int bp_scene_destroy(bp_scene* scene);
 int bp_scene_size(const bp_scene* scene);
 
@@ -378,7 +393,9 @@ typedef struct {
 } bp_plan_out;
 
 /* bp_plan_create takes a box or a polytope scene batch with one scene per query; the per-scene limits of the kernels
- * the rounds launch are checked here, not in the middle of a run (polytope scenes: at most 16384 obstacles). */
+ * the rounds launch are checked here, not in the middle of a run (polytope scenes: at most 16384 obstacles).  The plan
+ * keeps the scene batch, not a copy: after bp_scene_update_batch / bp_scene_update_polytopes_batch, bp_plan_run plans
+ * against the new obstacles, checks its inputs against the batch's current offsets and re-checks the limit. */
 typedef struct bp_plan bp_plan;
 int bp_plan_create(const bp_scene* scene_batch, int Q, bp_plan** out);
 int bp_plan_run(bp_plan* plan, const bp_plan_in* in, bp_plan_out* out, void* stream);

@@ -10,8 +10,7 @@
 // statement of the loop and the thing this file is tested against (same paths, set sequences and via points).
 // bpplan::run_lockstep advances all queries of a batch together: every round it collects the pending request of
 // every live query, hands them to an Executor by KIND (one batched kernel chain per kind on the GPU executor of
-// bpgeo.cu; callbacks into the test harnesses tests/host_harness.cpp and tests/host_harness_replan.cpp), and resumes
-// the queries.
+// bpgeo.cu; callbacks into the test harness tests/host_harness.cpp), and resumes the queries.
 // What is NOT here (as in planner.py): the final via-point NLP with rotations (Ipopt, :540-555).
 #pragma once
 #include <algorithm>

@@ -169,8 +169,8 @@ void hh_fk_kin(const double* q, const double* dq, int n, double* T_ee, double* j
 double hh_min_eig(const double* A) { return bp_sym3_min_eig(A); }
 
 
-// ---- the native lock-step planner driver (csrc/bp_planner.h) with its requests answered by callbacks: the CPU
-// test plugs the oracle in and compares with the Python planner (tests/test_planner_native.py) ----
+// ---- the native lock-step planner driver (csrc/bp_planner.h) with every request kind answered by callbacks: the
+// CPU tests plug the oracle in and compare with the Python planner (tests/util.py: run_native_with_oracle) ----
 typedef int (*hh_cb_set)(int qid, const bpplan::SetReq* req, int n_nodes, const bpplan::Node* nodes, bpplan::SetAns* out);
 typedef int (*hh_cb_edges)(int qid, int id_new, int n_nodes, const bpplan::Node* nodes, const int* has_target,
                            const double* xd, bpplan::EdgeAns* out);
@@ -178,13 +178,14 @@ typedef int (*hh_cb_project)(int qid, int id0, int id1, const double* xd, int n_
                              bpplan::ProjAns* out);
 typedef int (*hh_cb_path)(int qid, int n_nodes, const int* edge_off, const int* edge_dst, const double* edge_w,
                           int* path_out, int* path_len);
+// reduce_ineqs of a given set (the start fallback's previous end set): fills out->m_red, Ar, br
+typedef int (*hh_cb_reduce)(int qid, const bpplan::ReduceReq* req, bpplan::SetAns* out);
 
 struct HhCallbackExecutor : bpplan::Executor {
-  hh_cb_set cb_set; hh_cb_edges cb_edges; hh_cb_project cb_project; hh_cb_path cb_path;
-  int commits = 0;
+  hh_cb_set cb_set; hh_cb_edges cb_edges; hh_cb_project cb_project; hh_cb_path cb_path; hh_cb_reduce cb_reduce;
   int n_lanes = 1;
   int lanes() const override { return n_lanes; }
-  void commit_node(int, int, int, const bpplan::Node&) override { ++commits; }
+  void commit_node(int, int, int, const bpplan::Node&) override {}
   int collect(int, bpplan::Round&) override { return 0; }
   int submit(int, bpplan::Round& r, const std::vector<bpplan::Query>& qs) override {
     for (size_t k = 0; k < r.sets.size(); ++k) {
@@ -209,17 +210,26 @@ struct HhCallbackExecutor : bpplan::Executor {
       if (int rc = cb_path(r.paths[k].qid, r.paths[k].n_nodes, r.edge_off.data() + n0, r.edge_dst.data(), r.edge_w.data(),
                            r.path_out.data() + k * (size_t)bpplan::MAX_PATH, &r.path_len[k])) return rc;
     }
+    for (size_t k = 0; k < r.reduces.size(); ++k)
+      if (int rc = cb_reduce(r.reduces[k].qid, &r.reduces[k], &r.reduce_ans[k])) return rc;
     return 0;
   }
 };
 
+// the driver as bp_plan_run runs it: returns 3 (and err_msg[0] = the reason) when check_replan_inputs rejects the
+// replanning inputs, before any callback runs
 int hh_plan_batch(const bp_plan_in* in, bp_plan_out* out, hh_cb_set cb_set, hh_cb_edges cb_edges,
-                  hh_cb_project cb_project, hh_cb_path cb_path, int lanes) {
+                  hh_cb_project cb_project, hh_cb_path cb_path, hh_cb_reduce cb_reduce, int lanes) {
+  const std::string bad = bpplan::check_replan_inputs(*in);
+  if (!bad.empty()) {
+    std::snprintf(out->err_msg, 160, "%s", bad.c_str());
+    return 3;
+  }
   bpplan::Params par;
   std::vector<bpplan::Query> qs;
   bpplan::load_queries(*in, par, qs);
   HhCallbackExecutor ex;
-  ex.cb_set = cb_set; ex.cb_edges = cb_edges; ex.cb_project = cb_project; ex.cb_path = cb_path;
+  ex.cb_set = cb_set; ex.cb_edges = cb_edges; ex.cb_project = cb_project; ex.cb_path = cb_path; ex.cb_reduce = cb_reduce;
   ex.n_lanes = lanes > 0 ? lanes : 1;
   bpplan::RunStats st;
   std::vector<int> fin(qs.size(), -1);
@@ -238,9 +248,20 @@ void hh_pcg64_uniform3(unsigned long long* state4, const double* lo, const doubl
   g.uniform3(lo, range, n, out);
   g.get((uint64_t*)state4);
 }
+
+// sizes of the records the Python side mirrors with ctypes
 int hh_sizeof(int what) {
-  return what == 0 ? (int)sizeof(bpplan::SetReq) : what == 1 ? (int)sizeof(bpplan::SetAns) : what == 2 ? (int)sizeof(bpplan::Node)
-       : what == 3 ? (int)sizeof(bpplan::EdgeAns) : what == 4 ? (int)sizeof(bpplan::ProjAns) : -1;
+  switch (what) {
+    case 0: return (int)sizeof(bpplan::SetReq);
+    case 1: return (int)sizeof(bpplan::SetAns);
+    case 2: return (int)sizeof(bpplan::Node);
+    case 3: return (int)sizeof(bpplan::EdgeAns);
+    case 4: return (int)sizeof(bpplan::ProjAns);
+    case 5: return (int)sizeof(bpplan::ReduceReq);
+    case 6: return (int)sizeof(bp_plan_in);
+    case 7: return (int)sizeof(bp_plan_out);
+    default: return -1;
+  }
 }
 
 }  // extern "C"

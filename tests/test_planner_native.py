@@ -4,249 +4,26 @@ with its requests answered by callbacks into the oracle -- the same answers the 
 sequences, via points, graph sizes, error exits and the generator state after the query must agree exactly.
 GPU: ``bp_plan_batch`` (requests answered by the kernels) against ``planner.plan_batch`` on the same kernels."""
 import ctypes
-import re
 
-import networkx as nx
 import numpy as np
 import pytest
 from scipy.spatial.transform import Rotation as R
 
 from boundplanner_b200 import planner_native as pn
 from boundplanner_b200 import scenes
-from boundplanner_b200.planner import SetSequencePlanner
-from tests.util import OracleBackend
+from tests.util import (R0, EdgeAns, MemoBackend, Node, ProjAns, ReduceReq, SetAns, SetReq, _dp, assert_same_result,
+                        python_plan, run_native_with_oracle)
 
-R0 = R.from_euler("XYZ", [0, 90, 0], degrees=True).as_matrix()
 R1 = R.from_euler("XYZ", [20, 70, -30], degrees=True).as_matrix()
-_dp = ctypes.POINTER(ctypes.c_double)
-_ip = ctypes.POINTER(ctypes.c_int)
-
-
-class SetReq(ctypes.Structure):
-    _fields_ = [("qid", ctypes.c_int), ("kind", ctypes.c_int), ("fixed_mid", ctypes.c_int), ("optimize", ctypes.c_int),
-                ("with_dv", ctypes.c_int), ("n_cand", ctypes.c_int), ("p0", ctypes.c_double * 3),
-                ("p1", ctypes.c_double * 3), ("cand", _dp)]
-
-
-class SetAns(ctypes.Structure):
-    _fields_ = [("status", ctypes.c_int), ("rows_peak", ctypes.c_int), ("m", ctypes.c_int), ("m_red", ctypes.c_int),
-                ("collision", ctypes.c_int), ("first", ctypes.c_int), ("dv", ctypes.c_double),
-                ("A", ctypes.c_double * (pn.SET_ROWS * 3)), ("b", ctypes.c_double * pn.SET_ROWS),
-                ("Ar", ctypes.c_double * (pn.SET_ROWS * 3)), ("br", ctypes.c_double * pn.SET_ROWS),
-                ("Q", ctypes.c_double * 9), ("P", ctypes.c_double * 3)]
-
-
-class Node(ctypes.Structure):
-    _fields_ = [("m", ctypes.c_int), ("A", ctypes.c_double * (pn.NODE_ROWS * 3)), ("b", ctypes.c_double * pn.NODE_ROWS),
-                ("Q", ctypes.c_double * 9), ("P", ctypes.c_double * 3), ("size", ctypes.c_double),
-                ("c_size", ctypes.c_double)]
-
-
-class EdgeAns(ctypes.Structure):
-    _fields_ = [("ok", ctypes.c_int), ("fits", ctypes.c_int), ("x", ctypes.c_double * 3), ("omega", ctypes.c_double),
-                ("proj_ok", ctypes.c_int), ("proj", ctypes.c_double * 3)]
-
-
-class ProjAns(ctypes.Structure):
-    _fields_ = [("x", ctypes.c_double * 3), ("status", ctypes.c_int)]
-
-
-CB_SET = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_int, ctypes.POINTER(SetReq), ctypes.c_int, ctypes.POINTER(Node),
-                          ctypes.POINTER(SetAns))
-CB_EDGES = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.POINTER(Node), _ip, _dp,
-                            ctypes.POINTER(EdgeAns))
-CB_PROJECT = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, _dp, ctypes.c_int,
-                              ctypes.POINTER(Node), ctypes.POINTER(ProjAns))
-CB_PATH = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_int, ctypes.c_int, _ip, _ip, _dp, _ip, _ip)
-
-
-class MemoBackend(OracleBackend):
-    """OracleBackend with its answers memoised by request content: the Python planner and the native driver ask
-    the same questions, the oracle answers each once."""
-
-    def __init__(self, *a):
-        super().__init__(*a)
-        self.memo = {}
-
-    @staticmethod
-    def _key(x):
-        if isinstance(x, np.ndarray):
-            return x.tobytes()
-        if isinstance(x, (list, tuple)):
-            return tuple(MemoBackend._key(v) for v in x)
-        if isinstance(x, (float, np.floating)):
-            return float(x)
-        return x
-
-    def execute(self, req):
-        k = self._key(req)
-        if k not in self.memo:
-            try:
-                self.memo[k] = super().execute(req)
-            except (RuntimeError, ValueError) as e:
-                self.memo[k] = e
-        ans = self.memo[k]
-        if isinstance(ans, Exception):
-            raise ans
-        return ans
-
-
-def _node_set(nd):
-    m = nd.m
-    return [np.array(nd.A[: 3 * m]).reshape(m, 3), np.array(nd.b[:m])]
-
-
-def _fill_set(out, ans, with_line):
-    if with_line:
-        A, b, Q, p, coll, Ar, br = ans
-        out.collision = int(bool(coll))
-    else:
-        A, b, Q, p, Ar, br = ans[:6]
-    m, mr = A.shape[0], Ar.shape[0]
-    assert m <= pn.SET_ROWS
-    out.status, out.m, out.m_red, out.rows_peak = 0, m, mr, m
-    out.A[: 3 * m] = A.reshape(-1).tolist()
-    out.b[:m] = b.tolist()
-    out.Ar[: 3 * mr] = Ar.reshape(-1).tolist()
-    out.br[:mr] = br.tolist()
-    out.Q[:] = np.asarray(Q).reshape(-1).tolist()
-    out.P[:] = np.asarray(p).reshape(-1).tolist()
-
-
-def _error_status(e, out):
-    msg = str(e)
-    if "Ellipse violates" in msg:
-        out.status = 1
-    elif "could not broadcast" in msg:
-        out.status, out.rows_peak, out.m = 5, int(re.search(r"shape \((\d+),\)", msg).group(1)), 0
-        out.m = out.rows_peak
-    else:
-        raise e
-
-
-def run_native_with_oracle(host_harness, queries, inflate, ws_max, ws_min, seeds, backends, sample_chunk=32, lanes=1):
-    pk = pn.PackedQueries(queries, inflate, ws_max, ws_min, seeds, sample_chunk)
-    helpers = [SetSequencePlanner(q["obstacles"], inflate, list(ws_max), list(ws_min), backend=backends[i],
-                                  obs_sets=backends[i].obs_sets) for i, q in enumerate(queries)]
-    ee = []
-    for q in queries:
-        omega = R.from_matrix(q["r1"] @ q["r0"].T).as_rotvec()
-        on = np.linalg.norm(omega)
-        ee.append((q["r0"] @ np.array([-0.05, 0, 0]), omega / on if on > 1e-6 else np.array([0, 0, 1.0]), on))
-    errors = []
-
-    def in_safe(nodes, n, x):
-        return any(np.max(_node_set(nodes[k])[0] @ x - _node_set(nodes[k])[1]) < 1e-3 for k in range(n))
-
-    def dvertex(nodes, n, Q, p):
-        if n == 0:
-            return np.inf
-        return min(np.linalg.norm(np.array(nodes[k].Q[:]).reshape(3, 3) - Q) + np.linalg.norm(np.array(nodes[k].P[:]) - p)
-                   for k in range(n))
-
-    def cb_set(qid, req, n_nodes, nodes, out):
-        try:
-            r, o = req.contents, out.contents
-            o.first, o.dv, o.collision = 0, np.inf, 0
-            p0 = np.array(r.p0[:])
-            if r.kind == 1:
-                try:
-                    _fill_set(o, backends[qid].execute(("set_line", p0, np.array(r.p1[:]))), True)
-                except (RuntimeError, ValueError) as e:
-                    _error_status(e, o)
-                return 0
-            if r.kind == 2:
-                cand = np.ctypeslib.as_array(r.cand, shape=(r.n_cand, 3)).copy()
-                o.first = -1
-                for i, c in enumerate(cand):
-                    if not helpers[qid]._in_collision(c) and not in_safe(nodes, n_nodes, c):
-                        o.first, p0 = i, c
-                        break
-                if o.first < 0:
-                    return 0
-            try:
-                ans = backends[qid].execute(("set_point", p0, bool(r.fixed_mid), bool(r.optimize)))
-            except (RuntimeError, ValueError) as e:
-                _error_status(e, o)
-                return 0
-            _fill_set(o, ans, False)
-            if r.with_dv:
-                o.dv = dvertex(nodes, n_nodes, ans[2], ans[3])
-            return 0
-        except Exception as e:                               # noqa: BLE001 -- surfaces in the test below
-            errors.append(e)
-            return 7
-
-    def cb_edges(qid, id_new, n_nodes, nodes, has_target, xd, out):
-        try:
-            others = [_node_set(nodes[k]) for k in range(id_new)]
-            new = _node_set(nodes[id_new])
-            res = backends[qid].execute(("edges", others, new, 0.01, ee[qid]))
-            for k, (x, ok, fits, via) in enumerate(res):
-                out[k].ok, out[k].fits, out[k].proj_ok = int(bool(ok)), int(bool(fits)), 0
-                if ok:
-                    out[k].x[:] = np.asarray(x).tolist()
-                    out[k].omega = float(via[3]) if fits else -1.0
-                    if has_target[k]:                         # the hit's projection, asked for with the edges
-                        pr = backends[qid].execute(("project", np.concatenate((others[k][0], new[0])),
-                                                    np.concatenate((others[k][1], new[1])),
-                                                    np.array([xd[3 * k], xd[3 * k + 1], xd[3 * k + 2]])))
-                        out[k].proj[:] = np.asarray(pr).tolist()
-                        out[k].proj_ok = 1
-            return 0
-        except Exception as e:                               # noqa: BLE001
-            errors.append(e)
-            return 7
-
-    def cb_project(qid, id0, id1, xd, n_nodes, nodes, out):
-        try:
-            s0, s1 = _node_set(nodes[id0]), _node_set(nodes[id1])
-            x = backends[qid].execute(("project", np.concatenate((s0[0], s1[0])), np.concatenate((s0[1], s1[1])),
-                                       np.array([xd[0], xd[1], xd[2]])))
-            out.contents.x[:] = np.asarray(x).tolist()
-            return 0
-        except Exception as e:                               # noqa: BLE001
-            errors.append(e)
-            return 7
-
-    def cb_path(qid, n, edge_off, edge_dst, edge_w, path_out, path_len):
-        try:
-            g = nx.Graph()
-            g.add_nodes_from(range(n))
-            for v in range(n):                                # adjacency dicts in the driver's insertion order
-                for e in range(edge_off[v], edge_off[v + 1]):
-                    g._adj[v][edge_dst[e]] = {"weight": edge_w[e]}
-            p = nx.shortest_path(g, 0, 1, weight="weight")
-            path_len[0] = len(p)
-            for k, v in enumerate(p[: pn.MAX_PATH]):
-                path_out[k] = v
-            return 0
-        except Exception as e:                               # noqa: BLE001
-            errors.append(e)
-            return 7
-
-    cbs = (CB_SET(cb_set), CB_EDGES(cb_edges), CB_PROJECT(cb_project), CB_PATH(cb_path))
-    host_harness.hh_plan_batch.restype = ctypes.c_int
-    rc = host_harness.hh_plan_batch(ctypes.byref(pk.inp), ctypes.byref(pk.out), *cbs, int(lanes))
-    assert not errors, errors[0]
-    assert rc == 0
-    return pk
-
-
-def _python_plan(query, inflate, ws_max, ws_min, seed, backend):
-    pl = SetSequencePlanner(query["obstacles"], inflate, list(ws_max), list(ws_min), backend=backend,
-                            rng=np.random.default_rng(seed), obs_sets=backend.obs_sets)
-    try:
-        res = pl.plan_set_sequence(query["start"].copy(), query["end"].copy(), query["r0"], query["r1"],
-                                   query.get("first_sample"))
-    except (RuntimeError, ValueError) as e:
-        res = e
-    return res, pl
 
 
 def test_struct_layouts(host_harness):
-    for k, t in enumerate((SetReq, SetAns, Node, EdgeAns, ProjAns)):
+    """The ctypes mirrors have the sizes of the C records (hh_sizeof), and the last fields of bp_plan_in / bp_plan_out
+    end their records."""
+    for k, t in enumerate((SetReq, SetAns, Node, EdgeAns, ProjAns, ReduceReq, pn.BpPlanIn, pn.BpPlanOut)):
         assert host_harness.hh_sizeof(k) == ctypes.sizeof(t), t.__name__
+    assert pn.BpPlanIn.prev_rows.offset + ctypes.sizeof(_dp) == ctypes.sizeof(pn.BpPlanIn)
+    assert pn.BpPlanOut.p_horizon_max.offset + ctypes.sizeof(_dp) == ctypes.sizeof(pn.BpPlanOut)
 
 
 def test_pcg64_stream_is_numpys(host_harness):
@@ -297,23 +74,12 @@ def test_native_driver_equals_python_planner_on_cpu(host_harness):
 def _check(host_harness, queries, inflate, ws_max, ws_min, seeds, chunk, lanes=1, backends=None):
     if backends is None:
         backends = [MemoBackend(q["obstacles"], inflate, ws_max, ws_min) for q in queries]
-    want = [_python_plan(q, inflate, ws_max, ws_min, s, be) for q, s, be in zip(queries, seeds, backends)]
+    want = [python_plan(q, inflate, ws_max, ws_min, s, be) for q, s, be in zip(queries, seeds, backends)]
     pk = run_native_with_oracle(host_harness, queries, inflate, ws_max, ws_min, seeds, backends, sample_chunk=chunk,
                                 lanes=lanes)
     pk.backends = backends
-    got = pk.results()
-    for i, ((w, pl), g) in enumerate(zip(want, got)):
-        if isinstance(w, Exception):
-            assert isinstance(g, Exception), f"query {i}: native planned, python raised {w!r}"
-            assert type(g) is type(w) and str(g).split("(")[0] == str(w).split("(")[0], (i, g, w)
-        else:
-            assert not isinstance(g, Exception), f"query {i}: {g!r}"
-            assert g["path"] == w["path"] and g["set_ids"] == w["set_ids"], i
-            assert np.array_equal(g["p_via"], w["p_via"]), i
-            assert g["n_nodes"] == w["graph"].number_of_nodes() and g["n_inter"] == w["inter_graph"].number_of_nodes()
-            assert g["n_edges"] == w["inter_graph"].number_of_edges()
-            for (ga, gb), (wa, wb) in zip(g["sets_via"], w["sets_via"]):
-                assert np.array_equal(ga, wa) and np.array_equal(gb, wb)
+    for i, ((w, pl), g) in enumerate(zip(want, pk.results())):
+        assert_same_result(g, w, pl, i)
         assert [int(v) for v in pk.rng_out[i]] == pn.rng_state_words(pl.rng), f"query {i}: generator state"
     return pk
 

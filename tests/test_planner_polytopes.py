@@ -8,35 +8,15 @@ GPU: bp_plan_run over a polytope scene batch against planner.plan_batch; plan_se
 against the oracle backend; boxes handed over as polytopes against the same boxes; the kind checks."""
 import ctypes
 
-import networkx as nx
 import numpy as np
 import pytest
-from scipy.spatial.transform import Rotation as R
 
 from boundplanner_b200 import planner_native as pn
 from boundplanner_b200 import scenes
 from boundplanner_b200.planner import SetSequencePlanner
-from tests.test_planner_native import (CB_EDGES, CB_PATH, CB_PROJECT, CB_SET, MemoBackend, _error_status, _fill_set,
-                                       _node_set)
+from tests.util import R0, PolytopeOracleBackend, _c3_poly, assert_same_result, python_plan, run_native_with_oracle
 
-R0 = R.from_euler("XYZ", [0, 90, 0], degrees=True).as_matrix()
 ORDER_TOL = 1e-15          # general push-out vs the reference's `@` (BLAS may fuse): last bits only
-
-
-class PolytopeOracleBackend(MemoBackend):
-    """The oracle's ConvexSetFinder over polytope obstacles (obs_sets + obs_points_sets), answers memoised."""
-
-    def __init__(self, obs_sets, obs_points_sets, workspace_max, workspace_min):
-        from oracle.convex_set_finder import ConvexSetFinder as OracleFinder
-
-        self.obs_sets = obs_sets
-        self.set_finder = OracleFinder(obs_sets, obs_points_sets, list(workspace_max), list(workspace_min))
-        self.memo = {}
-
-
-def _polytope_query(i):
-    obs_sets, pts, infl, st, en, wmin, wmax = scenes.config_c3_polytope_query(i)
-    return dict(obs_sets=obs_sets, obs_points_sets=pts, start=st, end=en, r0=R0, r1=R0), infl, list(wmin), list(wmax)
 
 
 def _literal_push_out(obs_sets, end, r):
@@ -66,124 +46,13 @@ def _box_rows(lo, hi, cut=None):
 
 
 # ---- CPU: the native driver's state machines against the Python planner, the oracle answering both -----------
-def run_native_with_oracle(host_harness, queries, inflate, ws_max, ws_min, seeds, backends, sample_chunk=32):
-    """tests.test_planner_native.run_native_with_oracle for polytope queries (obs_sets instead of obstacles)."""
-    pk = pn.PackedQueries(queries, inflate, ws_max, ws_min, seeds, sample_chunk)
-    assert pk.kind == "polytopes" and pk.boxes is None
-    helpers = [SetSequencePlanner((), inflate, list(ws_max), list(ws_min), backend=backends[i], obs_sets=q["obs_sets"])
-               for i, q in enumerate(queries)]
-    ee = []
-    for q in queries:
-        omega = R.from_matrix(q["r1"] @ q["r0"].T).as_rotvec()
-        on = np.linalg.norm(omega)
-        ee.append((q["r0"] @ np.array([-0.05, 0, 0]), omega / on if on > 1e-6 else np.array([0, 0, 1.0]), on))
-    errors = []
-
-    def in_safe(nodes, n, x):
-        return any(np.max(_node_set(nodes[k])[0] @ x - _node_set(nodes[k])[1]) < 1e-3 for k in range(n))
-
-    def dvertex(nodes, n, Q, p):
-        if n == 0:
-            return np.inf
-        return min(np.linalg.norm(np.array(nodes[k].Q[:]).reshape(3, 3) - Q) + np.linalg.norm(np.array(nodes[k].P[:]) - p)
-                   for k in range(n))
-
-    def cb_set(qid, req, n_nodes, nodes, out):
-        try:
-            r, o = req.contents, out.contents
-            o.first, o.dv, o.collision = 0, np.inf, 0
-            p0 = np.array(r.p0[:])
-            if r.kind == 1:
-                try:
-                    _fill_set(o, backends[qid].execute(("set_line", p0, np.array(r.p1[:]))), True)
-                except (RuntimeError, ValueError) as e:
-                    _error_status(e, o)
-                return 0
-            if r.kind == 2:
-                cand = np.ctypeslib.as_array(r.cand, shape=(r.n_cand, 3)).copy()
-                o.first = -1
-                for i, c in enumerate(cand):
-                    if not helpers[qid]._in_collision(c) and not in_safe(nodes, n_nodes, c):
-                        o.first, p0 = i, c
-                        break
-                if o.first < 0:
-                    return 0
-            try:
-                ans = backends[qid].execute(("set_point", p0, bool(r.fixed_mid), bool(r.optimize)))
-            except (RuntimeError, ValueError) as e:
-                _error_status(e, o)
-                return 0
-            _fill_set(o, ans, False)
-            if r.with_dv:
-                o.dv = dvertex(nodes, n_nodes, ans[2], ans[3])
-            return 0
-        except Exception as e:                               # noqa: BLE001 -- surfaces in the test below
-            errors.append(e)
-            return 7
-
-    def cb_edges(qid, id_new, n_nodes, nodes, has_target, xd, out):
-        try:
-            others = [_node_set(nodes[k]) for k in range(id_new)]
-            new = _node_set(nodes[id_new])
-            res = backends[qid].execute(("edges", others, new, 0.01, ee[qid]))
-            for k, (x, ok, fits, via) in enumerate(res):
-                out[k].ok, out[k].fits, out[k].proj_ok = int(bool(ok)), int(bool(fits)), 0
-                if ok:
-                    out[k].x[:] = np.asarray(x).tolist()
-                    out[k].omega = float(via[3]) if fits else -1.0
-                    if has_target[k]:
-                        pr = backends[qid].execute(("project", np.concatenate((others[k][0], new[0])),
-                                                    np.concatenate((others[k][1], new[1])),
-                                                    np.array([xd[3 * k], xd[3 * k + 1], xd[3 * k + 2]])))
-                        out[k].proj[:] = np.asarray(pr).tolist()
-                        out[k].proj_ok = 1
-            return 0
-        except Exception as e:                               # noqa: BLE001
-            errors.append(e)
-            return 7
-
-    def cb_project(qid, id0, id1, xd, n_nodes, nodes, out):
-        try:
-            s0, s1 = _node_set(nodes[id0]), _node_set(nodes[id1])
-            x = backends[qid].execute(("project", np.concatenate((s0[0], s1[0])), np.concatenate((s0[1], s1[1])),
-                                       np.array([xd[0], xd[1], xd[2]])))
-            out.contents.x[:] = np.asarray(x).tolist()
-            return 0
-        except Exception as e:                               # noqa: BLE001
-            errors.append(e)
-            return 7
-
-    def cb_path(qid, n, edge_off, edge_dst, edge_w, path_out, path_len):
-        try:
-            g = nx.Graph()
-            g.add_nodes_from(range(n))
-            for v in range(n):
-                for e in range(edge_off[v], edge_off[v + 1]):
-                    g._adj[v][edge_dst[e]] = {"weight": edge_w[e]}
-            p = nx.shortest_path(g, 0, 1, weight="weight")
-            path_len[0] = len(p)
-            for k, v in enumerate(p[: pn.MAX_PATH]):
-                path_out[k] = v
-            return 0
-        except Exception as e:                               # noqa: BLE001
-            errors.append(e)
-            return 7
-
-    cbs = (CB_SET(cb_set), CB_EDGES(cb_edges), CB_PROJECT(cb_project), CB_PATH(cb_path))
-    host_harness.hh_plan_batch.restype = ctypes.c_int
-    rc = host_harness.hh_plan_batch(ctypes.byref(pk.inp), ctypes.byref(pk.out), *cbs, 1)
-    assert not errors, errors[0]
-    assert rc == 0
-    return pk
-
-
 def test_native_driver_equals_python_planner_over_polytopes_on_cpu(host_harness):
     """Six C3 polytope queries (one with its `end` inside an obstacle) through the native state machines and through
     SetSequencePlanner, the oracle answering both: the same paths, set ids, via points (bit for bit), graph sizes,
     sets, error exits and generator states."""
     queries, seeds, backends = [], [], []
     for i in range(6):
-        q, infl, wmin, wmax = _polytope_query(i)
+        q, infl, wmin, wmax = _c3_poly(i)
         queries.append(q)
         seeds.append(i)
         backends.append(PolytopeOracleBackend(q["obs_sets"], q["obs_points_sets"], wmax, wmin))
@@ -195,28 +64,11 @@ def test_native_driver_equals_python_planner_over_polytopes_on_cpu(host_harness)
     assert pl.polytopes and pl._in_collision(q["end"])
     assert not np.array_equal(pl._push_out_general(q["end"].copy()), q["end"])
 
-    want = []
-    for q, s, be in zip(queries, seeds, backends):
-        pl = SetSequencePlanner((), infl, wmax, wmin, backend=be, rng=np.random.default_rng(s), obs_sets=q["obs_sets"])
-        try:
-            res = pl.plan_set_sequence(q["start"].copy(), q["end"].copy(), q["r0"], q["r1"])
-        except (RuntimeError, ValueError) as e:
-            res = e
-        want.append((res, pl))
+    want = [python_plan(q, infl, wmax, wmin, s, be) for q, s, be in zip(queries, seeds, backends)]
     pk = run_native_with_oracle(host_harness, queries, infl, wmax, wmin, seeds, backends)
-    got = pk.results()
-    for i, ((w, pl), g) in enumerate(zip(want, got)):
-        if isinstance(w, Exception):
-            assert isinstance(g, Exception), f"query {i}: native planned, python raised {w!r}"
-            assert type(g) is type(w) and str(g).split("(")[0] == str(w).split("(")[0], (i, g, w)
-        else:
-            assert not isinstance(g, Exception), f"query {i}: {g!r}"
-            assert g["path"] == w["path"] and g["set_ids"] == w["set_ids"], i
-            assert np.array_equal(g["p_via"], w["p_via"]), i
-            assert g["n_nodes"] == w["graph"].number_of_nodes() and g["n_inter"] == w["inter_graph"].number_of_nodes()
-            assert g["n_edges"] == w["inter_graph"].number_of_edges()
-            for (ga, gb), (wa, wb) in zip(g["sets_via"], w["sets_via"]):
-                assert np.array_equal(ga, wa) and np.array_equal(gb, wb)
+    assert pk.kind == "polytopes" and pk.boxes is None
+    for i, ((w, pl), g) in enumerate(zip(want, pk.results())):
+        assert_same_result(g, w, pl, i)
         assert [int(v) for v in pk.rng_out[i]] == pn.rng_state_words(pl.rng), f"query {i}: generator state"
     assert (pk.err_kind != 0).sum() >= 1 and (pk.err_kind == 0).sum() >= 2, pk.err_kind
 
@@ -231,7 +83,7 @@ def test_push_out_cases_match_the_reference_loop():
     cut = (np.array([1.0, 1.0, 1.0]) / np.sqrt(3.0), 5.0)                       # redundant row: a general polytope
     cases = []
     # inside one polytope (a random one of the C3 polytope scene, at its centroid)
-    q, *_ = _polytope_query(0)
+    q, *_ = _c3_poly(0)
     cases.append((q["obs_sets"], q["obs_points_sets"][7].mean(axis=0), "inside one"))
     # two overlapping polytopes: pushed out of the first through x = 0.1; the moved `end` (not the given one) lies in
     # the second, which pushes it out through y = 0.045
@@ -287,7 +139,7 @@ def test_push_out_general_rows_equal_the_box_path_on_boxes():
 def test_new_obs_with_start_inside_a_polytope_raises_attribute_error():
     """Quirk Q12 on polytopes: with new_obs, a start inside an inflated obstacle ends in the reference's
     AttributeError (`ob.A()` on a list), as on boxes."""
-    q, infl, wmin, wmax = _polytope_query(1)
+    q, infl, wmin, wmax = _c3_poly(1)
     backend = PolytopeOracleBackend(q["obs_sets"], q["obs_points_sets"], wmax, wmin)
     inside = q["obs_points_sets"][3].mean(axis=0)
     pl = SetSequencePlanner((), infl, wmax, wmin, backend=backend, rng=np.random.default_rng(0), obs_sets=q["obs_sets"])
@@ -298,7 +150,7 @@ def test_new_obs_with_start_inside_a_polytope_raises_attribute_error():
 
 
 def test_mixed_batches_raise_value_error():
-    q, infl, wmin, wmax = _polytope_query(0)
+    q, infl, wmin, wmax = _c3_poly(0)
     boxes, _, st, en, *_ = scenes.config_c3_query(0)
     qb = dict(obstacles=boxes, start=st, end=en, r0=R0, r1=R0)
     assert pn.query_kind([q, q]) == "polytopes" and pn.query_kind([qb]) == "boxes"
@@ -342,7 +194,7 @@ def test_native_plan_batch_equals_python_plan_batch_over_polytopes_on_gpu():
     ids = list(range(24))
     queries = []
     for i in ids:
-        q, infl, wmin, wmax = _polytope_query(i)
+        q, infl, wmin, wmax = _c3_poly(i)
         queries.append(q)
     want, _ = plan_batch(queries, infl, wmax, wmin, rng_seeds=ids)
     got, stats = pn.plan_batch_native(queries, infl, wmax, wmin, rng_seeds=ids)
@@ -363,7 +215,7 @@ def test_polytope_queries_gpu_backend_matches_oracle_sequence():
     """plan_set_sequence on the GPU backend (the default backend of a polytope planner) == the oracle backend."""
     n_ok = 0
     for i in range(8):
-        q, infl, wmin, wmax = _polytope_query(i)
+        q, infl, wmin, wmax = _c3_poly(i)
         out = []
         for backend in (None, PolytopeOracleBackend(q["obs_sets"], q["obs_points_sets"], wmax, wmin)):
             pl = SetSequencePlanner((), infl, wmax, wmin, backend=backend, rng=np.random.default_rng(i),
@@ -414,7 +266,7 @@ def test_bp_plan_run_refuses_the_other_obstacle_kind():
     """bp_plan_run fails, without planning, when the input's obstacle kind or counts are not the scene batch's."""
     from boundplanner_b200 import _lib
 
-    q, infl, wmin, wmax = _polytope_query(0)
+    q, infl, wmin, wmax = _c3_poly(0)
     ob, _, st, en, *_ = scenes.config_c3_query(0)
     qb = dict(obstacles=ob, start=st, end=en, r0=R0, r1=R0)
     lib = _lib.load()

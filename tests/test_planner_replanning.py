@@ -10,228 +10,21 @@ type and message and the generator state afterwards.
 GPU: bp_plan_run against planner.plan_batch over the kernels (and both against plan_set_sequence on the GpuBackend),
 a 5-step MPC loop, and batches without replanning inputs against batches with all of them zero."""
 import ctypes
-import os
-import subprocess
 
-import networkx as nx
 import numpy as np
 import pytest
-from scipy.spatial.transform import Rotation as R
 
 from boundplanner_b200 import planner_native as pn
 from boundplanner_b200 import scenes
 from boundplanner_b200.planner import SetSequencePlanner, plan_batch
-from tests.test_planner_native import (CB_EDGES, CB_PATH, CB_PROJECT, CB_SET, MemoBackend, SetAns, _error_status,
-                                       _fill_set, _node_set)
-from tests.test_planner_polytopes import PolytopeOracleBackend
+from tests.util import (ERRORS, R0, MemoBackend, OracleLockstepExecutor, _backend, _c3, _c3_poly, _dp, _ip, _is_poly,
+                        _same_sets, assert_same_result, mpc_step, python_plan, run_native_with_oracle)
 
-R0 = R.from_euler("XYZ", [0, 90, 0], degrees=True).as_matrix()
 P0 = np.array([0.3, 0.0, 0.7])                  # boundplanner_example.py:89-92
 P1 = np.array([0.45, -0.5, 0.2])
-_dp = ctypes.POINTER(ctypes.c_double)
-_ip = ctypes.POINTER(ctypes.c_int)
-ERRORS = (RuntimeError, ValueError, IndexError, AttributeError)
-
-
-class ReduceReq(ctypes.Structure):
-    _fields_ = [("qid", ctypes.c_int), ("m", ctypes.c_int), ("rows", _dp)]
-
-
-CB_REDUCE = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_int, ctypes.POINTER(ReduceReq), ctypes.POINTER(SetAns))
-
-
-@pytest.fixture(scope="module")
-def replan_harness():
-    """TEST-ONLY host build of the native driver with a reduce callback (tests/host_harness_replan.cpp, g++)."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    build = os.path.join(root, "tests", "_build")
-    os.makedirs(build, exist_ok=True)
-    so = os.path.join(build, "libbp_host_harness_replan.so")
-    src = os.path.join(root, "tests", "host_harness_replan.cpp")
-    deps = [src, os.path.join(root, "boundplanner_b200", "csrc", "bp_planner.h"), os.path.join(root, "include", "bpgeo.h")]
-    if not os.path.exists(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-pthread", "-ffp-contract=off", "-o", so, src])
-    lib = ctypes.CDLL(so)
-    lib.hr_plan_batch.restype = ctypes.c_int
-    lib.hr_sizeof.restype = ctypes.c_int
-    return lib
 
 
 # ---- the two sides, the oracle answering both -------------------------------------------------------------------
-def _is_poly(q):
-    return q.get("obs_sets") is not None
-
-
-def _backend(q, inflate, ws_max, ws_min):
-    if _is_poly(q):
-        return PolytopeOracleBackend(q["obs_sets"], q["obs_points_sets"], ws_max, ws_min)
-    return MemoBackend(q["obstacles"], inflate, ws_max, ws_min)
-
-
-def _planner(q, inflate, ws_max, ws_min, backend, seed=None):
-    return SetSequencePlanner(() if _is_poly(q) else q["obstacles"], inflate, list(ws_max), list(ws_min),
-                              backend=backend, rng=np.random.default_rng(seed),
-                              obs_sets=q["obs_sets"] if _is_poly(q) else backend.obs_sets)
-
-
-def python_plan(q, inflate, ws_max, ws_min, seed, backend):
-    """The sequential driver on one query, its planner holding the query's previous sets."""
-    pl = _planner(q, inflate, ws_max, ws_min, backend, seed)
-    pl.sets_via_prev = [[np.array(a, float), np.array(b, float)] for a, b in q.get("sets_via_prev", ())]
-    try:
-        res = pl.plan_set_sequence(q["start"].copy(), q["end"].copy(), q["r0"], q["r1"], q.get("first_sample"),
-                                   q.get("replanning", False), q.get("p_horizon", ()), q.get("new_obs", False))
-    except ERRORS as e:
-        res = e
-    return res, pl
-
-
-def run_native_with_oracle(harness, queries, inflate, ws_max, ws_min, seeds, backends, sample_chunk=32):
-    """The native state machines (hr_plan_batch) with every request answered by the queries' oracle
-    backends; boxes or polytopes."""
-    pk = pn.PackedQueries(queries, inflate, ws_max, ws_min, seeds, sample_chunk)
-    helpers = [_planner(q, inflate, ws_max, ws_min, backends[i]) for i, q in enumerate(queries)]
-    ee = []
-    for q in queries:
-        omega = R.from_matrix(q["r1"] @ q["r0"].T).as_rotvec()
-        on = np.linalg.norm(omega)
-        ee.append((q["r0"] @ np.array([-0.05, 0, 0]), omega / on if on > 1e-6 else np.array([0, 0, 1.0]), on))
-    errors = []
-
-    def guarded(fn):
-        def call(*a):
-            try:
-                return fn(*a)
-            except Exception as e:                           # noqa: BLE001 -- surfaces in the assert below
-                errors.append(e)
-                return 7
-        return call
-
-    @guarded
-    def cb_set(qid, req, n_nodes, nodes, out):
-        r, o = req.contents, out.contents
-        o.first, o.dv, o.collision = 0, np.inf, 0
-        p0 = np.array(r.p0[:])
-        if r.kind == 1:
-            try:
-                _fill_set(o, backends[qid].execute(("set_line", p0, np.array(r.p1[:]))), True)
-            except (RuntimeError, ValueError) as e:
-                _error_status(e, o)
-            return 0
-        if r.kind == 2:
-            cand = np.ctypeslib.as_array(r.cand, shape=(r.n_cand, 3)).copy()
-            o.first = -1
-            for i, c in enumerate(cand):
-                safe = any(np.max(_node_set(nodes[k])[0] @ c - _node_set(nodes[k])[1]) < 1e-3 for k in range(n_nodes))
-                if not helpers[qid]._in_collision(c) and not safe:
-                    o.first, p0 = i, c
-                    break
-            if o.first < 0:
-                return 0
-        try:
-            ans = backends[qid].execute(("set_point", p0, bool(r.fixed_mid), bool(r.optimize)))
-        except (RuntimeError, ValueError) as e:
-            _error_status(e, o)
-            return 0
-        _fill_set(o, ans, False)
-        if r.with_dv:
-            o.dv = min((np.linalg.norm(np.array(nodes[k].Q[:]).reshape(3, 3) - ans[2]) +
-                        np.linalg.norm(np.array(nodes[k].P[:]) - ans[3]) for k in range(n_nodes)), default=np.inf)
-        return 0
-
-    @guarded
-    def cb_edges(qid, id_new, n_nodes, nodes, has_target, xd, out):
-        others = [_node_set(nodes[k]) for k in range(id_new)]
-        new = _node_set(nodes[id_new])
-        res = backends[qid].execute(("edges", others, new, 0.01, ee[qid]))
-        for k, (x, ok, fits, via) in enumerate(res):
-            out[k].ok, out[k].fits, out[k].proj_ok = int(bool(ok)), int(bool(fits)), 0
-            if ok:
-                out[k].x[:] = np.asarray(x).tolist()
-                out[k].omega = float(via[3]) if fits else -1.0
-                if has_target[k]:
-                    pr = backends[qid].execute(("project", np.concatenate((others[k][0], new[0])),
-                                                np.concatenate((others[k][1], new[1])),
-                                                np.array([xd[3 * k], xd[3 * k + 1], xd[3 * k + 2]])))
-                    out[k].proj[:] = np.asarray(pr).tolist()
-                    out[k].proj_ok = 1
-        return 0
-
-    @guarded
-    def cb_project(qid, id0, id1, xd, n_nodes, nodes, out):
-        s0, s1 = _node_set(nodes[id0]), _node_set(nodes[id1])
-        x = backends[qid].execute(("project", np.concatenate((s0[0], s1[0])), np.concatenate((s0[1], s1[1])),
-                                   np.array([xd[0], xd[1], xd[2]])))
-        out.contents.x[:] = np.asarray(x).tolist()
-        return 0
-
-    @guarded
-    def cb_path(qid, n, edge_off, edge_dst, edge_w, path_out, path_len):
-        g = nx.Graph()
-        g.add_nodes_from(range(n))
-        for v in range(n):
-            for e in range(edge_off[v], edge_off[v + 1]):
-                g._adj[v][edge_dst[e]] = {"weight": edge_w[e]}
-        p = nx.shortest_path(g, 0, 1, weight="weight")
-        path_len[0] = len(p)
-        for k, v in enumerate(p[: pn.MAX_PATH]):
-            path_out[k] = v
-        return 0
-
-    @guarded
-    def cb_reduce(qid, req, out):
-        r, o = req.contents, out.contents
-        rows = np.ctypeslib.as_array(r.rows, shape=(r.m, 4)).copy()
-        Ar, br = backends[qid].execute(("reduce", rows[:, :3].copy(), rows[:, 3].copy()))
-        mr = Ar.shape[0]
-        o.status, o.m, o.m_red = 0, r.m, mr
-        o.Ar[: 3 * mr] = Ar.reshape(-1).tolist()
-        o.br[:mr] = br.tolist()
-        return 0
-
-    cbs = (CB_SET(cb_set), CB_EDGES(cb_edges), CB_PROJECT(cb_project), CB_PATH(cb_path), CB_REDUCE(cb_reduce))
-    rc = harness.hr_plan_batch(ctypes.byref(pk.inp), ctypes.byref(pk.out), *cbs, 1)
-    assert not errors, errors[0]
-    assert rc == 0
-    return pk
-
-
-def _same_sets(got, want, tol=0.0):
-    assert len(got) == len(want)
-    for (ga, gb), (wa, wb) in zip(got, want):
-        ga, gb, wa, wb = (np.asarray(v, float) for v in (ga, gb, wa, wb))
-        assert ga.shape == wa.shape and gb.shape == wb.shape
-        assert np.abs(ga - wa).max(initial=0.0) <= tol and np.abs(gb - wb).max(initial=0.0) <= tol
-
-
-def assert_same_result(g, w, pl, i, exact=True):
-    """g: a batched driver's result; w, pl: plan_set_sequence's result and planner."""
-    if isinstance(w, Exception):
-        assert isinstance(g, Exception), f"query {i}: planned, plan_set_sequence raised {w!r}"
-        assert type(g) is type(w), (i, g, w)
-        if exact:
-            assert str(g) == str(w), (i, g, w)
-        else:
-            assert str(g).split("(")[0] == str(w).split("(")[0], (i, g, w)
-        return False
-    assert not isinstance(g, Exception), f"query {i}: {g!r}"
-    assert g["path"] == w["path"] and g["set_ids"] == w["set_ids"], i
-    tol = 0.0 if exact else 1e-9
-    assert g["p_via"].shape == w["p_via"].shape and np.abs(g["p_via"] - w["p_via"]).max() <= tol, i
-    n_nodes = g["n_nodes"] if "n_nodes" in g else g["graph"].number_of_nodes()
-    n_inter = g["n_inter"] if "n_inter" in g else g["inter_graph"].number_of_nodes()
-    assert n_nodes == w["graph"].number_of_nodes() and n_inter == w["inter_graph"].number_of_nodes(), i
-    if "n_edges" in g:
-        assert g["n_edges"] == w["inter_graph"].number_of_edges(), i
-    set_tol = 0.0 if exact else 1e-9
-    _same_sets(g["sets_via"], w["sets_via"], set_tol)
-    _same_sets(g["sets_via_prev"], pl.sets_via_prev, set_tol)
-    assert ("p_horizon_max" in g) == pl.replanning, i
-    if pl.replanning:
-        assert np.array_equal(g["p_horizon_max"], pl.p_horizon_max), i
-    return True
-
-
 def check_native(harness, queries, inflate, ws_max, ws_min, seeds):
     """plan_set_sequence, the native state machines and plan_batch (oracle executor) on one batch: identical."""
     backends = [_backend(q, inflate, ws_max, ws_min) for q in queries]
@@ -249,48 +42,7 @@ def check_native(harness, queries, inflate, ws_max, ws_min, seeds):
     return want, got
 
 
-class OracleLockstepExecutor:
-    """CPU stand-in for planner.BatchedGpuExecutor: every pending request answered by the query's oracle backend."""
-
-    def __init__(self, backends):
-        self.backends = backends
-        self.calls = 0
-
-    def execute(self, pending):
-        out = {}
-        self.calls += 1
-        for qid, req in pending.items():
-            try:
-                out[qid] = self.backends[qid].execute(req)
-            except (RuntimeError, ValueError) as e:
-                out[qid] = e
-        return out
-
-
 # ---- queries -------------------------------------------------------------------------------------------------
-def mpc_step(q, res, frac=0.02, n_horizon=10):
-    """The next MPC call after a planned result: start `frac` along the first segment, a horizon of n_horizon
-    points along the path from there, the result's sets_via_prev."""
-    p_via = res["p_via"]
-    start = p_via[0] + frac * (p_via[1] - p_via[0])
-    t = np.linspace(0.0, 1.0, n_horizon + 1)[1:]
-    pts = np.vstack((start, p_via[1:]))
-    seg = np.cumsum(np.r_[0.0, np.linalg.norm(np.diff(pts, axis=0), axis=1)])
-    s = t * seg[-1] * 0.6
-    horizon = np.stack([np.interp(s, seg, pts[:, k]) for k in range(3)], axis=1)
-    return dict(q, start=start, replanning=True, p_horizon=horizon, sets_via_prev=res["sets_via_prev"])
-
-
-def _c3(i):
-    ob, infl, st, en, wmin, wmax = scenes.config_c3_query(i)
-    return dict(obstacles=ob, start=st, end=en, r0=R0, r1=R0), infl, list(wmin), list(wmax)
-
-
-def _c3_poly(i):
-    obs_sets, pts, infl, st, en, wmin, wmax = scenes.config_c3_polytope_query(i)
-    return dict(obs_sets=obs_sets, obs_points_sets=pts, start=st, end=en, r0=R0, r1=R0), infl, list(wmin), list(wmax)
-
-
 def _inside_point(q, away_from):
     """A point inside one of the query's inflated obstacles, 0.15 m or more from `away_from`."""
     if _is_poly(q):
@@ -314,19 +66,7 @@ def fallback_queries(q, prev_sets):
 
 
 # ---- CPU ------------------------------------------------------------------------------------------------------
-def test_struct_layouts_v4(replan_harness):
-    from tests.test_planner_native import Node, SetReq
-
-    assert replan_harness.hr_sizeof(3) == ctypes.sizeof(pn.BpPlanIn)
-    assert replan_harness.hr_sizeof(4) == ctypes.sizeof(pn.BpPlanOut)
-    assert replan_harness.hr_sizeof(5) == ctypes.sizeof(ReduceReq)
-    assert pn.BpPlanIn.prev_rows.offset + ctypes.sizeof(_dp) == ctypes.sizeof(pn.BpPlanIn)
-    assert pn.BpPlanOut.p_horizon_max.offset + ctypes.sizeof(_dp) == ctypes.sizeof(pn.BpPlanOut)
-    for k, t in enumerate((SetReq, SetAns, Node)):                    # unchanged by the reduce request
-        assert replan_harness.hr_sizeof(k) == ctypes.sizeof(t)
-
-
-def test_c1_replanning_and_fallbacks_native_equals_python(replan_harness):
+def test_c1_replanning_and_fallbacks_native_equals_python(host_harness):
     """The C1 scenario of the sequential driver's replanning test, and every fallback, in one lock-step batch."""
     boxes, ws_min, ws_max, inflate = scenes.example_scene()
     ws_min, ws_max = list(ws_min), list(ws_max)
@@ -344,7 +84,7 @@ def test_c1_replanning_and_fallbacks_native_equals_python(replan_harness):
                dict(base, start=below, sets_via_prev=prev),                               # previous end set reused
                dict(base, start=below, new_obs=True)]                                     # rebuilt around start
     queries += fallback_queries(base, prev)
-    want, got = check_native(replan_harness, queries, inflate, ws_max, ws_min, list(range(len(queries))))
+    want, got = check_native(host_harness, queries, inflate, ws_max, ws_min, list(range(len(queries))))
     kinds = [type(w).__name__ if isinstance(w, Exception) else "planned" for w, _ in want]
     assert kinds[:3] == ["planned"] * 3 and kinds[3] == "IndexError" and kinds[4:6] == ["planned"] * 2, kinds
     assert kinds[6:] == ["IndexError", "planned", "planned", "AttributeError", "IndexError", "IndexError"], kinds
@@ -357,7 +97,7 @@ def test_c1_replanning_and_fallbacks_native_equals_python(replan_harness):
 
 
 @pytest.mark.parametrize("kind", ["boxes", "polytopes"])
-def test_mpc_sequences_native_equals_python(replan_harness, kind):
+def test_mpc_sequences_native_equals_python(host_harness, kind):
     """3-step MPC sequences on six C3 queries: every step's batch mixes replanning queries (the planned ones, their
     sets threaded forward) with first plans (the failed ones, which keep the caller's sets) and fallbacks."""
     make = _c3 if kind == "boxes" else _c3_poly
@@ -368,7 +108,7 @@ def test_mpc_sequences_native_equals_python(replan_harness, kind):
     queries, seeds = list(base), list(range(len(base)))
     n_replanned = 0
     for step in range(3):
-        want, _ = check_native(replan_harness, queries, infl, wmax, wmin, seeds)
+        want, _ = check_native(host_harness, queries, infl, wmax, wmin, seeds)
         nxt = []
         for q, (w, pl) in zip(queries, want):
             if isinstance(w, Exception):
@@ -384,7 +124,7 @@ def test_mpc_sequences_native_equals_python(replan_harness, kind):
     assert n_replanned >= 6
 
 
-def test_native_driver_rejects_malformed_replanning_inputs(replan_harness):
+def test_native_driver_rejects_malformed_replanning_inputs(host_harness):
     q, infl, wmin, wmax = _c3(0)
     good = [[np.eye(3), np.ones(3)]]
     with pytest.raises(ValueError, match="previous sets"):
@@ -404,13 +144,13 @@ def test_native_driver_rejects_malformed_replanning_inputs(replan_harness):
         rows = np.zeros((65, 4))
         pk.inp.prev_rows = rows.ctypes.data_as(_dp)
         pk.keep_rows = rows
-        assert replan_harness.hr_plan_batch(ctypes.byref(pk.inp), ctypes.byref(pk.out), None, None, None, None,
-                                                 None, 1) == 3
+        assert host_harness.hh_plan_batch(ctypes.byref(pk.inp), ctypes.byref(pk.out), None, None, None, None,
+                                          None, 1) == 3
         assert msg in pk.err_msg.value.decode(), (field, pk.err_msg.value)
     pk = pn.PackedQueries([dict(q, replanning=True)], infl, wmax, wmin, [0])
     pk.inp.horizon_off = None
-    assert replan_harness.hr_plan_batch(ctypes.byref(pk.inp), ctypes.byref(pk.out), None, None, None, None,
-                                             None, 1) == 3
+    assert host_harness.hh_plan_batch(ctypes.byref(pk.inp), ctypes.byref(pk.out), None, None, None, None,
+                                      None, 1) == 3
     assert b"without horizon_off" in pk.err_msg.value
 
 

@@ -14,7 +14,7 @@ from boundplanner_b200 import geometry as geo
 from boundplanner_b200 import planner_native as pn
 from boundplanner_b200 import scenes
 from boundplanner_b200.planner import plan_batch
-from tests.test_planner_replanning import _c3, _c3_poly, _same_sets, mpc_step
+from tests.util import _c3, _c3_poly, _same_sets, mpc_step
 
 WMIN, WMAX = scenes.WORKSPACE_MIN, scenes.WORKSPACE_MAX
 

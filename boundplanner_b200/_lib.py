@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libbpgeo.so")
 
 BP_MAX_ROWS = 48
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 STATUS_OK = 0
 STATUS_ELLIPSE_VIOLATION = 1
@@ -92,8 +92,9 @@ SIGNATURES = {
     "bp_debug_counters": (_i, [_c.POINTER(_c.c_ulonglong), _i, _i]),
     "bp_fk_iiwa14_kin": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "bp_probe_fp64": (_i, [_i, _i, _i, _i, _vp, _vp]),
-    # native lock-step planner driver: (scene batch, Q, &handle) / (handle, &bp_plan_in, &bp_plan_out, stream)
+    # native lock-step planner driver: (scene batch, Q[, query -> scene map], &handle) / (handle, &bp_plan_in, &bp_plan_out, stream)
     "bp_plan_create": (_i, [_vp, _i, _c.POINTER(_vp)]),
+    "bp_plan_create_mapped": (_i, [_vp, _i, _c.POINTER(_c.c_int), _c.POINTER(_vp)]),
     "bp_plan_run": (_i, [_vp, _vp, _vp, _vp]),
     "bp_plan_destroy": (_i, [_vp]),
 }

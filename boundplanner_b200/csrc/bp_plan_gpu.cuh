@@ -213,7 +213,7 @@ struct PlanLane {
         const SetReq& s = r.sets[order[j]];
         const Query& q = qs[r.set_owner[order[j]]];
         for (int k = 0; k < 3; ++k) { IN_H(double, i_p0)[3 * j + k] = s.p0[k]; IN_H(double, i_p1)[3 * j + k] = s.p1[k]; }
-        IN_H(int, i_scene)[j] = s.qid;
+        IN_H(int, i_scene)[j] = q.scene;                  // (the node tables stay per query)
         IN_H(int, i_nbeg)[j] = s.qid * MAX_NODES;
         IN_H(int, i_ncnt)[j] = s.with_dv ? (int)q.nodes.size() : 0;
         if (s.kind == SET_SAMPLE) {
@@ -221,7 +221,7 @@ struct PlanLane {
           memcpy(c, s.cand, sizeof(double) * 3 * s.n_cand);
           for (int e = s.n_cand; e < C; ++e) memcpy(c + 3 * e, s.cand, sizeof(double) * 3);   // padding never wins
           IN_H(int, i_sslot)[js] = j;
-          IN_H(int, i_sscene)[js] = s.qid;
+          IN_H(int, i_sscene)[js] = q.scene;
           IN_H(int, i_sbeg)[js] = s.qid * MAX_NODES;
           IN_H(int, i_scnt)[js] = (int)q.nodes.size();
           smp_of[j] = js++;
@@ -485,6 +485,8 @@ struct PlanLane {
 struct bp_plan : bpplan::Executor {
   const bp_scene* scene = nullptr;
   int Q = 0, L = 1;
+  bool mapped = false;                           // created by bp_plan_create_mapped
+  std::vector<int> query_scene;                  // [Q] the scene of every query (the identity when not mapped)
   bool polytopes = false;                        // the scene batch holds polytopes (bp_plan_in::obs_rows) or boxes
   double *tabA = nullptr, *tabb = nullptr, *tabq = nullptr, *tabp = nullptr, *tabaabb = nullptr;
   int* tabm = nullptr;
@@ -523,16 +525,16 @@ static int plan_scene_limits(const bp_scene* sc, const char* fn) {
   return 0;
 }
 
-extern "C" {
-
-int bp_plan_create(const bp_scene* scene_batch, int Q, bp_plan** out) {
-  if (!scene_batch || Q < 1 || !out) return bp_fail("bp_plan_create: bad arguments");
-  if (!scene_batch->seg_off || scene_batch->n_seg != Q) return bp_fail("bp_plan_create: needs a scene batch with one scene per query");
+// bp_plan_create / bp_plan_create_mapped once the query -> scene map is known and checked
+static int plan_create(const bp_scene* scene_batch, int Q, std::vector<int>&& query_scene, bool mapped, const char* fn,
+                       bp_plan** out) {
   // reported here rather than by the first round that builds a set
-  if (plan_scene_limits(scene_batch, "bp_plan_create")) return 1;
+  if (plan_scene_limits(scene_batch, fn)) return 1;
   bp_plan* pl = new bp_plan();
   pl->scene = scene_batch;
   pl->Q = Q;
+  pl->mapped = mapped;
+  pl->query_scene = std::move(query_scene);
   pl->polytopes = scene_batch->rows != nullptr;
   // two lanes once there is enough work to split (BPGEO_PLAN_LANES=1 forces plain lock step)
   pl->L = Q >= 32 ? 2 : 1;
@@ -569,10 +571,34 @@ int bp_plan_create(const bp_scene* scene_batch, int Q, bp_plan** out) {
   if (e != cudaSuccess) {
     pl->release();
     delete pl;
-    return bp_fail("bp_plan_create", e);
+    return bp_fail(fn, e);
   }
   *out = pl;
   return 0;
+}
+
+extern "C" {
+
+int bp_plan_create(const bp_scene* scene_batch, int Q, bp_plan** out) {
+  if (!scene_batch || Q < 1 || !out) return bp_fail("bp_plan_create: bad arguments");
+  if (!scene_batch->seg_off || scene_batch->n_seg != Q) return bp_fail("bp_plan_create: needs a scene batch with one scene per query");
+  std::vector<int> ident((size_t)Q);
+  for (int q = 0; q < Q; ++q) ident[(size_t)q] = q;
+  return plan_create(scene_batch, Q, std::move(ident), false, "bp_plan_create", out);
+}
+
+int bp_plan_create_mapped(const bp_scene* scene_batch, int Q, const int* query_scene_host, bp_plan** out) {
+  if (!scene_batch || Q < 1 || !query_scene_host || !out) return bp_fail("bp_plan_create_mapped: bad arguments");
+  if (!scene_batch->seg_off || scene_batch->n_seg < 1) return bp_fail("bp_plan_create_mapped: needs a scene batch");
+  const int n_scenes = scene_batch->n_seg;
+  for (int q = 0; q < Q; ++q)
+    if (query_scene_host[q] < 0 || query_scene_host[q] >= n_scenes) {
+      snprintf(g_err, sizeof(g_err), "bp_plan_create_mapped: query %d maps to scene %d, the batch has %d scenes", q,
+               query_scene_host[q], n_scenes);
+      return 1;
+    }
+  return plan_create(scene_batch, Q, std::vector<int>(query_scene_host, query_scene_host + Q), true, "bp_plan_create_mapped",
+                     out);
 }
 
 int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* stream) {
@@ -589,11 +615,16 @@ int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* strea
     return bp_fail("bp_plan_run: the plan's scene batch holds polytopes, the input has no obs_rows");
   if (!pl->polytopes && in->obs_rows)
     return bp_fail("bp_plan_run: the plan's scene batch holds boxes, the input has obs_rows");
-  for (int q = 0; q < pl->Q; ++q) {
+  // (a mapped plan's input holds every scene once: box_off has n_scenes + 1 entries)
+  for (int s = 0; s < pl->scene->n_seg; ++s) {
     const int* so = pl->scene->seg_off_host;
-    const int n_in = in->box_off[q + 1] - in->box_off[q], n_scene = so[q + 1] - so[q];
+    const int n_in = in->box_off[s + 1] - in->box_off[s], n_scene = so[s + 1] - so[s];
     if (n_in != n_scene) {
-      snprintf(g_err, sizeof(g_err), "bp_plan_run: query %d has %d obstacles, its scene %d", q, n_in, n_scene);
+      if (pl->mapped)
+        snprintf(g_err, sizeof(g_err), "bp_plan_run: scene %d has %d obstacles in the input, %d in the plan's scene batch", s,
+                 n_in, n_scene);
+      else
+        snprintf(g_err, sizeof(g_err), "bp_plan_run: query %d has %d obstacles, its scene %d", s, n_in, n_scene);
       return 1;
     }
   }
@@ -603,7 +634,7 @@ int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* strea
   bpplan::Params par;
   std::vector<bpplan::Query> qs;
   const auto t_run0 = std::chrono::steady_clock::now();
-  bpplan::load_queries(*in, par, qs);
+  bpplan::load_queries(*in, par, qs, pl->query_scene.data());
   const auto t_run1 = std::chrono::steady_clock::now();
   // the work queued on the caller's stream so far precedes the run on every lane
   BP_CUDA(cudaStreamSynchronize((cudaStream_t)stream));

@@ -171,6 +171,7 @@ struct Query {
   enum After { AFTER_START_NODE, AFTER_END_NODE, AFTER_SAMPLE_NODE };
 
   int qid = 0;
+  int scene = 0;              // the scene of the batch this query plans against (query_scene[qid], else qid)
   const Params* par = nullptr;
   QueryInput in;
   Pcg64 rng;
@@ -1124,7 +1125,9 @@ inline std::string check_replan_inputs(const bp_plan_in& in) {
   return "";
 }
 
-inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& qs) {
+// query_scene [Q] (or NULL: query q plans in scene q): query q's obstacles are scene query_scene[q]'s, i.e.
+// in.box_off has one entry per scene + 1 and the boxes / obs_rows of every scene appear once
+inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& qs, const int* query_scene = nullptr) {
   par.obs_size_increase = in.inflate;
   for (int k = 0; k < 3; ++k) { par.ws_min[k] = in.ws_min[k]; par.ws_max[k] = in.ws_max[k]; }
   if (in.sample_chunk > 0) par.sample_chunk = in.sample_chunk;
@@ -1141,9 +1144,10 @@ inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& 
   qs.resize((size_t)in.Q);
   for (int q = 0; q < in.Q; ++q) {
     QueryInput qi;
-    qi.boxes = in.obs_rows ? nullptr : in.boxes + 6 * (size_t)in.box_off[q];
-    qi.obs_rows = in.obs_rows ? in.obs_rows + (size_t)OBS_ROWS * 4 * in.box_off[q] : nullptr;
-    qi.n_obs = in.box_off[q + 1] - in.box_off[q];
+    const int s = query_scene ? query_scene[q] : q;
+    qi.boxes = in.obs_rows ? nullptr : in.boxes + 6 * (size_t)in.box_off[s];
+    qi.obs_rows = in.obs_rows ? in.obs_rows + (size_t)OBS_ROWS * 4 * in.box_off[s] : nullptr;
+    qi.n_obs = in.box_off[s + 1] - in.box_off[s];
     for (int k = 0; k < 3; ++k) {
       qi.start[k] = in.starts[3 * q + k]; qi.end[k] = in.ends[3 * q + k];
       qi.l_ee[k] = in.l_ee[3 * q + k]; qi.l_ee_end[k] = in.l_ee_end[3 * q + k];
@@ -1160,6 +1164,7 @@ inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& 
     qi.prev_row_off = in.prev_off && in.prev_row_off ? in.prev_row_off + in.prev_off[q] : nullptr;
     qi.prev_rows = in.prev_rows;
     qs[(size_t)q].init(q, &par, qi);
+    qs[(size_t)q].scene = s;
   }
 }
 

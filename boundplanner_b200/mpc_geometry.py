@@ -23,18 +23,26 @@ from . import geometry as geo
 COL_JOINT_SIZES = (0.09, 0.12, 0.09, 0.10, 0.07, 0.09, 0.075)      # RobotModel.py:37 (iiwa14)
 
 
-def collision_sets(scene, q0, qf, ws_min, ws_max, e_max=0.7, n_points=6, max_set_size=15):
+def collision_sets(scene, q0, qf, ws_min, ws_max, e_max=0.7, n_points=6, max_set_size=15, robot_scene=None):
     """q0, qf: [7] or [T,7].  Returns (a_set_joints [T,6,15,3], b_set_joints [T,6,15], collision [T,6]) as
-    NumPy arrays, padded like normalize_set_size(set_joints, 15) with b already reduced by the joint sizes."""
+    NumPy arrays, padded like normalize_set_size(set_joints, 15) with b already reduced by the joint sizes.
+    robot_scene [T]: ``scene`` is a scene batch (SceneBatch / PolytopeSceneBatch) and robot t's segments are built
+    against its scene robot_scene[t] (a fleet of robots in a few shared cells); without it, ``scene`` is one scene."""
     q0 = np.asarray(q0, float).reshape(-1, 7)
     qf = np.asarray(qf, float).reshape(-1, 7)
     T = q0.shape[0]
+    item_scene = None
+    if robot_scene is not None:
+        robot_scene = np.asarray(robot_scene).reshape(-1)
+        if robot_scene.shape[0] != T:
+            raise ValueError(f"robot_scene has {robot_scene.shape[0]} entries for {T} robots")
+        item_scene = np.repeat(robot_scene.astype(np.int32), n_points)
     q = torch.as_tensor(np.concatenate((q0, qf))).cuda()
     _, p_col, _, _ = geo.fk_iiwa14(q)                                  # [2T,7,3]
     pl = p_col[:T, :n_points].reshape(-1, 3)                           # fk_pos_col(q0, i), i < 6
     pf = p_col[T:, :n_points].reshape(-1, 3)
     out = geo.build_sets_line(scene, pl, pf, ws_min, ws_max, compute_ellipsoid=False, limit_space=True, e_max=e_max,
-                              m_max=max_set_size)
+                              m_max=max_set_size, item_scene=item_scene)
     sizes = torch.as_tensor(COL_JOINT_SIZES[:n_points], dtype=torch.float64, device="cuda").repeat(T)
     rows = torch.arange(max_set_size, device="cuda").unsqueeze(0) < out.m.unsqueeze(1)
     b = torch.where(rows, out.b - sizes.unsqueeze(1), out.b)           # b_c - joint_sizes[i]; padding stays 10

@@ -572,7 +572,7 @@ class SetSequencePlanner:
 
 
 # ---------------------------------------------------------------------------------------------
-# Batched driver (BASELINE config C3): many independent queries, one scene each, in lock step
+# Batched driver (BASELINE config C3): many independent queries, one scene each (or shared scenes), in lock step
 # ---------------------------------------------------------------------------------------------
 class BatchedGpuExecutor:
     """Answers the pending requests of many queries with one batched kernel call per primitive.
@@ -586,9 +586,12 @@ class BatchedGpuExecutor:
     MAX_NODES = 64           # graph nodes per query the tables hold (2 + 20 samples + via-point re-samples)
     NODE_ROWS = 24           # rows per reduced node set (the reference's sets have at most 20)
 
-    def __init__(self, obstacles_list, obs_size_increase, workspace_max, workspace_min, polytope_scenes=None):
+    def __init__(self, obstacles_list, obs_size_increase, workspace_max, workspace_min, polytope_scenes=None,
+                 query_scene=None):
         """obstacles_list: one [N_k,6] box array per query; or polytope_scenes: one (obs_sets, obs_points_sets |
-        None) pair per query (inflated polytopes, PolytopeSceneBatch), obstacles_list then unused."""
+        None) pair per query (inflated polytopes, PolytopeSceneBatch), obstacles_list then unused.  query_scene [Q]:
+        the queries share the scenes, query q plans in scene query_scene[q] (the lists then hold one entry per
+        scene)."""
         from . import geometry as geo
 
         self.geo = geo
@@ -598,6 +601,10 @@ class BatchedGpuExecutor:
         else:
             self.scene = geo.SceneBatch(obstacles_list, obs_size_increase)
             self._n_queries = len(obstacles_list)
+        self._scene_of = None
+        if query_scene is not None:
+            self._scene_of = np.asarray(query_scene, np.int32).reshape(-1)
+            self._n_queries = self._scene_of.shape[0]
         self.ws_min = np.asarray(workspace_min, float)
         self.ws_max = np.asarray(workspace_max, float)
         self.calls = 0
@@ -667,6 +674,11 @@ class BatchedGpuExecutor:
                                                tab["begin"][qi], tab["count"][qi])[0]
 
     # -- helpers ----------------------------------------------------------------
+    def _item_scene(self, qids):
+        """The scene index of every query of qids (the query itself without a query -> scene map)."""
+        qids = np.asarray(qids, np.int32)
+        return qids if self._scene_of is None else self._scene_of[qids]
+
     def _reduced(self, batch):
         import torch
 
@@ -729,7 +741,7 @@ class BatchedGpuExecutor:
             seeds = np.array([pending[q][1] for q in qids])
             batch = geo.build_sets_point(self.scene, seeds, self.ws_min, self.ws_max, fixed_mid=fixed_mid,
                                          optimize=optimize, row_cap=REFERENCE_MAX_ROWS,
-                                         item_scene=np.asarray(qids, np.int32))
+                                         item_scene=self._item_scene(qids))
             dv = None
             if with_dv:
                 import torch
@@ -766,13 +778,13 @@ class BatchedGpuExecutor:
                 cand[k, counts[k]:] = c[0]               # padding: copies of the first candidate never win
             cand_d = torch.as_tensor(cand).cuda()
             qi = torch.as_tensor(np.asarray(qids, np.int64)).cuda()
+            si = qi.to(torch.int32) if self._scene_of is None else torch.as_tensor(self._item_scene(qids)).cuda()
             first_d = geo.sample_filter_tables(self.scene, cand_d, tab["A"], tab["b"], tab["m"], tab["begin"][qi],
-                                               tab["count"][qi], item_scene=qi.to(torch.int32))
+                                               tab["count"][qi], item_scene=si)
             pick = first_d.clamp(min=0).to(torch.int64)
             seeds_d = cand_d[torch.arange(len(qids), device="cuda"), pick]
             batch = geo.build_sets_point(self.scene, seeds_d, self.ws_min, self.ws_max, fixed_mid=True,
-                                         optimize=optimize, row_cap=REFERENCE_MAX_ROWS,
-                                         item_scene=qi.to(torch.int32))
+                                         optimize=optimize, row_cap=REFERENCE_MAX_ROWS, item_scene=si)
             dv = self._dvertex(batch, qi).cpu().numpy()
             first = first_d.cpu().numpy()
             peak = batch.rows_peak.cpu().numpy()
@@ -823,7 +835,7 @@ class BatchedGpuExecutor:
             p0 = np.array([pending[q][1] for q in qids])
             p1 = np.array([pending[q][2] for q in qids])
             batch = geo.build_sets_line(self.scene, p0, p1, self.ws_min, self.ws_max, compute_ellipsoid=True,
-                                        item_scene=np.asarray(qids, np.int32))
+                                        item_scene=self._item_scene(qids))
             coll = batch.collision.cpu().numpy()
             A, b, m, Q, P, st, Ar, br, mr = self._reduced(batch)
             for k, q in enumerate(qids):
@@ -942,7 +954,7 @@ def _planned(res, pl):
 
 
 def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0),
-               rng_seeds=None, executor=None):
+               rng_seeds=None, executor=None, scenes=None):
     """Plan many independent queries in lock step.
 
     queries: list of dicts(obstacles [N,6], start, end, r0, r1[, first_sample]); or, for polytope obstacles,
@@ -953,28 +965,42 @@ def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), w
     start-in-collision fallback of a first plan, :296-324).  A batch may mix replanning and first-plan queries.
     Returns (results, stats): results[i] is the planner's dict or the exception the sequential planner
     would have raised for that query.  A planned query's dict also holds ``sets_via_prev`` (what the planner keeps
-    for its next call) and, when it replanned, ``p_horizon_max``."""
-    from .planner_native import query_kind
+    for its next call) and, when it replanned, ``p_horizon_max``.
+    scenes: queries over shared scenes (planner_native.scene_map): a list of dicts with the obstacle keys above, each
+    query carrying ``scene`` (its index) instead; every scene is stored on the device, and its host obstacle sets
+    built, once."""
+    from .planner_native import query_kind, scene_map
 
-    polytopes = query_kind(queries) == "polytopes"
+    query_scene = scene_map(queries, scenes)
+    holders = queries if scenes is None else scenes
+    polytopes = query_kind(holders, "query" if scenes is None else "scene") == "polytopes"
     if executor is None:
         if polytopes:
             executor = BatchedGpuExecutor(None, obs_size_increase, workspace_max, workspace_min,
-                                          polytope_scenes=[(q["obs_sets"], q.get("obs_points_sets")) for q in queries])
+                                          polytope_scenes=[(h["obs_sets"], h.get("obs_points_sets")) for h in holders],
+                                          query_scene=query_scene)
         else:
-            executor = BatchedGpuExecutor([q["obstacles"] for q in queries], obs_size_increase, workspace_max,
-                                          workspace_min)
+            executor = BatchedGpuExecutor([h["obstacles"] for h in holders], obs_size_increase, workspace_max,
+                                          workspace_min, query_scene=query_scene)
+    # the obstacles of query i (its own, or its scene's) and, over shared scenes, the host obstacle sets of every
+    # box scene, built once
+    obs_of = (lambda i: queries[i]) if scenes is None else (lambda i: scenes[query_scene[i]])
+    scene_sets = None
+    if scenes is not None and not polytopes:
+        scene_sets = [obstacle_sets(h["obstacles"], obs_size_increase) for h in scenes]
     import time
 
     t_start = time.perf_counter()
     planners, gens, pending, results = [], {}, {}, [None] * len(queries)
     finish = [0.0] * len(queries)              # seconds after the start of the batch at which query i was answered
     for i, q in enumerate(queries):
-        pl = SetSequencePlanner(() if polytopes else q["obstacles"], obs_size_increase, workspace_max, workspace_min,
+        ob = obs_of(i)
+        pl = SetSequencePlanner(() if polytopes else ob["obstacles"], obs_size_increase, workspace_max, workspace_min,
                                 rng=np.random.default_rng(rng_seeds[i] if rng_seeds is not None else None),
                                 device_loop=bool(getattr(executor, "device_loop", False)),
-                                obs_sets=q["obs_sets"] if polytopes else None,
-                                obs_points_sets=q.get("obs_points_sets") if polytopes else None)
+                                obs_sets=ob["obs_sets"] if polytopes else
+                                (scene_sets[query_scene[i]] if scene_sets is not None else None),
+                                obs_points_sets=ob.get("obs_points_sets") if polytopes else None)
         pl.sets_via_prev = [[np.array(a, float), np.array(b, float)] for a, b in q.get("sets_via_prev", ())]
         planners.append(pl)
         gens[i] = pl.plan_gen(q["start"], q["end"], q["r0"], q["r1"], q.get("first_sample"),

@@ -103,19 +103,69 @@ def ee_setup(r0, r1, length_ee=LENGTH_EE):
     return l_ee, l_ee_end, samples
 
 
-def query_kind(queries):
+def query_kind(queries, what="query"):
     """'boxes' when every query carries ``obstacles`` ([N,6] lb | ub), 'polytopes' when every query carries
     ``obs_sets`` (inflated [A (<= 15 x 3), b] per obstacle, optionally ``obs_points_sets``).  One scene batch holds
-    one kind: a batch that mixes them, or a query with both or neither, raises ValueError."""
+    one kind: a batch that mixes them, or a query with both or neither, raises ValueError.  (Also the kind of a list
+    of shared scenes, ``what="scene"``.)"""
     kinds = set()
     for i, q in enumerate(queries):
         has_boxes, has_sets = q.get("obstacles") is not None, q.get("obs_sets") is not None
         if has_boxes == has_sets:
-            raise ValueError(f"query {i} must carry either 'obstacles' (boxes) or 'obs_sets' (polytopes)")
+            raise ValueError(f"{what} {i} must carry either 'obstacles' (boxes) or 'obs_sets' (polytopes)")
         kinds.add("polytopes" if has_sets else "boxes")
     if len(kinds) > 1:
-        raise ValueError("a batch mixes box and polytope queries: one scene batch holds one obstacle kind")
+        raise ValueError(f"a batch mixes box and polytope {'queries' if what == 'query' else what + 's'}: one scene "
+                         "batch holds one obstacle kind")
     return kinds.pop() if kinds else "boxes"
+
+
+_OBSTACLE_KEYS = ("obstacles", "obs_sets", "obs_points_sets")
+
+
+def scene_map(queries, scenes=None):
+    """The query -> scene map of a batch over shared scenes: None without ``scenes`` (every query carries its own
+    obstacles), else int32 [Q] of the queries' ``scene`` indices.  ``scenes`` is a list of dicts with the obstacle keys
+    a query carries otherwise (``obstacles``, or ``obs_sets`` [+ ``obs_points_sets``]), all of one kind; each query
+    then carries ``scene`` (an int in [0, len(scenes))) and no obstacles.  ValueError (before anything touches the
+    device) for a ``scene`` out of range or not an int, a query with both a scene and obstacles or neither, scenes of
+    mixed kinds and ``scene`` keys without ``scenes``."""
+    if scenes is None:
+        for i, q in enumerate(queries):
+            if "scene" in q:
+                raise ValueError(f"query {i} carries 'scene' but no scenes were given")
+        return None
+    if len(scenes) == 0:
+        raise ValueError("scenes is empty")
+    query_kind(scenes, "scene")
+    out = np.zeros(len(queries), np.int32)
+    for i, q in enumerate(queries):
+        has_obs = any(q.get(k) is not None for k in _OBSTACLE_KEYS)
+        if "scene" not in q:
+            raise ValueError(f"query {i} carries no 'scene'" + (" (it carries obstacles)" if has_obs else ""))
+        if has_obs:
+            raise ValueError(f"query {i} carries both 'scene' and obstacles")
+        s = q["scene"]
+        if isinstance(s, (bool, np.bool_)) or not isinstance(s, (int, np.integer)):
+            raise ValueError(f"query {i}: scene {s!r} is not an int")
+        if not 0 <= s < len(scenes):
+            raise ValueError(f"query {i}: scene {s} out of range (0 .. {len(scenes) - 1})")
+        out[i] = s
+    return out
+
+
+def pack_obstacles(holders, kind):
+    """(box_off [n+1], boxes [sum N, 6] or None, obs_rows [sum N, 15, 4] or None) of a list of queries or scenes (the
+    obstacle layout of bp_plan_in)."""
+    n = len(holders)
+    box_off = np.zeros(n + 1, np.int32)
+    if kind == "polytopes":
+        rows = [obs_rows_of(h["obs_sets"]) for h in holders]
+        box_off[1:] = np.cumsum([r.shape[0] for r in rows])
+        return box_off, None, np.ascontiguousarray(np.concatenate(rows)) if n else np.zeros((0, OBS_ROWS, 4))
+    boxes = [np.asarray(h["obstacles"], float).reshape(-1, 6) for h in holders]
+    box_off[1:] = np.cumsum([b.shape[0] for b in boxes])
+    return box_off, np.ascontiguousarray(np.vstack(boxes)) if n else np.zeros((0, 6)), None
 
 
 def obs_rows_of(obs_sets):
@@ -133,8 +183,9 @@ def obs_rows_of(obs_sets):
 
 
 def scene_batch(queries, obs_size_increase):
-    """The device scene batch of a batch of queries: SceneBatch over the boxes, or PolytopeSceneBatch over the
-    obs_sets (vertex lists from ``obs_points_sets``, enumerated on the device when missing)."""
+    """The device scene batch of a batch of queries (or of shared scenes): SceneBatch over the boxes, or
+    PolytopeSceneBatch over the obs_sets (vertex lists from ``obs_points_sets``, enumerated on the device when
+    missing)."""
     from . import geometry as geo
 
     if query_kind(queries) == "polytopes":
@@ -153,24 +204,20 @@ def rng_state_words(rng):
 
 
 class PackedQueries:
-    """Host arrays of a batch in the layout of bp_plan_in / bp_plan_out (kept alive with the ctypes views)."""
+    """Host arrays of a batch in the layout of bp_plan_in / bp_plan_out (kept alive with the ctypes views).
+    With ``scenes`` (see scene_map) the obstacles are the scenes', packed once (box_off of len(scenes) + 1), and
+    ``query_scene`` is the batch's query -> scene map (else None).  ``scene_arrays``: the scenes already packed
+    (pack_obstacles of the same scenes), for a planner that plans new queries over its resident scenes."""
 
     def __init__(self, queries, obs_size_increase, workspace_max, workspace_min, rng_seeds=None, sample_chunk=32,
-                 want_nodes=True):
+                 want_nodes=True, scenes=None, scene_arrays=None):
         Q = len(queries)
         self.Q = Q
-        self.kind = query_kind(queries)
-        self.box_off = np.zeros(Q + 1, np.int32)
-        if self.kind == "polytopes":
-            rows = [obs_rows_of(q["obs_sets"]) for q in queries]
-            self.box_off[1:] = np.cumsum([r.shape[0] for r in rows])
-            self.obs_rows = np.ascontiguousarray(np.concatenate(rows)) if Q else np.zeros((0, OBS_ROWS, 4))
-            self.boxes = None
-        else:
-            boxes = [np.asarray(q["obstacles"], float).reshape(-1, 6) for q in queries]
-            self.box_off[1:] = np.cumsum([b.shape[0] for b in boxes])
-            self.boxes = np.ascontiguousarray(np.vstack(boxes)) if Q else np.zeros((0, 6))
-            self.obs_rows = None
+        self.query_scene = scene_map(queries, scenes)
+        holders = queries if scenes is None else scenes
+        self.kind = query_kind(holders, "query" if scenes is None else "scene")
+        self.box_off, self.boxes, self.obs_rows = (scene_arrays if scene_arrays is not None else
+                                                   pack_obstacles(holders, self.kind))
         self.ws_min = np.ascontiguousarray(np.asarray(workspace_min, float).reshape(3))
         self.ws_max = np.ascontiguousarray(np.asarray(workspace_max, float).reshape(3))
         self.starts = np.ascontiguousarray([np.asarray(q["start"], float) for q in queries]).reshape(Q, 3)
@@ -280,61 +327,103 @@ class PackedQueries:
 class NativePlanner:
     """A batch of independent planning queries, one scene each, planned in lock step by libbpgeo's native driver.
     The queries carry boxes (``obstacles``) or polytopes (``obs_sets`` [, ``obs_points_sets``]), all of one kind.
+    With ``scenes`` (a list of dicts with those obstacle keys), the queries share them instead: each query carries
+    ``scene``, the index of the scene it plans in, and no obstacles (see scene_map).  Every scene is then packed,
+    ingested and stored on the device once however many queries plan in it, and every query's results are the ones it
+    gets with a copy of its scene of its own.
     The scene batch and the device tables are created once; ``run`` can be called again (same scenes), also with
     new per-query inputs (``queries=``: an MPC loop's replanning calls) over the same obstacles.  When the obstacles
     move, ``update_obstacles`` rewrites the resident scenes in place."""
 
-    def __init__(self, queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0)):
+    def __init__(self, queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0),
+                 scenes=None):
         import torch
 
         from . import _lib
 
-        self.kind = query_kind(queries)          # (a mixed batch fails before anything touches the device)
+        # (a malformed or mixed batch fails before anything touches the device)
+        self.query_scene = scene_map(queries, scenes)
+        self.kind = query_kind(queries) if scenes is None else query_kind(scenes, "scene")
         if not torch.cuda.is_available():
             raise _lib.BpGeoError("boundplanner_b200 needs a CUDA device (no CPU fallback)")
         self._lib = _lib.load()
         self.queries = queries
+        self.scenes = scenes
         self.infl, self.ws_max, self.ws_min = float(obs_size_increase), list(workspace_max), list(workspace_min)
-        self.scene = scene_batch(queries, obs_size_increase)
+        self.scene = scene_batch(queries if scenes is None else scenes, obs_size_increase)
         self._obstacles = None                   # (kind, offsets, rows) of the scenes, for run(queries=...)
+        self._scene_pack = None                  # the shared scenes, packed (pack_obstacles)
         self._h = ctypes.c_void_p(0)
         self._packed = {}
-        _lib.check(self._lib.bp_plan_create(self.scene._h, len(queries), ctypes.byref(self._h)))
+        if scenes is None:
+            _lib.check(self._lib.bp_plan_create(self.scene._h, len(queries), ctypes.byref(self._h)))
+        else:
+            _lib.check(self._lib.bp_plan_create_mapped(self.scene._h, len(queries),
+                                                       self.query_scene.ctypes.data_as(_ip), ctypes.byref(self._h)))
 
-    def update_obstacles(self, queries):
+    def update_obstacles(self, queries, scenes=None):
         """Move the obstacles: the scenes become those of ``queries`` (the constructor's format, as many queries, the
         same obstacle kind; ValueError before the device is touched otherwise), written into the resident scene batch
         in place (SceneBatch / PolytopeSceneBatch.update_scenes), and ``queries`` become the planner's queries.
+        A planner over shared scenes takes the new ``scenes`` instead (as many as before, of the same kind), and
+        ``queries`` must carry the planner's scene indices.
         ``run()`` and ``run(queries=...)`` then plan against the new obstacles.  A failed update leaves the planner
         as it was."""
         if len(queries) != len(self.queries):
             raise ValueError(f"{len(queries)} queries for a planner of {len(self.queries)} scenes")
-        kind = query_kind(queries)
+        if (scenes is None) != (self.scenes is None):
+            raise ValueError("a planner over shared scenes is updated with scenes=, a planner of one scene per query "
+                             "without")
+        holders = queries
+        if scenes is not None:
+            if len(scenes) != len(self.scenes):
+                raise ValueError(f"{len(scenes)} scenes for a planner of {len(self.scenes)} scenes")
+            m = scene_map(queries, scenes)
+            if not np.array_equal(m, self.query_scene):
+                raise ValueError("the queries' scene indices differ from the planner's")
+            holders = scenes
+        kind = query_kind(holders, "query" if scenes is None else "scene")
         if kind != self.kind:
-            raise ValueError(f"the planner's scenes hold {self.kind}, the queries {kind}")
+            raise ValueError(f"the planner's scenes hold {self.kind}, the {'queries' if scenes is None else 'scenes'} "
+                             f"{kind}")
         if kind == "polytopes":
-            n_max = max(len(q["obs_sets"]) for q in queries)
+            n_max = max(len(h["obs_sets"]) for h in holders)
             if n_max > MAX_POLY_OBSTACLES:
                 raise ValueError(f"polytope scenes hold at most {MAX_POLY_OBSTACLES} obstacles (largest scene: {n_max})")
-            self.scene.update_scenes([(q["obs_sets"], q.get("obs_points_sets")) for q in queries])
+            self.scene.update_scenes([(h["obs_sets"], h.get("obs_points_sets")) for h in holders])
         else:
-            self.scene.update_scenes([q["obstacles"] for q in queries])
+            self.scene.update_scenes([h["obstacles"] for h in holders])
         self.queries = queries
+        if scenes is not None:
+            self.scenes = scenes
         self._packed = {}
         self._obstacles = None
+        self._scene_pack = None
 
     @staticmethod
     def _obstacles_of(pk):
         return pk.kind, pk.box_off, pk.boxes if pk.obs_rows is None else pk.obs_rows
 
+    def _scene_arrays(self):
+        """The shared scenes packed once (pack_obstacles), for run(queries=...)."""
+        if self._scene_pack is None:
+            self._scene_pack = pack_obstacles(self.scenes, self.kind)
+        return self._scene_pack
+
     def run(self, rng_seeds=None, sample_chunk=32, want_nodes=True, queries=None):
         """Plan the batch: (results, stats).  queries: new per-query inputs (start, end, r0, r1, first_sample and the
         replanning keys of planner.plan_batch) to plan against the scenes of this planner; their obstacles must be
         the ones it was created with, or last updated to (ValueError otherwise: the host push-out of `end` and the
-        device scene must agree)."""
+        device scene must agree).  Over shared scenes, they carry the planner's scene indices instead (ValueError
+        otherwise)."""
         if queries is not None:
             if len(queries) != len(self.queries):
                 raise ValueError(f"{len(queries)} queries for a planner of {len(self.queries)} scenes")
+            if self.scenes is not None:
+                if not np.array_equal(scene_map(queries, self.scenes), self.query_scene):
+                    raise ValueError("the queries' scene indices differ from the planner's")
+                return self._run(PackedQueries(queries, self.infl, self.ws_max, self.ws_min, rng_seeds, sample_chunk,
+                                               want_nodes, scenes=self.scenes, scene_arrays=self._scene_arrays()))
             pk = PackedQueries(queries, self.infl, self.ws_max, self.ws_min, rng_seeds, sample_chunk, want_nodes)
             if self._obstacles is None:
                 self._obstacles = self._obstacles_of(
@@ -348,7 +437,9 @@ class NativePlanner:
         key = (None if rng_seeds is None else tuple(int(v) for v in rng_seeds), int(sample_chunk), bool(want_nodes))
         pk = self._packed.get(key) if rng_seeds is not None else None
         if pk is None:
-            pk = PackedQueries(self.queries, self.infl, self.ws_max, self.ws_min, rng_seeds, sample_chunk, want_nodes)
+            pk = PackedQueries(self.queries, self.infl, self.ws_max, self.ws_min, rng_seeds, sample_chunk, want_nodes,
+                               scenes=self.scenes,
+                               scene_arrays=self._scene_arrays() if self.scenes is not None else None)
             if rng_seeds is not None:
                 self._packed = {key: pk}
         return self._run(pk)
@@ -375,9 +466,10 @@ class NativePlanner:
 
 
 def plan_batch_native(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0),
-                      rng_seeds=None, sample_chunk=32):
-    """Drop-in for ``planner.plan_batch``: (results, stats).  Box or polytope queries, one kind per batch."""
-    pl = NativePlanner(queries, obs_size_increase, workspace_max, workspace_min)
+                      rng_seeds=None, sample_chunk=32, scenes=None):
+    """Drop-in for ``planner.plan_batch``: (results, stats).  Box or polytope queries, one kind per batch; with
+    ``scenes``, queries over shared scenes (see NativePlanner)."""
+    pl = NativePlanner(queries, obs_size_increase, workspace_max, workspace_min, scenes=scenes)
     try:
         return pl.run(rng_seeds, sample_chunk)
     finally:

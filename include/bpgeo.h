@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define BPGEO_ABI_VERSION 5
+#define BPGEO_ABI_VERSION 6
 #define BP_MAX_ROWS 48 /* hard cap on rows per convex set (reference MVIE cap: 20, quirk Q5) */
 
 typedef struct bp_scene bp_scene;
@@ -343,7 +343,9 @@ typedef struct {
   int Q;
   const double* boxes;        /* all scenes back to back [sum n_obs, 6] (lb, ub), as given to bp_scene_create_batch;
                                  NULL when obs_rows is set */
-  const int* box_off;         /* [Q+1] obstacle offsets of every query (boxes or polytopes) */
+  const int* box_off;         /* [Q+1] obstacle offsets of every query (boxes or polytopes); for a plan from
+                                 bp_plan_create_mapped [n_scenes+1] offsets of every scene, whose obstacles boxes /
+                                 obs_rows hold once however many queries plan in it */
   double inflate;             /* obs_size_increase */
   const double* ws_min;       /* [3] */
   const double* ws_max;       /* [3] */
@@ -392,12 +394,20 @@ typedef struct {
   double* p_horizon_max;      /* [Q,3] or NULL (ABI 4): p_horizon[idx] of every replanning query */
 } bp_plan_out;
 
-/* bp_plan_create takes a box or a polytope scene batch with one scene per query; the per-scene limits of the kernels
+/* bp_plan_create takes a box or a polytope scene batch with one scene per query (query q plans in scene q: the
+ * identity map of bp_plan_create_mapped); the per-scene limits of the kernels
  * the rounds launch are checked here, not in the middle of a run (polytope scenes: at most 16384 obstacles).  The plan
  * keeps the scene batch, not a copy: after bp_scene_update_batch / bp_scene_update_polytopes_batch, bp_plan_run plans
- * against the new obstacles, checks its inputs against the batch's current offsets and re-checks the limit. */
+ * against the new obstacles, checks its inputs against the batch's current offsets and re-checks the limit.
+ * bp_plan_create_mapped (ABI 6) plans many queries over shared scenes: query q plans in scene query_scene_host[q] of a
+ * batch of any n_scenes >= 1 (scenes no query uses are allowed); every entry must lie in [0, n_scenes), else the call
+ * fails and names the query.  The plan keeps a copy of the map.  bp_plan_run then takes every scene's obstacles once
+ * (bp_plan_in::box_off of n_scenes + 1 entries, checked scene by scene against the batch); every other field of
+ * bp_plan_in stays per query.  A query planned in a shared scene gives the same results, bit for bit, as the same query
+ * in a scene batch of one copy per query. */
 typedef struct bp_plan bp_plan;
 int bp_plan_create(const bp_scene* scene_batch, int Q, bp_plan** out);
+int bp_plan_create_mapped(const bp_scene* scene_batch, int Q, const int* query_scene_host /*[Q]*/, bp_plan** out);
 int bp_plan_run(bp_plan* plan, const bp_plan_in* in, bp_plan_out* out, void* stream);
 int bp_plan_destroy(bp_plan* plan);
 

@@ -1189,7 +1189,7 @@ __global__ void __launch_bounds__(512) k_poly_point(SceneView sc_all, PolyParams
 // ---------------------------------------------------------------------------
 // Exact axis-aligned bounding box of the polytope {A x <= b} (ms rows) by vertex enumeration over all row
 // triples, by the 128 threads of a CTA; rows may live in global or shared memory.  out6 = lo[3] | hi[3]
-// (-inf / +inf when no vertex is found: unbounded or empty description -- never reject on such a set).
+// (-inf / +inf when the description is unbounded or has no vertex -- never reject on such a set).
 // Used by k_set_aabb and by the epilogue of the fused set build (same code, same bits).
 #define BP_AABB_EPS 1e-9
 __device__ __forceinline__ void cta_set_aabb(const double* As, const double* bs, int ms, double (*red)[6],
@@ -1231,6 +1231,32 @@ __device__ __forceinline__ void cta_set_aabb(const double* As, const double* bs,
       lo[2] = fmin(lo[2], v2); hi[2] = fmax(hi[2], v2);
     }
   }
+  // A set with a vertex can still be unbounded (a cone, a prism closed at one end): the box of its vertices would
+  // then be too small, and the pre-tests would reject pairs that meet the set away from them.  Such a set has a
+  // recession direction d != 0 with A d <= 0; when the rows span R^3 (else there is no vertex) that cone is pointed
+  // and has an extreme ray d = +-(a_i x a_j), so every row pair is tried.  The test is loose on purpose: a set that
+  // is bounded only to within rounding loses its box, which costs the pre-tests and never a pair.
+  bool ray = false;
+  const int npair = ms * (ms - 1) / 2;
+  for (int t = threadIdx.x; t < npair && !ray; t += 128) {
+    int i = 0, rem = t;
+    for (;;) { const int c = ms - 1 - i; if (rem < c) break; rem -= c; ++i; }
+    const int j = i + 1 + rem;
+    const double a0 = As[3 * i], a1 = As[3 * i + 1], a2 = As[3 * i + 2];
+    const double c0 = As[3 * j], c1 = As[3 * j + 1], c2 = As[3 * j + 2];
+    const double d0 = a1 * c2 - a2 * c1, d1 = a2 * c0 - a0 * c2, d2 = a0 * c1 - a1 * c0;
+    const double dd = d0 * d0 + d1 * d1 + d2 * d2;
+    if (!(dd > 1e-24 * (a0 * a0 + a1 * a1 + a2 * a2) * (c0 * c0 + c1 * c1 + c2 * c2))) continue;   // parallel rows
+    bool pos = true, neg = true;                          // A d <= 0 / A (-d) <= 0, up to rounding
+    for (int r = 0; r < ms && (pos || neg); ++r) {
+      const double q0 = As[3 * r], q1 = As[3 * r + 1], q2 = As[3 * r + 2];
+      const double q = q0 * d0 + q1 * d1 + q2 * d2;
+      const double lim = BP_AABB_EPS * (fabs(q0 * d0) + fabs(q1 * d1) + fabs(q2 * d2));
+      if (q > lim) pos = false;
+      if (-q > lim) neg = false;
+    }
+    ray = pos || neg;
+  }
 #pragma unroll
   for (int k = 0; k < 3; ++k) {
 #pragma unroll
@@ -1243,14 +1269,14 @@ __device__ __forceinline__ void cta_set_aabb(const double* As, const double* bs,
 #pragma unroll
     for (int k = 0; k < 3; ++k) { red[warp][k] = lo[k]; red[warp][3 + k] = hi[k]; }
   }
-  __syncthreads();
+  const int unbounded = __syncthreads_or(ray);
   if (threadIdx.x == 0) {
 #pragma unroll
     for (int w = 1; w < 4; ++w) {
 #pragma unroll
       for (int k = 0; k < 3; ++k) { lo[k] = fmin(lo[k], red[w][k]); hi[k] = fmax(hi[k], red[w][3 + k]); }
     }
-    const bool none = !(lo[0] <= hi[0]);
+    const bool none = !(lo[0] <= hi[0]) || unbounded;
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       out6[k] = none ? -BP_INF : lo[k];

@@ -13,7 +13,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libbpgeo.so")
 
 BP_MAX_ROWS = 48
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 STATUS_OK = 0
 STATUS_ELLIPSE_VIOLATION = 1
@@ -77,6 +77,8 @@ SIGNATURES = {
     "bp_pair_feasible": (_i, [_vp, _vp, _vp, _i, _i, _d, _i, _i, _vp, _vp, _vp, _vp, _sz, _vp]),
     "bp_pair_feasible_stages": (_i, [_vp, _vp, _vp, _i, _i, _d, _i, _i, _vp, _vp, _vp, _sz, _vp,
                                     _c.POINTER(_c.c_float)]),
+    "bp_sets_obstacles_workspace_bytes": (_sz, [_i]),
+    "bp_sets_obstacles": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _d, _vp, _vp, _sz, _vp]),
     "bp_reduce_ineqs": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "bp_check_fit": (_i, [_vp, _vp, _vp, _i, _i, _vp, _i, _vp, _vp, _dp, _i, _d, _vp, _vp, _vp]),
     "bp_project_points": (_i, [_vp, _vp, _vp, _i, _i, _vp, _i, _vp, _vp, _vp, _vp]),
@@ -96,6 +98,7 @@ SIGNATURES = {
     "bp_plan_create": (_i, [_vp, _i, _c.POINTER(_vp)]),
     "bp_plan_create_mapped": (_i, [_vp, _i, _c.POINTER(_c.c_int), _c.POINTER(_vp)]),
     "bp_plan_run": (_i, [_vp, _vp, _vp, _vp]),
+    "bp_plan_run_active": (_i, [_vp, _vp, _c.POINTER(_c.c_int), _vp, _vp]),
     "bp_plan_destroy": (_i, [_vp]),
 }
 

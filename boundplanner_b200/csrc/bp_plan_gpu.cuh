@@ -601,7 +601,10 @@ int bp_plan_create_mapped(const bp_scene* scene_batch, int Q, const int* query_s
                      out);
 }
 
-int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* stream) {
+}  // extern "C"
+
+// bp_plan_run / bp_plan_run_active: active [Q] or NULL (every query)
+static int plan_run(bp_plan* pl, const bp_plan_in* in, const int* active, bp_plan_out* out, void* stream) {
   if (!pl || !in || !out || in->Q != pl->Q || (!in->boxes && !in->obs_rows) || !in->box_off || !in->ws_min || !in->ws_max || !in->starts ||
       !in->ends || !in->l_ee || !in->l_ee_end || !in->ee_samples || !in->rng || !out->err_kind || !out->err_msg ||
       !out->path || !out->path_len || !out->set_ids || !out->n_ids || !out->p_via || !out->n_via || !out->n_nodes ||
@@ -634,7 +637,7 @@ int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* strea
   bpplan::Params par;
   std::vector<bpplan::Query> qs;
   const auto t_run0 = std::chrono::steady_clock::now();
-  bpplan::load_queries(*in, par, qs, pl->query_scene.data());
+  bpplan::load_queries(*in, par, qs, pl->query_scene.data(), active);
   const auto t_run1 = std::chrono::steady_clock::now();
   // the work queued on the caller's stream so far precedes the run on every lane
   BP_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
@@ -659,13 +662,13 @@ int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* strea
   bpplan::RunStats st;
   std::vector<int> fin(qs.size(), -1);
   std::vector<double> fin_ms(qs.size(), -1.0);
-  const int rc = bpplan::run_lockstep(qs, *pl, par, &st, fin.data(), fin_ms.data());
+  const int rc = bpplan::run_lockstep(qs, *pl, par, &st, fin.data(), fin_ms.data(), active);
   if (rc) {
     for (int l = 0; l < pl->L; ++l) cudaStreamSynchronize(pl->lane[l].stream);       // nothing of the run stays in flight
     return bp_fail(pl->error.empty() ? "bp_plan_run: executor failed" : pl->error.c_str());
   }
   const auto t_run2 = std::chrono::steady_clock::now();
-  bpplan::store_results(qs, st, fin.data(), fin_ms.data(), *out);
+  bpplan::store_results(qs, st, fin.data(), fin_ms.data(), *out, active);
   const auto t_run3 = std::chrono::steady_clock::now();
   long long chains = 0, wait = 0, pack = 0, launch = 0, unpack = 0;
   for (int l = 0; l < pl->L; ++l) {
@@ -682,6 +685,16 @@ int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* strea
             std::chrono::duration<double, std::milli>(t_run3 - t_run2).count(),
             std::chrono::duration<double, std::milli>(t_run3 - t_run0).count());
   return 0;
+}
+
+extern "C" {
+
+int bp_plan_run(bp_plan* pl, const bp_plan_in* in, bp_plan_out* out, void* stream) {
+  return plan_run(pl, in, nullptr, out, stream);
+}
+
+int bp_plan_run_active(bp_plan* pl, const bp_plan_in* in, const int* active_host, bp_plan_out* out, void* stream) {
+  return plan_run(pl, in, active_host, out, stream);
 }
 
 int bp_plan_destroy(bp_plan* pl) {

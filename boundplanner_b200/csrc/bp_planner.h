@@ -935,21 +935,30 @@ struct RunStats {
   double gather_ms = 0.0, resume_ms = 0.0;   // host time: building the rounds / resuming the state machines
 };
 
-// Advance all queries until every one is finished.  The queries are dealt to the executor's lanes (query i -> lane
-// i mod L); every lane is a lock-step group of its own: each of its rounds collects the pending request of every
-// live query of the lane, hands them to the executor and resumes the queries with the answers.  finish_round[q]
-// (or null) receives the round of its lane in which query q finished, finish_ms[q] (or null) the wall time since
-// the start of the run at that moment.
+// Advance all queries (or the active ones) until every one is finished.  The queries are dealt to the executor's
+// lanes; every lane is a lock-step group of its own: each of its rounds collects the pending request of every
+// live query of the lane, hands them to the executor and resumes the queries with the answers.  A query's requests
+// and answers do not depend on the other queries or on its lane, so an active query finishes as it does in a run of
+// the whole batch.  finish_round[q] (or null) receives the round of its lane in which query q finished, finish_ms[q]
+// (or null) the wall time since the start of the run at that moment.
 inline int run_lockstep(std::vector<Query>& qs, Executor& ex, const Params& par, RunStats* stats, int* finish_round,
-                        double* finish_ms = nullptr) {
-  const int L = std::max(1, std::min(ex.lanes(), (int)qs.size()));
+                        double* finish_ms = nullptr, const int* active = nullptr) {
+  // the queries that run: all, or those with active[i] != 0 (the others are not touched); the k-th of them goes to
+  // lane k mod L, so that a subset keeps every lane busy (without `active`: query i -> lane i mod L)
+  std::vector<int> run;
+  run.reserve(qs.size());
+  for (size_t i = 0; i < qs.size(); ++i)
+    if (!active || active[i]) run.push_back((int)i);
+  const int L = std::max(1, std::min(ex.lanes(), (int)run.size()));
+  std::vector<std::vector<int>> members(L);
+  for (size_t k = 0; k < run.size(); ++k) members[k % (size_t)L].push_back(run[k]);
   std::vector<Round> rounds_(L);
   std::vector<int> n_rounds(L, 0);
   std::vector<char> in_flight(L, 0);
   std::vector<size_t> committed(qs.size(), 0);
   const auto t_start = std::chrono::steady_clock::now();
   auto now_ms = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count(); };
-  for (auto& q : qs) q.resume(nullptr, nullptr, nullptr, nullptr, 0);
+  for (int i : run) qs[(size_t)i].resume(nullptr, nullptr, nullptr, nullptr, 0);
 
   // gather the pending requests of lane l into its round and submit it; returns the number of live queries (or < 0)
   auto launch = [&](int l) -> int {
@@ -957,7 +966,7 @@ inline int run_lockstep(std::vector<Query>& qs, Executor& ex, const Params& par,
     Round& r = rounds_[l];
     r.clear();
     size_t live = 0;
-    for (size_t i = (size_t)l; i < qs.size(); i += (size_t)L) {
+    for (const int i : members[(size_t)l]) {
       Query& q = qs[i];
       // nodes added since the last round go to the executor's tables first
       for (; committed[i] < q.nodes.size(); ++committed[i]) ex.commit_node(l, q.qid, (int)committed[i], q.nodes[committed[i]]);
@@ -1006,7 +1015,7 @@ inline int run_lockstep(std::vector<Query>& qs, Executor& ex, const Params& par,
     }
     ++n_rounds[l];
     if (n_rounds[l] > par.max_rounds) {
-      for (size_t i = (size_t)l; i < qs.size(); i += (size_t)L)
+      for (const int i : members[(size_t)l])
         if (!qs[i].finished) qs[i].fail(ERR_RUNTIME, "lock-step round limit reached");
       return 0;
     }
@@ -1053,7 +1062,7 @@ inline int run_lockstep(std::vector<Query>& qs, Executor& ex, const Params& par,
       qs[(size_t)t.owner].resume(t.sa, t.ea, t.pa, t.path, t.path_len);
     };
     pool.parallel_for(tasks.size(), fn);
-    for (size_t i = (size_t)l; i < qs.size(); i += (size_t)L)
+    for (const int i : members[(size_t)l])
       if (!qs[i].finished) qs[i].rounds = n_rounds[l];
     if (stats) stats->resume_ms += now_ms() - t_d0;
   };
@@ -1127,7 +1136,9 @@ inline std::string check_replan_inputs(const bp_plan_in& in) {
 
 // query_scene [Q] (or NULL: query q plans in scene q): query q's obstacles are scene query_scene[q]'s, i.e.
 // in.box_off has one entry per scene + 1 and the boxes / obs_rows of every scene appear once
-inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& qs, const int* query_scene = nullptr) {
+// active [Q] (or NULL: all): a query with active[q] == 0 is left default-constructed (no state machine)
+inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& qs, const int* query_scene = nullptr,
+                         const int* active = nullptr) {
   par.obs_size_increase = in.inflate;
   for (int k = 0; k < 3; ++k) { par.ws_min[k] = in.ws_min[k]; par.ws_max[k] = in.ws_max[k]; }
   if (in.sample_chunk > 0) par.sample_chunk = in.sample_chunk;
@@ -1143,6 +1154,7 @@ inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& 
   qs.clear();
   qs.resize((size_t)in.Q);
   for (int q = 0; q < in.Q; ++q) {
+    if (active && !active[q]) continue;
     QueryInput qi;
     const int s = query_scene ? query_scene[q] : q;
     qi.boxes = in.obs_rows ? nullptr : in.boxes + 6 * (size_t)in.box_off[s];
@@ -1168,9 +1180,14 @@ inline void load_queries(const bp_plan_in& in, Params& par, std::vector<Query>& 
   }
 }
 
+// active [Q] (or NULL: all): the outputs of a query with active[q] == 0 are not written, except finish_round[q] = -1
 inline void store_results(const std::vector<Query>& qs, const RunStats& st, const int* finish_round, const double* finish_ms,
-                          bp_plan_out& out) {
+                          bp_plan_out& out, const int* active = nullptr) {
   for (size_t q = 0; q < qs.size(); ++q) {
+    if (active && !active[q]) {
+      out.finish_round[q] = -1;
+      continue;
+    }
     const Query& Qy = qs[q];
     out.err_kind[q] = Qy.err_kind;
     std::snprintf(out.err_msg + 160 * q, 160, "%s", Qy.err_msg.c_str());

@@ -2462,6 +2462,117 @@ __global__ void __launch_bounds__(256) k_pair_list(const double* __restrict__ A,
 }
 
 // ---------------------------------------------------------------------------
+// Set-obstacle hit test (bp_sets_obstacles): which obstacle of its scene, if any, does a planned set meet after the
+// obstacles moved?  Set s is hit by obstacle o when set_intersection([A_s, b_s], [A_o, b_o], tol) succeeds -- the
+// decision of an edge of the set graph.  The obstacle rows are the scene's: box o gives [I; -I] x <= [ub; -lb] from
+// the inflated columns (make_box + obs_size_increase, bit for bit: -(lb - r) == -lb + r in fp64), a polytope its
+// nrows[o] rows.  One warp per set walks its scene's obstacles in index order, 32 at a time: every lane tests one
+// obstacle's box against the set's (k_set_aabb), the survivors go through the warp LP one after another in index
+// order, and the warp stops at the first hit, which is then the lowest index.
+// ---------------------------------------------------------------------------
+// rows of the set, then of obstacle o (box or polytope), every offset shrunk by tol
+struct BpSetObstacleRows {
+  const double *As, *bs;
+  int ms;
+  const double* prow;    // [nrows, 4] rows of a polytope obstacle, or NULL: the box lo[3] | hi[3] at box
+  const double* box;
+  double tol;
+  __device__ __forceinline__ void operator()(int i, double* a, double& c) const {
+    if (i < ms) {
+      a[0] = As[3 * i]; a[1] = As[3 * i + 1]; a[2] = As[3 * i + 2];
+      c = bs[i] - tol;
+      return;
+    }
+    const int r = i - ms;
+    if (prow) {
+      a[0] = prow[4 * r]; a[1] = prow[4 * r + 1]; a[2] = prow[4 * r + 2];
+      c = prow[4 * r + 3] - tol;
+      return;
+    }
+    const int k = r < 3 ? r : r - 3;
+    const double sg = r < 3 ? 1.0 : -1.0;
+    a[0] = k == 0 ? sg : 0.0; a[1] = k == 1 ? sg : 0.0; a[2] = k == 2 ? sg : 0.0;
+    c = (r < 3 ? box[3 + k] : -box[k]) - tol;
+  }
+};
+
+// (the boxes, the start point and the region of the LP live in shared memory: held in registers next to the
+// two-rows-per-lane LP they spilled)
+__global__ void __launch_bounds__(256) k_sets_obstacles(SceneView sc, int n_scenes, const int* __restrict__ set_scene,
+                                                        const double* __restrict__ A, const double* __restrict__ b,
+                                                        const int* __restrict__ m, int S, int m_max, double tol,
+                                                        const double* __restrict__ aabb, int* __restrict__ first_hit) {
+  __shared__ double scratch[8][BP_LP_SCRATCH_DOUBLES];
+  __shared__ double boxes[8][24];    // set box [0, 6) | obstacle box [6, 12) | LP region [12, 18) | start point [18, 21)
+  const unsigned full = 0xffffffffu;
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+  const int s = blockIdx.x * 8 + wib;
+  if (s >= S) return;
+  const int k = set_scene ? set_scene[s] : 0;
+  if (k < 0 || k >= n_scenes) {
+    if (lane == 0) first_hit[s] = -2;
+    return;
+  }
+  const int o0 = sc.seg_off ? sc.seg_off[k] : 0;
+  const int n = sc.seg_off ? sc.seg_off[k + 1] - o0 : sc.n;
+  double* wb = boxes[wib];
+  if (lane < 6) wb[lane] = __ldg(aabb + (size_t)s * 6 + lane);
+  // this lane's axis (lanes 0-2) of the obstacle columns
+  const int ax = lane < 3 ? lane : 0;
+  const double* lb = ax == 0 ? sc.lb[0] : (ax == 1 ? sc.lb[1] : sc.lb[2]);
+  const double* ub = ax == 0 ? sc.ub[0] : (ax == 1 ? sc.ub[1] : sc.ub[2]);
+  __syncwarp();
+  BpSetObstacleRows rows;
+  rows.As = A + (size_t)s * m_max * 3;
+  rows.bs = b + (size_t)s * m_max;
+  rows.ms = min(max(m[s], 0), m_max);
+  rows.box = wb + 6;
+  rows.tol = tol;
+  int hit = -1;
+  for (int base = 0; base < n && hit < 0; base += 32) {
+    const int j = base + lane;
+    bool keep = false;
+    if (j < n) {
+      keep = true;
+#pragma unroll
+      for (int e = 0; e < 3; ++e) {
+        const double lo = __ldg(sc.lb[e] + o0 + j), hi = __ldg(sc.ub[e] + o0 + j);
+        if (wb[e] > hi + BP_AABB_EPS || lo > wb[3 + e] + BP_AABB_EPS) keep = false;
+      }
+    }
+    unsigned int mask = __ballot_sync(full, keep);
+    while (mask && hit < 0) {
+      const int f = __ffs(mask) - 1;
+      mask &= mask - 1u;
+      const int o = o0 + base + f;
+      bool finite = true;
+      if (lane < 3) {
+        const double olo = __ldg(lb + o), ohi = __ldg(ub + o);
+        const double lo = fmax(wb[lane], olo), hi = fmin(wb[3 + lane], ohi);
+        const double x0 = 0.5 * (lo + hi);
+        wb[6 + lane] = olo; wb[9 + lane] = ohi;
+        wb[12 + lane] = lo - BP_AABB_EPS; wb[15 + lane] = hi + BP_AABB_EPS;   // every common point lies in this box
+        wb[18 + lane] = fabs(x0) < 1e6 ? x0 : 0.0;                          // start at the middle of the overlap
+        finite = fabs(lo) < 1e6 && fabs(hi) < 1e6;
+      }
+      const bool have_region = __all_sync(full, finite);
+      __syncwarp();
+      rows.prow = sc.rows ? sc.rows + (size_t)o * BP_OBS_ROWS * 4 : nullptr;
+      const int mt = rows.ms + (sc.rows ? __ldg(sc.nrows + o) : 6);
+      const double* reg = have_region ? wb + 12 : nullptr;
+      // at most 48 + 15 rows: one or two rows per lane
+      const int res = mt <= 32 ? bp_lp_feasible_warp_impl<1>(rows, mt, scratch[wib], nullptr, nullptr, wb + 18,
+                                                              BP_LP_T0_SCALE, reg)
+                               : bp_lp_feasible_warp_impl<2>(rows, mt, scratch[wib], nullptr, nullptr, wb + 18,
+                                                              BP_LP_T0_SCALE, reg);
+      if (res) hit = base + f;
+      __syncwarp();
+    }
+  }
+  if (lane == 0) first_hit[s] = hit;
+}
+
+// ---------------------------------------------------------------------------
 // K8 ("next" row 1): redundancy removal of a set's rows.
 // Replaces reduce_ineqs (bound_planner/utils/util_functions.py:82-88; cddlib
 // dd_MatrixRedundancyRemove): a row is kept iff it supports a facet, i.e. the
@@ -4197,6 +4308,26 @@ int bp_pairs_feasible_list(const double* A_dev, const double* b_dev, const int* 
   k_set_aabb<<<S, 128, 0, stream>>>(A_dev, b_dev, m_dev, S, m_max, aabb);
   k_pair_list<<<(P + 7) / 8, 256, 0, stream>>>(A_dev, b_dev, m_dev, m_max, tol, aabb, (const int2*)pairs_dev, P,
                                                result_dev, x_feas_dev);
+  BP_CUDA(cudaGetLastError());
+  return 0;
+}
+
+size_t bp_sets_obstacles_workspace_bytes(int S) { return sizeof(double) * 6 * (size_t)(S > 0 ? S : 0); }
+
+int bp_sets_obstacles(const bp_scene* scene, const int* set_scene_dev, const double* A_dev, const double* b_dev,
+                      const int* m_dev, int S, int m_max, double tol, int* first_hit_dev, void* workspace_dev,
+                      size_t workspace_bytes, void* stream_) {
+  if (!scene || S < 0 || m_max < 1 || m_max > BP_MAX_ROWS) return bp_fail("bp_sets_obstacles: bad arguments (m_max 1 .. 48)");
+  if (!(tol >= 0.0) || !isfinite(tol)) return bp_fail("bp_sets_obstacles: tol must be finite and >= 0");
+  if (S == 0) return 0;
+  if (!A_dev || !b_dev || !m_dev || !first_hit_dev) return bp_fail("bp_sets_obstacles: bad arguments");
+  if (!workspace_dev || workspace_bytes < bp_sets_obstacles_workspace_bytes(S))
+    return bp_fail("bp_sets_obstacles: workspace too small");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  double* aabb = (double*)workspace_dev;
+  k_set_aabb<<<S, 128, 0, stream>>>(A_dev, b_dev, m_dev, S, m_max, aabb);
+  k_sets_obstacles<<<(S + 7) / 8, 256, 0, stream>>>(view_of(scene), scene->seg_off ? scene->n_seg : 1, set_scene_dev,
+                                                    A_dev, b_dev, m_dev, S, m_max, tol, aabb, first_hit_dev);
   BP_CUDA(cudaGetLastError());
   return 0;
 }

@@ -626,6 +626,26 @@ def pairs_feasible_list(A, b, m, pairs, tol=0.01):
     return res.bool(), x
 
 
+def sets_obstacle_hits(scene, A, b, m, set_scene=None, tol=1e-3):
+    """Which obstacle of its scene does each of S sets meet (bp_sets_obstacles)?  A [S,m_max,3], b [S,m_max], m [S]
+    (padded rows A = 0, b = 10 allowed), set_scene [S] (scene index of every set in a scene batch; None: scene 0).
+    Returns first_hit, int32 [S] on the device: the lowest obstacle index (local to the set's scene) for which
+    set_intersection([A_s, b_s], [A_o, b_o], tol) (BoundPlanner.py:774-787) succeeds, -1 where none does, -2 where
+    set_scene lies outside the batch.  Box or polytope scenes, single scenes and batches."""
+    lib = _lib.load()
+    A = _dev(A)
+    S, m_max = A.shape[0], A.shape[1]
+    b = _dev(b).reshape(S, m_max)
+    m = _dev(m, torch.int32).reshape(S)
+    if set_scene is not None:
+        set_scene = _dev(set_scene, torch.int32).reshape(S)
+    out = torch.empty((S,), dtype=torch.int32, device="cuda")
+    work = torch.empty((max(lib.bp_sets_obstacles_workspace_bytes(S), 1),), dtype=torch.uint8, device="cuda")
+    check(lib.bp_sets_obstacles(scene._h, _ptr(set_scene), _ptr(A), _ptr(b), _ptr(m), S, m_max, float(tol), _ptr(out),
+                                _ptr(work), work.numel(), _stream()))
+    return out
+
+
 def sample_filter(scene, cand, A=None, b=None, m=None, set_off=None, item_scene=None, want_flags=False):
     """Rejection loop of plan_convex_set_path (BoundPlanner.py:459-478) for Q queries: cand [Q,C,3] candidate
     points in draw order; known sets of query q are rows set_off[q]:set_off[q+1] of (A, b, m).

@@ -954,7 +954,7 @@ def _planned(res, pl):
 
 
 def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0),
-               rng_seeds=None, executor=None, scenes=None):
+               rng_seeds=None, executor=None, scenes=None, active=None):
     """Plan many independent queries in lock step.
 
     queries: list of dicts(obstacles [N,6], start, end, r0, r1[, first_sample]); or, for polytope obstacles,
@@ -968,10 +968,13 @@ def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), w
     for its next call) and, when it replanned, ``p_horizon_max``.
     scenes: queries over shared scenes (planner_native.scene_map): a list of dicts with the obstacle keys above, each
     query carrying ``scene`` (its index) instead; every scene is stored on the device, and its host obstacle sets
-    built, once."""
-    from .planner_native import query_kind, scene_map
+    built, once.
+    active: [Q] flags (or None: all): only the queries with a true flag are planned, each as in a run of the whole
+    batch; the result of a skipped query is None (planner_native.NativePlanner.run takes the same argument)."""
+    from .planner_native import active_mask, query_kind, scene_map
 
     query_scene = scene_map(queries, scenes)
+    active = active_mask(active, len(queries))
     holders = queries if scenes is None else scenes
     polytopes = query_kind(holders, "query" if scenes is None else "scene") == "polytopes"
     if executor is None:
@@ -994,6 +997,9 @@ def plan_batch(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), w
     planners, gens, pending, results = [], {}, {}, [None] * len(queries)
     finish = [0.0] * len(queries)              # seconds after the start of the batch at which query i was answered
     for i, q in enumerate(queries):
+        if active is not None and not active[i]:
+            planners.append(None)
+            continue
         ob = obs_of(i)
         pl = SetSequencePlanner(() if polytopes else ob["obstacles"], obs_size_increase, workspace_max, workspace_min,
                                 rng=np.random.default_rng(rng_seeds[i] if rng_seeds is not None else None),

@@ -83,6 +83,53 @@ def replan_arrays(queries):
                 prev_row_off=row_off, prev_rows=np.ascontiguousarray(np.concatenate(rows)) if rows else np.zeros((0, 4)))
 
 
+def active_mask(active, Q):
+    """The ``active`` argument of the batched drivers as int32 [Q] (None stays None); ValueError for another
+    length."""
+    if active is None:
+        return None
+    a = np.asarray(active).reshape(-1)
+    if a.shape[0] != Q:
+        raise ValueError(f"active has {a.shape[0]} entries for {Q} queries")
+    return np.ascontiguousarray(a.astype(bool).astype(np.int32))
+
+
+def pack_corridors(sets, query_scene):
+    """Host packing of NativePlanner.corridor_hits: (buffer uint8, offsets of A [S,m_max,3] | b [S,m_max] | m [S] |
+    set_scene [S] in it, S, m_max, per-query (first, count) or None).  Sets are padded with rows A = 0, b = 10.
+    ValueError for a set without rows or with more than 48 rows, or rows and offsets of different counts."""
+    spans, A_list, b_list, scene_of = [], [], [], []
+    for i, qs in enumerate(sets):
+        if qs is None:
+            spans.append(None)
+            continue
+        spans.append((len(A_list), len(qs)))
+        for a_set, b_set in qs:
+            a_set = np.asarray(a_set, float).reshape(-1, 3)
+            b_set = np.asarray(b_set, float).reshape(-1)
+            if not 1 <= a_set.shape[0] <= SET_ROWS or b_set.shape[0] != a_set.shape[0]:
+                raise ValueError(f"query {i}: a set has {a_set.shape[0]} rows (1 .. {SET_ROWS}, one b each)")
+            A_list.append(a_set)
+            b_list.append(b_set)
+            scene_of.append(i if query_scene is None else int(query_scene[i]))
+    S = len(A_list)
+    m_max = max((a.shape[0] for a in A_list), default=1)
+    sizes = (8 * S * m_max * 3, 8 * S * m_max, 4 * S, 4 * S)
+    offs = np.concatenate(([0], np.cumsum([(n + 15) // 16 * 16 for n in sizes])))
+    buf = np.zeros(int(offs[-1]), np.uint8)
+    A = buf[offs[0]: offs[0] + sizes[0]].view(np.float64).reshape(S, m_max, 3)
+    b = buf[offs[1]: offs[1] + sizes[1]].view(np.float64).reshape(S, m_max)
+    b[:] = 10.0
+    m = buf[offs[2]: offs[2] + sizes[2]].view(np.int32)
+    sc = buf[offs[3]: offs[3] + sizes[3]].view(np.int32)
+    for k, (a_set, b_set) in enumerate(zip(A_list, b_list)):
+        A[k, : a_set.shape[0]] = a_set
+        b[k, : b_set.shape[0]] = b_set
+        m[k] = a_set.shape[0]
+    sc[:] = scene_of
+    return buf, [int(o) for o in offs[:4]], S, m_max, spans
+
+
 def _rodrigues(omega, phi):
     k = np.array([[0.0, -omega[2], omega[1]], [omega[2], 0.0, -omega[0]], [-omega[1], omega[0], 0.0]])
     return np.eye(3) + np.sin(phi) * k + (1.0 - np.cos(phi)) * (k @ k)
@@ -289,9 +336,9 @@ class PackedQueries:
                              self.stats.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)),
                              self.p_horizon_max.ctypes.data_as(_dp))
 
-    def results(self):
+    def results(self, active=None):
         """Per query: dict(path, set_ids, sets_via, p_via, n_nodes, n_inter, n_edges) or the exception the Python
-        planner raises for it.  With the node sets (want_nodes), a planned query also gets ``sets_via_prev``: what the
+        planner raises for it (None for a query that ``active`` skipped).  With the node sets (want_nodes), a planned query also gets ``sets_via_prev``: what the
         planner keeps for its next call -- sets_via, or after the early exit of :361-375 (path [0]) the start set
         padded to 15 rows (:371-372).  A replanning query also gets ``p_horizon_max``."""
         from .utils import normalize_set_size
@@ -299,6 +346,9 @@ class PackedQueries:
         out = []
         raw = self.err_msg.raw
         for q in range(self.Q):
+            if active is not None and not active[q]:
+                out.append(None)
+                continue
             if self.err_kind[q]:
                 msg = raw[160 * q: 160 * (q + 1)].split(b"\0", 1)[0].decode()
                 out.append(_ERRORS[int(self.err_kind[q])](msg))
@@ -410,12 +460,52 @@ class NativePlanner:
             self._scene_pack = pack_obstacles(self.scenes, self.kind)
         return self._scene_pack
 
-    def run(self, rng_seeds=None, sample_chunk=32, want_nodes=True, queries=None):
+    def corridor_hits(self, sets, tol=1e-3):
+        """Check corridors against the resident scenes (after update_obstacles, say): ``sets`` has one entry per
+        query, a list of [A, b] (e.g. a result's ``sets_via_prev``) or None.  Every set is tested against the
+        obstacles of its query's scene (geometry.sets_obstacle_hits: the set and an obstacle, each shrunk by tol,
+        share a point).  Returns per query None or np.int32 [n_sets]: the lowest index of an obstacle of the scene
+        that hits the set, -1 where none does.  One host-to-device copy, one kernel chain and one device-to-host copy;
+        ``corridor_events`` are CUDA events recorded around the library call.  ValueError, before the device is
+        touched, for another number of entries than queries or a set without rows or with more than 48 rows."""
+        import torch
+
+        from . import _lib
+
+        if len(sets) != len(self.queries):
+            raise ValueError(f"{len(sets)} corridors for a planner of {len(self.queries)} queries")
+        buf, offs, S, m_max, spans = pack_corridors(sets, self.query_scene)
+        out = [None if sp is None else np.zeros(0, np.int32) for sp in spans]
+        if S == 0:
+            return out
+        dev = torch.from_numpy(buf).to("cuda", non_blocking=False)
+        base = dev.data_ptr()
+        work = torch.empty((self._lib.bp_sets_obstacles_workspace_bytes(S),), dtype=torch.uint8, device="cuda")
+        hit = torch.empty((S,), dtype=torch.int32, device="cuda")
+        stream = torch.cuda.current_stream()
+        self.corridor_events = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+        self.corridor_events[0].record(stream)
+        _lib.check(self._lib.bp_sets_obstacles(self.scene._h, ctypes.c_void_p(base + offs[3]),
+                                               ctypes.c_void_p(base + offs[0]), ctypes.c_void_p(base + offs[1]),
+                                               ctypes.c_void_p(base + offs[2]), S, m_max, float(tol),
+                                               ctypes.c_void_p(hit.data_ptr()), ctypes.c_void_p(work.data_ptr()),
+                                               work.numel(), ctypes.c_void_p(stream.cuda_stream)))
+        self.corridor_events[1].record(stream)
+        h = hit.cpu().numpy()
+        for i, sp in enumerate(spans):
+            if sp is not None:
+                out[i] = h[sp[0]: sp[0] + sp[1]].copy()
+        return out
+
+    def run(self, rng_seeds=None, sample_chunk=32, want_nodes=True, queries=None, active=None):
         """Plan the batch: (results, stats).  queries: new per-query inputs (start, end, r0, r1, first_sample and the
         replanning keys of planner.plan_batch) to plan against the scenes of this planner; their obstacles must be
         the ones it was created with, or last updated to (ValueError otherwise: the host push-out of `end` and the
         device scene must agree).  Over shared scenes, they carry the planner's scene indices instead (ValueError
-        otherwise)."""
+        otherwise).  active: [Q] flags (or None: all): only the queries with a true flag are planned
+        (bp_plan_run_active), each with the results it gets in a run of the whole batch; a skipped query's result is
+        None and the stats count the active queries only."""
+        active = active_mask(active, len(self.queries))
         if queries is not None:
             if len(queries) != len(self.queries):
                 raise ValueError(f"{len(queries)} queries for a planner of {len(self.queries)} scenes")
@@ -423,7 +513,8 @@ class NativePlanner:
                 if not np.array_equal(scene_map(queries, self.scenes), self.query_scene):
                     raise ValueError("the queries' scene indices differ from the planner's")
                 return self._run(PackedQueries(queries, self.infl, self.ws_max, self.ws_min, rng_seeds, sample_chunk,
-                                               want_nodes, scenes=self.scenes, scene_arrays=self._scene_arrays()))
+                                               want_nodes, scenes=self.scenes, scene_arrays=self._scene_arrays()),
+                                 active)
             pk = PackedQueries(queries, self.infl, self.ws_max, self.ws_min, rng_seeds, sample_chunk, want_nodes)
             if self._obstacles is None:
                 self._obstacles = self._obstacles_of(
@@ -431,7 +522,7 @@ class NativePlanner:
             mine, theirs = self._obstacles, self._obstacles_of(pk)
             if mine[0] != theirs[0] or not np.array_equal(mine[1], theirs[1]) or not np.array_equal(mine[2], theirs[2]):
                 raise ValueError("the queries' obstacles differ from the scenes this planner was created with")
-            return self._run(pk)
+            return self._run(pk, active)
         # the packed host arrays of the batch (inputs incl. every query's generator state, output buffers) are kept
         # per seed list: planning the same batch again only runs the driver
         key = (None if rng_seeds is None else tuple(int(v) for v in rng_seeds), int(sample_chunk), bool(want_nodes))
@@ -442,16 +533,20 @@ class NativePlanner:
                                scene_arrays=self._scene_arrays() if self.scenes is not None else None)
             if rng_seeds is not None:
                 self._packed = {key: pk}
-        return self._run(pk)
+        return self._run(pk, active)
 
-    def _run(self, pk):
+    def _run(self, pk, active=None):
         import torch
 
         from . import _lib
 
-        _lib.check(self._lib.bp_plan_run(self._h, ctypes.byref(pk.inp), ctypes.byref(pk.out),
-                                         ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
-        return pk.results(), pk.stats_dict()
+        stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+        if active is None:
+            _lib.check(self._lib.bp_plan_run(self._h, ctypes.byref(pk.inp), ctypes.byref(pk.out), stream))
+        else:
+            _lib.check(self._lib.bp_plan_run_active(self._h, ctypes.byref(pk.inp), active.ctypes.data_as(_ip),
+                                                    ctypes.byref(pk.out), stream))
+        return pk.results(active), pk.stats_dict()
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
@@ -466,11 +561,13 @@ class NativePlanner:
 
 
 def plan_batch_native(queries, obs_size_increase=0.01, workspace_max=(1.0, 1.0, 1.2), workspace_min=(-1.0, -1.0, 0.0),
-                      rng_seeds=None, sample_chunk=32, scenes=None):
+                      rng_seeds=None, sample_chunk=32, scenes=None, active=None):
     """Drop-in for ``planner.plan_batch``: (results, stats).  Box or polytope queries, one kind per batch; with
-    ``scenes``, queries over shared scenes (see NativePlanner)."""
+    ``scenes``, queries over shared scenes (see NativePlanner); ``active``: plan only the flagged queries (see
+    NativePlanner.run)."""
+    active_mask(active, len(queries))
     pl = NativePlanner(queries, obs_size_increase, workspace_max, workspace_min, scenes=scenes)
     try:
-        return pl.run(rng_seeds, sample_chunk)
+        return pl.run(rng_seeds, sample_chunk, active=active)
     finally:
         pl.close()

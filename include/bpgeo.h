@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define BPGEO_ABI_VERSION 6
+#define BPGEO_ABI_VERSION 7
 #define BP_MAX_ROWS 48 /* hard cap on rows per convex set (reference MVIE cap: 20, quirk Q5) */
 
 typedef struct bp_scene bp_scene;
@@ -256,6 +256,23 @@ int bp_pairs_feasible_list(const double* A_dev, const double* b_dev, const int* 
                            const int* pairs_dev, int P, int* result_dev, double* x_feas_dev, void* workspace_dev,
                            size_t workspace_bytes, void* stream);
 
+/* ---- set-obstacle hit test (ABI 7): are planned sets still free after the obstacles moved? ----------------
+ * For S sets (A[S,m_max,3] | b | m, padded rows A = 0, b = 10 accepted), first_hit[s] = the lowest obstacle index,
+ * local to the set's scene, of an obstacle that set s intersects in the sense of BoundPlanner.set_intersection
+ * (BoundPlanner.py:774-787): the set and the obstacle, each shrunk by tol, share a point -- the decision of an edge of
+ * the set graph.  -1: no obstacle of the scene does; -2: set_scene_dev[s] lies outside [0, n_scenes) (checked on the
+ * device, nothing out of range is read).  The obstacle rows are the scene's: a box gives [I; -I] x <= [ub; -lb] of
+ * the inflated columns (the reference's make_box + obs_size_increase rows, bit for bit), a polytope its rows.
+ * set_scene_dev [S] or NULL (every set in scene 0; a single scene has n_scenes = 1).  Box and polytope scenes, single
+ * scenes and batches.  A set whose box (bp_set_aabb) misses an obstacle's box is not tested against it; the others
+ * go through the LP of bp_pair_feasible in index order and the first hit ends the set's search.  Workspace:
+ * bp_sets_obstacles_workspace_bytes(S) (the set boxes).  Fails for m_max outside 1 .. 48 and for a negative or
+ * non-finite tol.  Used by an MPC loop to replan only the queries whose corridor (sets_via_prev) an obstacle entered. */
+size_t bp_sets_obstacles_workspace_bytes(int S);
+int bp_sets_obstacles(const bp_scene* scene, const int* set_scene_dev /*[S] or NULL: scene 0*/, const double* A_dev,
+                      const double* b_dev, const int* m_dev, int S, int m_max, double tol, int* first_hit_dev /*[S]*/,
+                      void* workspace_dev, size_t workspace_bytes, void* stream);
+
 /* ---- K8 (next row 1): redundancy removal ---------------------------------------------
  * Replaces reduce_ineqs (bound_planner/utils/util_functions.py:82-88, cddlib
  * matrix_redundancy_remove) for S sets.  Kept rows keep their order and coefficients;
@@ -409,6 +426,14 @@ typedef struct bp_plan bp_plan;
 int bp_plan_create(const bp_scene* scene_batch, int Q, bp_plan** out);
 int bp_plan_create_mapped(const bp_scene* scene_batch, int Q, const int* query_scene_host /*[Q]*/, bp_plan** out);
 int bp_plan_run(bp_plan* plan, const bp_plan_in* in, bp_plan_out* out, void* stream);
+/* bp_plan_run_active (ABI 7) plans the queries q with active_host[q] != 0 only (NULL: all, as bp_plan_run), e.g. the
+ * queries of an MPC step whose corridor bp_sets_obstacles found hit.  `in` and `out` are the whole batch's, checked as
+ * by bp_plan_run.  A skipped query gets no state machine, no request and no table write; its outputs are left as they
+ * are, except finish_round[q] = -1, and stats count the active queries only.  An active query's outputs are bit for
+ * bit the ones bp_plan_run gives it over the whole batch (generator state and errors included), on plans from
+ * bp_plan_create and bp_plan_create_mapped.  The active queries are dealt to the lanes in turn (k-th -> lane k mod L). */
+int bp_plan_run_active(bp_plan* plan, const bp_plan_in* in, const int* active_host /*[Q] or NULL*/, bp_plan_out* out,
+                       void* stream);
 int bp_plan_destroy(bp_plan* plan);
 
 /* ---- multi-GPU exchange by peer stores (SURVEY 8e) -------------------------------------------------------
